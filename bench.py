@@ -116,6 +116,36 @@ def make_clip():
     return harness.synth_pcm(seconds=CLIP_SECONDS, sr=RATE, channels=CHANNELS, bits=BITS, seed=1)
 
 
+DUMP_LIMIT_BYTES = 64_000_000        # all files --dump-outputs writes, together
+DUMP_FRAMES = 1 << 17                # decoded frames kept per preset
+
+
+def dump_outputs(path, streams, decoded):
+    """--dump-outputs: what the last timed sweep step returned, as float32 .npy files, so that two builds can be compared
+    file for file.  m<preset>_stream.npy is the whole compressed stream of that preset (one value per byte);
+    m<preset>_decoded.npy is its decoded PCM [channel][frame] at DUMP_FRAMES frame positions drawn once with a fixed seed
+    (sorted, the same for every preset and run): eight full planes would not fit the size limit beside the streams.
+    The clip is 16-bit, so every value is exact in float32.  Should the streams leave less room than that, fewer frames
+    are kept (with a warning on stderr), and nothing is written if the streams alone exceed the limit: the bench itself
+    goes on either way."""
+    arrays = {f"m{m}_stream": streams[m].cpu().numpy().astype(np.float32) for m in sorted(streams)}
+    room = DUMP_LIMIT_BYTES - sum(a.nbytes for a in arrays.values()) - 2 * 128 * len(arrays)     # 128: an .npy header
+    nch, n = next(iter(decoded.values())).shape
+    if room < 0:
+        print(f"bench.py: --dump-outputs writes nothing: the streams alone exceed {DUMP_LIMIT_BYTES} bytes", file=sys.stderr)
+        return
+    keep = min(n, DUMP_FRAMES, room // (4 * nch * len(decoded)))
+    if keep < min(n, DUMP_FRAMES):
+        print(f"bench.py: --dump-outputs keeps {keep} decoded frames per preset to stay within {DUMP_LIMIT_BYTES} bytes",
+              file=sys.stderr)
+    frames = np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+    for m in sorted(decoded):
+        arrays[f"m{m}_decoded"] = decoded[m].cpu().numpy()[:, frames].astype(np.float32)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # =================================================================================================
 # reference arm
 # =================================================================================================
@@ -1037,6 +1067,8 @@ def run_b200(args, rank, world, local_rank):
     sampler.start()
     ms_res, launches = timed(step_resident, args.steps, args.warmup, profile=True)
     sampler.stop_flag.set(); sampler.join(timeout=3)
+    if args.dump_outputs and rank == 0:         # before the legs below run the same handles again
+        dump_outputs(args.dump_outputs, {m: d_out[m][:sizes[m]] for m in PRESETS}, {m: d_backs[m][:, :n] for m in PRESETS})
 
     # correctness of what was just timed (outside the timed region)
     torch.cuda.synchronize()
@@ -1324,7 +1356,14 @@ def main():
     ap.add_argument("--no-streaming", action="store_true", help="skip the EncodeBlock / DecodeBlock latency leg")
     ap.add_argument("--no-refine", action="store_true", help="skip the IRLS / SGD leg")
     ap.add_argument("--no-inlib", action="store_true", help="skip the in-library multi-GPU / pipelining leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the compressed streams and (a fixed sample of) the decoded PCM of the last timed sweep step "
+                         "to DIR/<name>.npy (float32, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 sweep")
     if args.sweep_only:
         args.c3_seconds = args.c4_seconds = 0.0
         if not args.with_inlib:

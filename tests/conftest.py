@@ -63,6 +63,14 @@ def ref():
 
 
 @pytest.fixture(scope="session")
+def reference():
+    """The reference's answers: live from oracle/_ref where it was built (and checked against the stored ones), else
+    the stored ones (tests/golden/reference_record.json)."""
+    import harness
+    return harness.ReferenceRecord(harness.Ref() if harness.have_ref() else None)
+
+
+@pytest.fixture(scope="session")
 def hostsim():
     import harness
     return harness.HostSim()

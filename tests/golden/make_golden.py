@@ -1,5 +1,5 @@
-"""Generate tests/golden/*.npz with the UNMODIFIED reference (oracle/_ref/liblinne_ref.so, built from
-/root/reference by oracle/Makefile).  Run in the build container:  python tests/golden/make_golden.py
+"""Generate tests/golden/*.npz with the UNMODIFIED reference (oracle/_ref/liblinne_ref.so, built from its sources
+by `make -C oracle ref REF=<reference checkout>`):  python tests/golden/make_golden.py
 
 Each fixture holds the PCM, the reference's .lnn bytes and, per compressed block-channel, the
 analysis results the reference kept in its handle (unit counts, shifts, quantised coefficients,
@@ -7,8 +7,16 @@ pre-emphasis state) plus the residual -- so the parity tests can check
   * oracle / GPU decode(reference bytes) == PCM                       (bit-exact decode)
   * oracle encode == reference bytes                                   (oracle pinned)
   * GPU pack(reference coefficients) == reference bytes                (identical coefficients -> identical bits)
-without /root/reference being present (it is not on the GPU box).
+without the reference being present.
+
+    python tests/golden/make_golden.py --record    writes tests/golden/reference_record.json instead: the answers
+the comparison tests of test_oracle_vs_reference.py and test_cli.py ask of the reference (CRCs, Huffman tables,
+stream digests), taken by running those tests with a recording harness.ReferenceRecord.  They come from
+oracle/_ref where it was built; otherwise from the oracle, which those same tests pin to the reference byte for
+byte wherever oracle/_ref exists (they then check every stored answer against the live reference).  The file names
+its source.
 """
+import json
 import os
 import sys
 
@@ -27,6 +35,27 @@ CASES = [
     ("eightch24_m7", 8, 24, 2304, 1024, 7, 25),
     ("mono24_m2", 1, 24, 4096, 4096, 2, 26),
 ]
+
+
+def record():
+    import test_cli
+    import test_oracle_vs_reference as t
+    oracle = harness.Oracle()
+    live, source = (harness.Ref(), "reference") if harness.have_ref() else (oracle, "oracle")
+    rec = harness.ReferenceRecord(live, recording=True)
+    t.test_live_crc_and_huffman(oracle, rec)
+    for preset in range(8):
+        t.test_live_streams_identical(oracle, rec, preset)
+    for channels, bits in [(1, 8), (2, 24), (8, 24), (3, 16)]:
+        t.test_live_formats_identical(oracle, rec, channels, bits)
+    t.test_live_reference_generators_roundtrip(oracle, rec)
+    t.test_live_af_and_learning_identical(oracle, rec)
+    for case in test_cli.CASES:
+        test_cli.reference_cli_answer(rec, case)
+    with open(harness.RECORD_JSON, "w") as f:
+        json.dump({"source": source, "answers": rec.answers}, f, indent=0, sort_keys=True)
+        f.write("\n")
+    print(harness.RECORD_JSON, len(rec.answers), "answers from the", source)
 
 
 def main():
@@ -62,4 +91,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    record() if sys.argv[1:] == ["--record"] else main()

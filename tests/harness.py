@@ -11,6 +11,8 @@ cpu_baseline / --impl reference legs import this module's `Ref` / `Oracle` class
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
 import os
 import sys
 import numpy as np
@@ -113,6 +115,40 @@ class Ref(LinneApi):
             return b"".join(stream), blocks
         finally:
             self.lib.LINNEEncoder_Destroy(enc)
+
+
+# ----------------------------------------------------------------------------------------------
+# The reference's answers for the inputs of the comparison tests, stored in tests/golden/reference_record.json
+# (made by tests/golden/make_golden.py --record), so that a checkout without oracle/_ref still compares
+# ----------------------------------------------------------------------------------------------
+RECORD_JSON = os.path.join(ROOT, "tests", "golden", "reference_record.json")
+
+
+def digest(data: bytes) -> str:
+    """A stream as it is recorded: its length and SHA-256."""
+    return f"{len(data)}:{hashlib.sha256(data).hexdigest()}"
+
+
+class ReferenceRecord:
+    """expect(key, ask) is what the reference answers to `ask`.  With a live reference (`live`, where oracle/_ref was
+    built) the answer is ask(live) and must equal the stored one; without it the stored answer stands in.  With
+    `recording` set, answers are taken from `live` and collected in `answers` instead of checked."""
+
+    def __init__(self, live=None, recording=False):
+        self.live, self.recording, self.answers = live, recording, {}
+        if not recording:
+            with open(RECORD_JSON) as f:
+                self.stored = json.load(f)["answers"]
+
+    def expect(self, key, ask):
+        if self.recording:
+            self.answers[key] = ask(self.live)
+            return self.answers[key]
+        assert key in self.stored, f"{key} is not in {os.path.relpath(RECORD_JSON, ROOT)}"
+        want = self.stored[key]
+        if self.live is not None:
+            assert ask(self.live) == want, f"the reference's answer to {key} differs from the stored one"
+        return want
 
 
 # ----------------------------------------------------------------------------------------------

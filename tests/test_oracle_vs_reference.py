@@ -1,6 +1,6 @@
 """Pin the oracle (oracle/linne_oracle.c) to the reference: known-answer vectors from the reference's
-own tests, the committed golden streams, and -- where oracle/_ref was built -- live byte-for-byte
-comparison with the unmodified reference."""
+own tests, the committed golden streams, and byte-for-byte comparison with the unmodified reference: live where
+oracle/_ref was built, otherwise with the reference's answers stored in tests/golden/reference_record.json."""
 import numpy as np
 import pytest
 
@@ -48,47 +48,47 @@ def test_golden_streams(oracle, name):
     assert oracle.encode(pcm, bits=int(g["bits"]), block=int(g["block"]), preset=int(g["preset"])) == stream
 
 
-# ---- live comparison with the unmodified reference (skipped where oracle/_ref is absent) ----------
-def test_live_crc_and_huffman(oracle, ref):
+# ---- comparison with the unmodified reference: live where oracle/_ref was built, else with its stored answers ----
+def test_live_crc_and_huffman(oracle, reference):
     rng = np.random.default_rng(3)
     for n in (1, 7, 64, 1000, 40971):
         data = rng.integers(0, 256, n, dtype=np.uint8).tobytes()
-        assert oracle.crc16(data) == ref.crc16(data)
-    for counts in ([1, 1, 1, 1], [0, 5, 0, 9, 2], list(rng.integers(0, 1000, 200))):
-        c0, l0 = oracle.huffman_codes(counts); c1, l1 = ref.huffman_codes(counts)
-        assert np.array_equal(c0, c1) and np.array_equal(l0, l1)
+        assert oracle.crc16(data) == reference.expect(f"crc16/{n}", lambda r: r.crc16(data))
+    for i, counts in enumerate(([1, 1, 1, 1], [0, 5, 0, 9, 2], list(rng.integers(0, 1000, 200)))):
+        ours = [a.tolist() for a in oracle.huffman_codes(counts)]
+        assert ours == reference.expect(f"huffman/{i}", lambda r: [a.tolist() for a in r.huffman_codes(counts)])
+
+
+def _encode_identical(oracle, reference, key, pcm, **kw):
+    """oracle.encode(pcm, **kw) gives the reference's bytes, and decodes back to pcm."""
+    ours = oracle.encode(pcm, **kw)
+    assert harness.digest(ours) == reference.expect(key, lambda r: harness.digest(r.encode(pcm, **kw))), key
+    assert np.array_equal(oracle.decode(ours), pcm), key
 
 
 @pytest.mark.parametrize("preset", range(8))
-def test_live_streams_identical(oracle, ref, preset):
+def test_live_streams_identical(oracle, reference, preset):
     pcm = harness.synth_pcm(seconds=1.2, channels=2, bits=16, seed=40 + preset)
-    a = ref.encode(pcm, preset=preset)
-    assert oracle.encode(pcm, preset=preset) == a
-    assert np.array_equal(oracle.decode(a), pcm)
+    _encode_identical(oracle, reference, f"streams/m{preset}", pcm, preset=preset)
 
 
 @pytest.mark.parametrize("channels,bits", [(1, 8), (2, 24), (8, 24), (3, 16)])
-def test_live_formats_identical(oracle, ref, channels, bits):
+def test_live_formats_identical(oracle, reference, channels, bits):
     pcm = harness.synth_pcm(n=2600, channels=channels, bits=bits, seed=7)
     for preset in (0, 5):
-        a = ref.encode(pcm, bits=bits, preset=preset, block=1024)
-        assert oracle.encode(pcm, bits=bits, preset=preset, block=1024) == a
-        assert np.array_equal(oracle.decode(a), pcm)
+        _encode_identical(oracle, reference, f"formats/{channels}ch{bits}/m{preset}", pcm, bits=bits, preset=preset, block=1024)
 
 
-def test_live_reference_generators_roundtrip(oracle, ref):
+def test_live_reference_generators_roundtrip(oracle, reference):
     # the nine generators of test/linne_encode_decode/main.cpp at 8192 samples / block 1024
     for name, gen in harness.reference_test_generators().items():
         for channels, bits, preset in ((1, 16, 0), (2, 8, 7), (2, 24, 7)):
             pcm = harness.to_fixed(gen(channels, 8192), bits)
-            a = ref.encode(pcm, bits=bits, rate=8000, block=1024, preset=preset)
-            b = oracle.encode(pcm, bits=bits, rate=8000, block=1024, preset=preset)
-            assert a == b, (name, channels, bits, preset)
-            assert np.array_equal(oracle.decode(a), pcm), (name, channels, bits, preset)
+            _encode_identical(oracle, reference, f"generators/{name}/{channels}ch{bits}/m{preset}", pcm,
+                              bits=bits, rate=8000, block=1024, preset=preset)
 
 
-def test_live_af_and_learning_identical(oracle, ref):
+def test_live_af_and_learning_identical(oracle, reference):
     pcm = harness.synth_pcm(n=2048, channels=1, bits=16, seed=9)
-    assert oracle.encode(pcm, preset=0, block=1024, af=2) == ref.encode(pcm, preset=0, block=1024, af=2)
-    pcm = pcm[:, :1024]
-    assert oracle.encode(pcm, preset=0, block=1024, learning=1) == ref.encode(pcm, preset=0, block=1024, learning=1)
+    _encode_identical(oracle, reference, "af2", pcm, preset=0, block=1024, af=2)
+    _encode_identical(oracle, reference, "learning1", pcm[:, :1024], preset=0, block=1024, learning=1)
