@@ -82,6 +82,52 @@ LINNEApiResult LINNEB200_EncodeFilesPacked(struct LINNEEncoder *encoder, const u
 LINNEApiResult LINNEB200_DecodeFilesPacked(struct LINNEDecoder *decoder, const uint8_t *data, uint32_t data_size,
         struct LINNEB200FileDesc *files, uint32_t num_files, uint8_t *pcm);
 
+/* ---- random access: seek index and sample-window decodes -----------------------------------------------
+ * Every block is self-contained, so an excerpt of a stream needs only the blocks it overlaps.  A seek index holds one
+ * point per block, in stream order: the block's first sample and the byte offset of its sync code, counted from the
+ * start of the image (30-byte header included).  The first point is always (0, 30).  A caller may keep the index next to
+ * the stream (a sidecar file); the library checks every index it is given and never reads outside the image because of it.
+ *
+ * BuildIndex hops once over the stream -- the host image `data`, or the device image `d_data` when data == NULL (the hop
+ * then runs on the device, as in DecodeWholeResident) -- latches the stream's header on the handle (as SetHeader does)
+ * and writes one point per block to `points`.  It returns the result the hop of DecodeWhole gives for the stream's
+ * framing; on a stream damaged part-way through, the points of the blocks before the damage are written.  `*num_points`
+ * is always the number of blocks found; if it exceeds `capacity`, the first `capacity` points are written and the call
+ * returns INSUFFICIENT_BUFFER (call again with that capacity; points may be NULL when capacity is 0). */
+struct LINNEB200SeekPoint { uint32_t first_sample, byte_offset; };
+LINNEApiResult LINNEB200_DecoderBuildIndex(struct LINNEDecoder *decoder, const uint8_t *data, const uint8_t *d_data,
+        uint32_t data_size, struct LINNEB200SeekPoint *points, uint32_t capacity, uint32_t *num_points);
+
+/* DecodeWindows decodes sample windows of the stream whose header is latched on the handle.  Window w receives samples
+ * [first_sample, first_sample + num_samples) of every channel, exactly as DecodeWhole writes them, at out_offset of the
+ * caller's planes (buffer[c][out_offset ...]; resident: d_pcm[c * pcm_stride + out_offset ...]).  The blocks the
+ * windows need go through the kernels as ONE batch and each is decoded once, even when windows overlap; windows may be
+ * unsorted, overlapping, repeated or empty.  A host image uploads only the bytes of the needed blocks.  The device image
+ * of DecodeWindowsResident must be followed by >= 16 readable bytes.  A handle with several devices decodes windows on
+ * its own device; the DecodeBlock read-ahead cache is left as it was.
+ *
+ * Rejected as a whole (nothing written, no status set): NULL pointers (INVALID_ARGUMENT), no latched header
+ * (PARAMETER_NOT_SET), fewer buffer channels than the stream has (INSUFFICIENT_BUFFER), and INVALID_ARGUMENT for a
+ * window that ends past the stream's num_samples or whose output range leaves the buffer (buffer_num_samples /
+ * pcm_stride), and for an index that does not start at (0, 30), is not strictly increasing in both fields, or has a
+ * point at or beyond data_size or num_samples.
+ *
+ * Stream damage is reported per window: `status` = the result of the first failing block the window needs, in stream
+ * order -- INVALID_FORMAT (no sync code at the indexed offset, a bad block type, a block that disagrees with the index
+ * in its sample count or runs past the next indexed block), INSUFFICIENT_DATA (a block that runs past the image),
+ * DETECT_DATA_CORRUPTION (CRC mismatch, when the handle checks CRCs).  A failed window's samples are undefined, every
+ * other window is exact.  The call returns the first non-OK status in window order.
+ *
+ * A player seeks without these calls: LINNEDecoder_DecodeBlock(decoder, data + points[k].byte_offset,
+ * data_size - points[k].byte_offset, ...) decodes block k and the ones after it, one per call. */
+struct LINNEB200Window { uint32_t first_sample, num_samples, out_offset; int32_t status; };
+LINNEApiResult LINNEB200_DecodeWindows(struct LINNEDecoder *decoder, const uint8_t *data, uint32_t data_size,
+        const struct LINNEB200SeekPoint *points, uint32_t num_points, struct LINNEB200Window *windows, uint32_t num_windows,
+        int32_t **buffer, uint32_t buffer_num_channels, uint32_t buffer_num_samples);
+LINNEApiResult LINNEB200_DecodeWindowsResident(struct LINNEDecoder *decoder, const uint8_t *d_data, uint32_t data_size,
+        const struct LINNEB200SeekPoint *points, uint32_t num_points, struct LINNEB200Window *windows, uint32_t num_windows,
+        int32_t *d_pcm, uint32_t pcm_stride);
+
 /* ---- packed PCM entry points (SURVEY 8f.2) ------------------------------------------------------------
  * `pcm` = interleaved little-endian samples exactly as in a WAV data chunk (8-bit unsigned with a bias of 128,
  * 16/24/32-bit signed; bits per sample = the encoder's parameter / the stream header).  The conversion to and

@@ -8,6 +8,6 @@ encode/decode path, behind the reference's own C API.
 
 Everything heavy lives in linne_b200/csrc (host C + CUDA); this package is a thin ctypes mirror.
 """
-from .api import (Product, LinneApi, load_library, EncoderSession, DecoderSession, DeviceBuffer, PeerMapping, ChannelParams, FileDesc, LINNEHeader, LINNEEncodeParameter,  # noqa: F401
+from .api import (Product, LinneApi, load_library, EncoderSession, DecoderSession, DeviceBuffer, PeerMapping, ChannelParams, FileDesc, SeekPoint, Window, LINNEHeader, LINNEEncodeParameter,  # noqa: F401
                   LINNEEncoderConfig, LINNEDecoderConfig, OK, INVALID_ARGUMENT, INVALID_FORMAT,
                   INSUFFICIENT_BUFFER, INSUFFICIENT_DATA, PARAMETER_NOT_SET, DATA_CORRUPTION, NG)

@@ -188,6 +188,82 @@ class LinneApi:
             self.lib.LINNEDecoder_Destroy(dec)
 
 
+    # -- random access (include/linne_b200.h: seek index, sample windows) ---------------------------
+    def _open_decoder(self, channels, check_crc):
+        cfg = LINNEDecoderConfig(max(channels, 1), 3, 128, check_crc)
+        dec = self.lib.LINNEDecoder_Create(C.byref(cfg), None, 0)
+        if not dec:
+            raise RuntimeError("LINNEDecoder_Create failed")
+        return dec
+
+    def _build_index(self, dec, data: bytes):
+        buf = np.frombuffer(data, dtype=np.uint8)
+        u8p = buf.ctypes.data_as(C.POINTER(C.c_uint8))
+        n = C.c_uint32(0)
+        rc = self.lib.LINNEB200_DecoderBuildIndex(dec, u8p, None, len(data), None, 0, C.byref(n))
+        if rc not in (OK, INSUFFICIENT_BUFFER) and n.value == 0:
+            return rc, np.zeros((0, 2), np.uint32)
+        pts = (SeekPoint * max(1, n.value))()
+        rc = self.lib.LINNEB200_DecoderBuildIndex(dec, u8p, None, len(data), pts, n.value, C.byref(n))
+        arr = np.frombuffer(bytes(pts), dtype=np.uint32).reshape(-1, 2)[:n.value].copy()
+        return rc, arr
+
+    def build_index(self, data: bytes, return_code=False):
+        """-> uint32 [N, 2]: (first sample, byte offset) of every block (LINNEB200_DecoderBuildIndex)"""
+        rc, hdr = self.decode_header(data)
+        dec = self._open_decoder(hdr.num_channels if rc == OK else 1, 1)
+        try:
+            rc, arr = self._build_index(dec, data)
+        finally:
+            self.lib.LINNEDecoder_Destroy(dec)
+        if return_code:
+            return rc, arr
+        if rc != OK:
+            raise RuntimeError(f"BuildIndex rc={rc}")
+        return arr
+
+    def decode_windows(self, data: bytes, starts, lengths, index=None, check_crc=1, return_code=False):
+        """Samples [starts[w], starts[w] + lengths[w]) of every channel -> list of int32 [C][len] arrays
+        (LINNEB200_DecodeWindows); with return_code: (rc, arrays, per-window statuses)."""
+        starts, lengths = [int(s) for s in starts], [int(n) for n in lengths]
+        if len(starts) != len(lengths):
+            raise ValueError("starts and lengths differ in length")
+        rc, hdr = self.decode_header(data)
+        if rc != OK:
+            if return_code:
+                return rc, [], []
+            raise RuntimeError(f"DecodeHeader rc={rc}")
+        nch = hdr.num_channels
+        dec = self._open_decoder(nch, check_crc)
+        try:
+            if index is None:
+                rc, index = self._build_index(dec, data)
+                if rc != OK:
+                    if return_code:
+                        return rc, [], []
+                    raise RuntimeError(f"BuildIndex rc={rc}")
+            else:
+                rc = self.lib.LINNEDecoder_SetHeader(dec, C.byref(hdr))
+                if rc != OK:
+                    raise RuntimeError(f"SetHeader rc={rc}")
+            pts, npts = index_points(index)
+            offs = np.concatenate([[0], np.cumsum(lengths, dtype=np.int64)]).astype(np.int64)
+            total = int(offs[-1])
+            out = np.zeros((max(nch, 1), max(total, 1)), dtype=np.int32)
+            wins = (Window * max(1, len(starts)))(*[Window(s, n, int(o), 0) for s, n, o in zip(starts, lengths, offs)])
+            buf = np.frombuffer(data, dtype=np.uint8)
+            rc = self.lib.LINNEB200_DecodeWindows(dec, buf.ctypes.data_as(C.POINTER(C.c_uint8)), len(data), pts, npts,
+                                                  wins, len(starts), _chan_ptrs(out), nch, out.shape[1])
+            res = [out[:, offs[w]:offs[w + 1]] for w in range(len(starts))]
+            status = [int(wins[w].status) for w in range(len(starts))]
+            if return_code:
+                return rc, res, status
+            if rc != OK:
+                raise RuntimeError(f"DecodeWindows rc={rc} (statuses {status})")
+            return res
+        finally:
+            self.lib.LINNEDecoder_Destroy(dec)
+
 
 def bind_ext_api(lib):
     """Declare the LINNEB200_* extension entry points (include/linne_b200.h)."""
@@ -238,6 +314,14 @@ def bind_ext_api(lib):
     lib.LINNEB200_EncodeFilesPacked.restype = C.c_int
     lib.LINNEB200_DecodeFilesPacked.argtypes = [C.c_void_p, u8p, C.c_uint32, C.POINTER(FileDesc), C.c_uint32, u8p]
     lib.LINNEB200_DecodeFilesPacked.restype = C.c_int
+    lib.LINNEB200_DecoderBuildIndex.argtypes = [C.c_void_p, u8p, C.c_void_p, C.c_uint32, C.POINTER(SeekPoint), C.c_uint32, u32p]
+    lib.LINNEB200_DecoderBuildIndex.restype = C.c_int
+    lib.LINNEB200_DecodeWindows.argtypes = [C.c_void_p, u8p, C.c_uint32, C.POINTER(SeekPoint), C.c_uint32, C.POINTER(Window),
+                                            C.c_uint32, C.POINTER(C.POINTER(C.c_int32)), C.c_uint32, C.c_uint32]
+    lib.LINNEB200_DecodeWindows.restype = C.c_int
+    lib.LINNEB200_DecodeWindowsResident.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(SeekPoint), C.c_uint32,
+                                                    C.POINTER(Window), C.c_uint32, C.c_void_p, C.c_uint32]
+    lib.LINNEB200_DecodeWindowsResident.restype = C.c_int
     lib.LINNEB200_DecoderSetReadahead.argtypes = [C.c_void_p, C.c_uint32]
     lib.LINNEB200_DecoderSetThroughputBlocks.argtypes = [C.c_void_p, C.c_uint32]
     lib.LINNEB200_EncoderSetDevices.argtypes = [C.c_void_p, C.c_uint32]
@@ -282,6 +366,22 @@ class FileDesc(C.Structure):
     """struct LINNEB200FileDesc (include/linne_b200.h)"""
     _fields_ = [("first_sample", C.c_uint32), ("num_samples", C.c_uint32), ("out_offset", C.c_uint32),
                 ("out_size", C.c_uint32), ("status", C.c_int32)]
+
+
+class SeekPoint(C.Structure):
+    """struct LINNEB200SeekPoint (include/linne_b200.h): one block of a seek index"""
+    _fields_ = [("first_sample", C.c_uint32), ("byte_offset", C.c_uint32)]
+
+
+class Window(C.Structure):
+    """struct LINNEB200Window (include/linne_b200.h): one sample window of LINNEB200_DecodeWindows"""
+    _fields_ = [("first_sample", C.c_uint32), ("num_samples", C.c_uint32), ("out_offset", C.c_uint32), ("status", C.c_int32)]
+
+
+def index_points(index):
+    """uint32 [N, 2] (first_sample, byte_offset) -> ctypes SeekPoint array"""
+    index = np.ascontiguousarray(index, dtype=np.uint32).reshape(-1, 2)
+    return (SeekPoint * max(1, len(index))).from_buffer_copy(index.tobytes() or bytes(8)), len(index)
 
 
 class ChannelParams(C.Structure):

@@ -36,6 +36,8 @@ struct LINNEDecoder {
     LnbBuf h_stream;                       /* pinned copy of a device-resident stream (block hop on the host: fallback only) */
     LnbBuf d_hop_files, d_hop_res, d_hop_table, h_hop;     /* device-side block hop: records, results, table; pinned staging */
     LnbBuf h_pcm;                          /* pinned int32 [C][stage_stride]: PCM staging of DecodeBlock / read-ahead cache */
+    LnbBuf h_win, d_win;                   /* window decodes: seek inputs + gather records (pinned staging, device copy) */
+    LnbBuf h_win_img, h_win_pcm;           /* window decodes of host buffers: the needed blocks' bytes, the windows' samples (pinned) */
     /* DecodeBlock read-ahead (SURVEY 8f.4): blocks decoded ahead of the caller in one batch and served from here */
     uint32_t readahead;                    /* blocks decoded per batch by DecodeBlock (<= 1: batch of one) */
     uint32_t tput_min_blocks;              /* batches of at least this many blocks take the throughput kernels (0 = never) */
@@ -147,6 +149,10 @@ void LINNEDecoder_Destroy(struct LINNEDecoder *dec)
         lnb_buf_release_host(&dec->h_blocks);
         lnb_buf_release_host(&dec->h_stream);
         lnb_buf_release_host(&dec->h_pcm);
+        lnb_buf_release_device(dec->dev, &dec->d_win);
+        lnb_buf_release_host(&dec->h_win);
+        lnb_buf_release_host(&dec->h_win_img);
+        lnb_buf_release_host(&dec->h_win_pcm);
         free(dec->ra_image); dec->ra_image = NULL; dec->ra_image_cap = 0;
         free(dec->ra_blocks); dec->ra_blocks = NULL; dec->ra_blocks_cap = 0;
         dec->ra_count = dec->ra_next = 0;
@@ -244,6 +250,29 @@ static int scan_blocks(const struct LINNEHeader *h, const uint8_t *data, uint32_
     return 0;
 }
 
+/* Routing of a decode batch, the same for every caller: compressed blocks go to the fused streaming kernel (unless
+ * LINNE_B200_SPLIT_DECODE=1), what is left is counted for the split kernels, the longest block sizes their shared-memory
+ * lines, and batches of at least tput_min_blocks blocks take the throughput kernels (eight lanes per block / one per
+ * (block, channel) instead of one CTA per block, lnb_tput_v2.cuh).  batch->cfg must be filled in. */
+static void route_batch(const struct LINNEDecoder *dec, LnbDecodeBatch *batch, const LnbBlockDesc *blocks, uint32_t nb,
+                        const int32_t *pcm_base)
+{
+    const char *split = getenv("LINNE_B200_SPLIT_DECODE");
+    const uint32_t min_blocks = dec->tput_min_blocks;
+    uint32_t i;
+    batch->fused_max_n = (split && *split == '1') ? 0u : lnb_shim_fused_max_n();
+    batch->num_plain_blocks = 0;
+    batch->max_nsmp = 0;
+    for (i = 0; i < nb; i++) {
+        if (blocks[i].type != LNB_BLOCK_COMPRESSED || blocks[i].nsmp == 0u || blocks[i].nsmp > batch->fused_max_n)
+            batch->num_plain_blocks++;
+        if (blocks[i].nsmp > batch->max_nsmp) batch->max_nsmp = blocks[i].nsmp;
+    }
+    batch->tput = (min_blocks && nb >= min_blocks && batch->fused_max_n
+                   && ((uintptr_t)pcm_base & 15u) == 0u && (batch->cfg.pcm_stride & 3u) == 0u
+                   && lnb_shim_tput_supported(&batch->cfg)) ? 1u : 0u;
+}
+
 /* shared by DecodeBlock (block_limit >= 1, staged) and DecodeWhole (block_limit = 0) */
 /* Resident mode (d_stream_ext / d_pcm_ext non-NULL): the stream image and/or the PCM planes already
  * live on the device, so the corresponding bulk copy is skipped; `data` (host) is still needed for
@@ -316,25 +345,7 @@ static LINNEApiResult decode_range(struct LINNEDecoder *dec, const uint8_t *data
 
     /* a terminal block with a post-CRC error takes part in the CRC pass only */
     for (i = scan.num_decodable; i < scan.num_blocks; i++) blocks[i].type = 0xFFu;
-    {   /* compressed blocks go to the fused streaming kernel; count what is left for the split kernels */
-        const char *split = getenv("LINNE_B200_SPLIT_DECODE");
-        batch.fused_max_n = (split && *split == '1') ? 0u : lnb_shim_fused_max_n();
-        batch.num_plain_blocks = 0;
-        batch.max_nsmp = 0;
-        for (i = 0; i < scan.num_blocks; i++) {
-            if (blocks[i].type != LNB_BLOCK_COMPRESSED || blocks[i].nsmp == 0u || blocks[i].nsmp > batch.fused_max_n)
-                batch.num_plain_blocks++;
-            if (blocks[i].nsmp > batch.max_nsmp) batch.max_nsmp = blocks[i].nsmp;
-        }
-    }
-
-    {   /* Large batches: eight lanes per block / one per (block, channel) instead of one CTA per block (lnb_tput_v2.cuh) */
-        const uint32_t min_blocks = dec->tput_min_blocks;
-        const int32_t *pcm_base = d_pcm_ext ? d_pcm_ext : (const int32_t *)dec->d_pcm.ptr;
-        batch.tput = (min_blocks && scan.num_blocks >= min_blocks && batch.fused_max_n
-                      && ((uintptr_t)pcm_base & 15u) == 0u && (batch.cfg.pcm_stride & 3u) == 0u
-                      && lnb_shim_tput_supported(&batch.cfg)) ? 1u : 0u;
-    }
+    route_batch(dec, &batch, blocks, scan.num_blocks, d_pcm_ext ? d_pcm_ext : (const int32_t *)dec->d_pcm.ptr);
 
     batch.tab = *lnb_shim_tables(dec->dev);
     batch.stream = d_stream_ext ? d_stream_ext : (const uint8_t *)dec->d_stream.ptr;
@@ -840,20 +851,7 @@ static LINNEApiResult decode_files(struct LINNEDecoder *dec, const uint8_t *host
         batch.cfg.check_crc = (dec->flags & DEC_FLAG_CHECK_CRC) ? 1u : 0u;
         if (lnb_buf_reserve_device(dec->dev, &dec->d_blocks, (size_t)nb * sizeof(LnbBlockDesc))
             || lnb_buf_reserve_device(dec->dev, &dec->d_params, (size_t)nb * C * sizeof(LnbChanParams))) { free(first_block); return LINNE_APIRESULT_NG; }
-        {
-            const char *split = getenv("LINNE_B200_SPLIT_DECODE");
-            batch.fused_max_n = (split && *split == '1') ? 0u : lnb_shim_fused_max_n();
-            batch.num_plain_blocks = 0;
-            batch.max_nsmp = 0;
-            for (k = 0; k < nb; k++) {
-                if (blocks[k].type != LNB_BLOCK_COMPRESSED || blocks[k].nsmp == 0u || blocks[k].nsmp > batch.fused_max_n)
-                    batch.num_plain_blocks++;
-                if (blocks[k].nsmp > batch.max_nsmp) batch.max_nsmp = blocks[k].nsmp;
-            }
-        }
-        batch.tput = (dec->tput_min_blocks && nb >= dec->tput_min_blocks && batch.fused_max_n
-                      && ((uintptr_t)d_pcm & 15u) == 0u && (pcm_stride & 3u) == 0u
-                      && lnb_shim_tput_supported(&batch.cfg)) ? 1u : 0u;
+        route_batch(dec, &batch, blocks, nb, d_pcm);
         batch.tab = *lnb_shim_tables(dec->dev);
         batch.stream = d_data;
         batch.stream_size = data_size;
@@ -972,4 +970,301 @@ LINNEApiResult LINNEB200_DecodeWholePacked(struct LINNEDecoder *dec, const uint8
     ret = decode_packed_range(dec, data, data_size, LINNE_HEADER_SIZE, pcm, header.num_samples, header.num_samples, 0, &decoded);
     *num_frames = decoded;
     return ret;
+}
+
+/* ---- seek index and sample-window decodes (include/linne_b200.h) ------------------------------------------------------
+ * Every block is self-contained, so an excerpt needs only the blocks it overlaps.  BuildIndex hops once over the stream
+ * and keeps (first sample, byte offset) per block; DecodeWindows finds each window's blocks by binary search in that index,
+ * decodes the union of them as ONE batch into compact scratch planes and copies every window out of those planes. */
+LINNEApiResult LINNEB200_DecoderBuildIndex(struct LINNEDecoder *dec, const uint8_t *data, const uint8_t *d_data,
+        uint32_t data_size, struct LINNEB200SeekPoint *points, uint32_t capacity, uint32_t *num_points)
+{
+    struct LINNEHeader h;
+    const LnbBlockDesc *table;
+    LINNEApiResult ret;
+    BlockScan scan;
+    uint32_t i, n;
+    if (dec == NULL || num_points == NULL || (data == NULL && d_data == NULL) || (points == NULL && capacity)) return LINNE_APIRESULT_INVALID_ARGUMENT;
+    *num_points = 0;
+    if (data == NULL) {
+        /* the image is in HBM: its header comes up first (the hop's table is sized from the sample count) */
+        uint8_t *hdr;
+        if (data_size < LINNE_HEADER_SIZE) return LINNE_APIRESULT_INSUFFICIENT_DATA;
+        if (lnb_buf_reserve_host(&dec->h_hop, 64u)) return LINNE_APIRESULT_NG;
+        hdr = (uint8_t *)dec->h_hop.ptr;
+        lnb_shim_d2h(dec->dev, hdr, d_data, LINNE_HEADER_SIZE);
+        if (lnb_shim_sync(dec->dev)) return LINNE_APIRESULT_NG;
+        if ((ret = LINNEDecoder_DecodeHeader(hdr, data_size, &h)) != LINNE_APIRESULT_OK) return ret;
+    } else if ((ret = LINNEDecoder_DecodeHeader(data, data_size, &h)) != LINNE_APIRESULT_OK) {
+        return ret;
+    }
+    if ((ret = LINNEDecoder_SetHeader(dec, &h)) != LINNE_APIRESULT_OK) return ret;
+
+    memset(&scan, 0, sizeof(scan));
+    if (data == NULL) {
+        /* the device hop of one stream (lnb_hop.cuh), as DecodeWholeResident without a host copy runs it */
+        LnbHopFile *hf;
+        LnbHopResult *hr;
+        const uint32_t cap = h.num_samples / 256u + 64u;
+        if (lnb_buf_reserve_host(&dec->h_hop, sizeof(LnbHopFile) + sizeof(LnbHopResult))
+            || lnb_buf_reserve_device(dec->dev, &dec->d_hop_files, sizeof(LnbHopFile))
+            || lnb_buf_reserve_device(dec->dev, &dec->d_hop_res, sizeof(LnbHopResult))
+            || lnb_buf_reserve_device(dec->dev, &dec->d_hop_table, (size_t)cap * sizeof(LnbBlockDesc))
+            || lnb_buf_reserve_host(&dec->h_blocks, (size_t)cap * sizeof(LnbBlockDesc))) return LINNE_APIRESULT_NG;
+        hf = (LnbHopFile *)dec->h_hop.ptr;
+        hr = (LnbHopResult *)(hf + 1);
+        hf->offset = 0; hf->size = data_size; hf->room_samples = h.num_samples; hf->table_first = 0; hf->table_cap = cap;
+        lnb_shim_h2d(dec->dev, dec->d_hop_files.ptr, hf, sizeof(LnbHopFile));
+        if (lnb_shim_hop(dec->dev, d_data, (const LnbHopFile *)dec->d_hop_files.ptr, 1u,
+                         (LnbBlockDesc *)dec->d_hop_table.ptr, (LnbHopResult *)dec->d_hop_res.ptr)) return LINNE_APIRESULT_NG;
+        lnb_shim_d2h(dec->dev, hr, dec->d_hop_res.ptr, sizeof(LnbHopResult));
+        if (lnb_shim_sync(dec->dev)) return LINNE_APIRESULT_NG;
+        if (!hr->overflow) {
+            lnb_shim_d2h(dec->dev, dec->h_blocks.ptr, dec->d_hop_table.ptr, (size_t)hr->num_blocks * sizeof(LnbBlockDesc));
+            if (lnb_shim_sync(dec->dev)) return LINNE_APIRESULT_NG;
+            scan.num_blocks = hr->num_blocks; scan.num_decodable = hr->num_decodable;
+            scan.framing_error = (LINNEApiResult)hr->framing_error; scan.post_crc_error = (LINNEApiResult)hr->post_crc_error;
+        } else {
+            /* a stream of tiny blocks: the image comes to the host once and the hop runs there (as in decode_files) */
+            if (lnb_buf_reserve_host(&dec->h_stream, (size_t)data_size + 16u)) return LINNE_APIRESULT_NG;
+            lnb_shim_d2h(dec->dev, dec->h_stream.ptr, d_data, data_size);
+            if (lnb_shim_sync(dec->dev)) return LINNE_APIRESULT_NG;
+            data = (const uint8_t *)dec->h_stream.ptr;
+        }
+    }
+    if (data != NULL) {
+        uint32_t guess = h.num_samples_per_block ? h.num_samples / h.num_samples_per_block * 2u + 32u : data_size / 64u + 16u;
+        for (;;) {
+            if (lnb_buf_reserve_host(&dec->h_blocks, (size_t)guess * sizeof(LnbBlockDesc))) return LINNE_APIRESULT_NG;
+            if (scan_blocks(&h, data, data_size, LINNE_HEADER_SIZE, h.num_samples, h.num_samples, 0,
+                            (LnbBlockDesc *)dec->h_blocks.ptr, guess, &scan) == 0) break;
+            guess *= 2u;
+        }
+    }
+    /* the blocks a DecodeWhole would decode; the result is what its hop reports for the stream's framing */
+    table = (const LnbBlockDesc *)dec->h_blocks.ptr;
+    n = scan.num_decodable;
+    for (i = 0; i < n && i < capacity; i++) { points[i].first_sample = table[i].smp_off; points[i].byte_offset = table[i].byte_off; }
+    *num_points = n;
+    if (n > capacity) return LINNE_APIRESULT_INSUFFICIENT_BUFFER;
+    return (scan.num_blocks > scan.num_decodable) ? scan.post_crc_error : scan.framing_error;
+}
+
+/* index of the block that holds sample s: the last point whose first sample is <= s */
+static uint32_t find_block(const struct LINNEB200SeekPoint *points, uint32_t num_points, uint32_t s)
+{
+    uint32_t lo = 0, hi = num_points - 1u;
+    while (lo < hi) {
+        const uint32_t mid = lo + (hi - lo + 1u) / 2u;
+        if (points[mid].first_sample <= s) lo = mid; else hi = mid - 1u;
+    }
+    return lo;
+}
+
+/* Shared by DecodeWindows (host image `data`, PCM into the caller's planes `buffer`) and DecodeWindowsResident (device
+ * image `d_data`, PCM into the device planes `d_pcm`); `out_stride` = samples per output plane. */
+static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *data, const uint8_t *d_data, uint32_t data_size,
+        const struct LINNEB200SeekPoint *points, uint32_t num_points, struct LINNEB200Window *windows, uint32_t num_windows,
+        int32_t **buffer, int32_t *d_pcm, uint32_t out_stride)
+{
+    const struct LINNEHeader *h = &dec->header;
+    const uint32_t C = h->num_channels, N = num_points;
+    const int resident = (d_pcm != NULL);
+    LnbDecodeBatch batch;
+    LnbSeekIn *seek;
+    LnbGatherWin *gw;
+    LnbBlockDesc *blocks;
+    LINNEApiResult overall = LINNE_APIRESULT_OK;
+    int32_t *mark;
+    uint32_t *cpos, *err, *first_bad, *ok_block, *wk, i, k, j, c, nneed = 0, nok = 0, ngw = 0, run_start = 0, img_bytes = 0, scratch = 0, stride, dense_stride = 0;
+    uint64_t items = 0, dense = 0;
+    size_t win_bytes;
+
+    /* ---- validation: nothing is written and no status is set when the request is rejected ---- */
+    if (num_points == 0 || points[0].first_sample != 0u || points[0].byte_offset != LINNE_HEADER_SIZE) return LINNE_APIRESULT_INVALID_ARGUMENT;
+    for (k = 0; k < N; k++) {
+        if (points[k].byte_offset >= data_size || points[k].first_sample >= h->num_samples) return LINNE_APIRESULT_INVALID_ARGUMENT;
+        if (k && (points[k].first_sample <= points[k - 1].first_sample || points[k].byte_offset <= points[k - 1].byte_offset))
+            return LINNE_APIRESULT_INVALID_ARGUMENT;
+    }
+    for (i = 0; i < num_windows; i++)
+        if ((uint64_t)windows[i].first_sample + windows[i].num_samples > h->num_samples
+            || (uint64_t)windows[i].out_offset + windows[i].num_samples > out_stride) return LINNE_APIRESULT_INVALID_ARGUMENT;
+
+    /* ---- planning: the blocks every window needs, marked as ranges; needed blocks in stream order, each once ---- */
+    if (!(mark = (int32_t *)calloc((size_t)5u * N + 1u + 2u * (size_t)num_windows, sizeof(uint32_t)))) return LINNE_APIRESULT_NG;
+    cpos = (uint32_t *)(mark + N + 1u);                 /* scratch sample offset of a needed block */
+    err = cpos + N;                                     /* result of every block (OK for the ones nobody needs) */
+    first_bad = err + N;                                /* the first failing block at or after a block (N: none) */
+    ok_block = first_bad + N;                           /* stream index of each block of the decode batch */
+    wk = ok_block + N;                                  /* first and last block of each window */
+    for (i = 0; i < num_windows; i++) {
+        if (windows[i].num_samples == 0u) continue;
+        wk[2u * i] = find_block(points, N, windows[i].first_sample);
+        wk[2u * i + 1u] = find_block(points, N, windows[i].first_sample + windows[i].num_samples - 1u);
+        mark[wk[2u * i]]++;
+        mark[wk[2u * i + 1u] + 1u]--;
+    }
+    win_bytes = LNB_ROUNDUP((size_t)N * sizeof(LnbSeekIn), 16u);
+    if (lnb_buf_reserve_host(&dec->h_win, win_bytes + (size_t)num_windows * sizeof(LnbGatherWin))
+        || lnb_buf_reserve_host(&dec->h_blocks, (size_t)N * sizeof(LnbBlockDesc))) { free(mark); return LINNE_APIRESULT_NG; }
+    seek = (LnbSeekIn *)dec->h_win.ptr;
+    gw = (LnbGatherWin *)((uint8_t *)dec->h_win.ptr + win_bytes);
+    blocks = (LnbBlockDesc *)dec->h_blocks.ptr;
+    {
+        int32_t depth = 0;
+        uint32_t last = 0;
+        for (k = 0; k < N; k++) {
+            const uint32_t end_byte = (k + 1u < N) ? points[k + 1u].byte_offset : data_size;
+            const uint32_t nsmp = ((k + 1u < N) ? points[k + 1u].first_sample : h->num_samples) - points[k].first_sample;
+            depth += mark[k];
+            if (depth <= 0) continue;
+            if (nneed == 0 || last + 1u != k) {
+                /* a run of adjacent blocks starts 4-aligned in the scratch planes (the throughput kernels want smp_off % 4 == 0);
+                 * inside a run the blocks follow each other, so that every window is one contiguous run of the planes */
+                scratch = (uint32_t)LNB_ROUNDUP(scratch, 4u);
+                img_bytes = (uint32_t)LNB_ROUNDUP(img_bytes, 16u);
+                run_start = points[k].byte_offset;
+            }
+            cpos[k] = scratch;
+            /* host image: the needed blocks' bytes are staged run after run; device image: read where they are */
+            seek[nneed].img_off = data ? img_bytes + (points[k].byte_offset - run_start) : points[k].byte_offset;
+            seek[nneed].span = end_byte - points[k].byte_offset;
+            seek[nneed].remain = data_size - points[k].byte_offset;
+            seek[nneed].nsmp = nsmp;
+            seek[nneed].smp_off = scratch;
+            scratch += nsmp;
+            if (data) img_bytes = seek[nneed].img_off + seek[nneed].span;
+            last = k;
+            nneed++;
+        }
+    }
+    stride = (uint32_t)LNB_ROUNDUP((size_t)scratch + 4u, 4u);
+    for (i = 0; i < num_windows; i++) {                  /* gather records (zero-length windows have none) */
+        const struct LINNEB200Window *w = &windows[i];
+        uint32_t dst;
+        if (w->num_samples == 0u) continue;
+        dense = LNB_ROUNDUP(dense, 4u);
+        dst = resident ? w->out_offset : (uint32_t)dense;
+        gw[ngw].src = cpos[wk[2u * i]] + (w->first_sample - points[wk[2u * i]].first_sample);
+        gw[ngw].dst = dst;
+        gw[ngw].len = w->num_samples;
+        gw[ngw].item_first = (uint32_t)items;
+        items += (uint64_t)(((dst + w->num_samples + 3u) >> 2) - (dst >> 2)) * C;
+        dense += w->num_samples;
+        ngw++;
+    }
+    dense_stride = (uint32_t)LNB_ROUNDUP(dense, 4u);
+    if (items > 0xFFFFFFFFull || dense > 0xFFFFFFF0ull) { free(mark); return LINNE_APIRESULT_NG; }   /* more than 2^32 items */
+
+    if (nneed) {
+        const uint8_t *image = d_data;
+        uint32_t image_size = data_size;
+        /* ---- the needed blocks' bytes: a host image uploads only those, adjacent blocks in one piece ---- */
+        if (data) {
+            const size_t padded = LNB_ROUNDUP((size_t)img_bytes + 16u, 16u);
+            uint8_t *stage;
+            if (lnb_buf_reserve_host(&dec->h_win_img, padded) || lnb_buf_reserve_device(dec->dev, &dec->d_stream, padded)) { free(mark); return LINNE_APIRESULT_NG; }
+            stage = (uint8_t *)dec->h_win_img.ptr;
+            for (j = 0; j < nneed; ) {
+                const uint32_t src = data_size - seek[j].remain, dst = seek[j].img_off;
+                uint32_t len = seek[j].span;
+                for (j++; j < nneed && seek[j].img_off == dst + len && data_size - seek[j].remain == src + len; j++) len += seek[j].span;
+                memcpy(stage + dst, data + src, len);
+            }
+            memset(stage + img_bytes, 0, padded - img_bytes);
+            lnb_shim_h2d(dec->dev, dec->d_stream.ptr, stage, padded);
+            image = (const uint8_t *)dec->d_stream.ptr;
+            image_size = img_bytes;
+        }
+        /* ---- seek: the block table, built in parallel from the index; back to the host for routing and status ---- */
+        if (lnb_buf_reserve_device(dec->dev, &dec->d_win, win_bytes + (size_t)num_windows * sizeof(LnbGatherWin))
+            || lnb_buf_reserve_device(dec->dev, &dec->d_blocks, (size_t)nneed * sizeof(LnbBlockDesc))
+            || lnb_buf_reserve_device(dec->dev, &dec->d_params, (size_t)nneed * C * sizeof(LnbChanParams))
+            || lnb_buf_reserve_device(dec->dev, &dec->d_pcm, (size_t)stride * C * sizeof(int32_t))
+            || (!resident && ngw && lnb_buf_reserve_device(dec->dev, &dec->d_packed, (size_t)dense_stride * C * sizeof(int32_t)))
+            || (!resident && ngw && lnb_buf_reserve_host(&dec->h_win_pcm, (size_t)dense_stride * C * sizeof(int32_t)))) { free(mark); return LINNE_APIRESULT_NG; }
+        lnb_shim_h2d(dec->dev, dec->d_win.ptr, dec->h_win.ptr, win_bytes + (size_t)ngw * sizeof(LnbGatherWin));
+        if (lnb_shim_seek_blocks(dec->dev, image, (const LnbSeekIn *)dec->d_win.ptr, nneed, C, h->bits_per_sample, (LnbBlockDesc *)dec->d_blocks.ptr))
+            { free(mark); return LINNE_APIRESULT_NG; }
+        lnb_shim_d2h(dec->dev, blocks, dec->d_blocks.ptr, (size_t)nneed * sizeof(LnbBlockDesc));
+        if (lnb_shim_sync(dec->dev)) { free(mark); return LINNE_APIRESULT_NG; }
+        /* blocks whose framing failed are neither CRC-checked nor decoded: the batch holds the others */
+        {
+            int32_t depth = 0;
+            for (k = 0, j = 0; k < N; k++) {
+                depth += mark[k];
+                if (depth <= 0) continue;
+                err[k] = blocks[j].status;
+                if (blocks[j].status == LINNE_APIRESULT_OK) { blocks[nok] = blocks[j]; blocks[nok].status = 0; ok_block[nok++] = k; }
+                j++;
+            }
+        }
+        /* ---- decode of the needed blocks into the scratch planes, then the gather of every window ---- */
+        if (nok) {
+            lnb_fill_stream_cfg(&batch.cfg, h);
+            batch.cfg.pcm_stride = stride;
+            batch.cfg.work_stride = 0;
+            batch.cfg.check_crc = (dec->flags & DEC_FLAG_CHECK_CRC) ? 1u : 0u;
+            route_batch(dec, &batch, blocks, nok, (const int32_t *)dec->d_pcm.ptr);
+            batch.tab = *lnb_shim_tables(dec->dev);
+            batch.stream = image;
+            batch.stream_size = image_size;
+            batch.blocks = (LnbBlockDesc *)dec->d_blocks.ptr;
+            batch.num_blocks = nok;
+            batch.params = (LnbChanParams *)dec->d_params.ptr;
+            batch.pcm = (int32_t *)dec->d_pcm.ptr;
+            lnb_shim_h2d(dec->dev, dec->d_blocks.ptr, blocks, (size_t)nok * sizeof(LnbBlockDesc));
+            if (lnb_shim_decode(dec->dev, &batch)) { free(mark); return LINNE_APIRESULT_NG; }
+            lnb_shim_d2h(dec->dev, blocks, dec->d_blocks.ptr, (size_t)nok * sizeof(LnbBlockDesc));
+            if (lnb_shim_gather_windows(dec->dev, (const int32_t *)dec->d_pcm.ptr, stride, (const LnbGatherWin *)((uint8_t *)dec->d_win.ptr + win_bytes),
+                                        ngw, (uint32_t)items, resident ? d_pcm : (int32_t *)dec->d_packed.ptr, resident ? out_stride : dense_stride))
+                { free(mark); return LINNE_APIRESULT_NG; }
+            if (!resident && ngw)
+                for (c = 0; c < C; c++)
+                    lnb_shim_d2h(dec->dev, (int32_t *)dec->h_win_pcm.ptr + (size_t)c * dense_stride,
+                                 (const int32_t *)dec->d_packed.ptr + (size_t)c * dense_stride, (size_t)dense * sizeof(int32_t));
+            if (lnb_shim_sync(dec->dev)) { free(mark); return LINNE_APIRESULT_NG; }
+            if (dec->flags & DEC_FLAG_CHECK_CRC)
+                for (j = 0; j < nok; j++) if (blocks[j].status & LNB_ST_CRC_MISMATCH) err[ok_block[j]] = LINNE_APIRESULT_DETECT_DATA_CORRUPTION;
+        }
+    }
+
+    /* ---- statuses: the first failing block a window needs, in stream order; host buffers get their samples ---- */
+    for (k = N; k-- > 0; ) first_bad[k] = (err[k] != LINNE_APIRESULT_OK) ? k : (k + 1u < N ? first_bad[k + 1u] : N);
+    for (i = 0, j = 0; i < num_windows; i++) {
+        struct LINNEB200Window *w = &windows[i];
+        const uint32_t f = w->num_samples ? first_bad[wk[2u * i]] : N;
+        w->status = (int32_t)((w->num_samples && f <= wk[2u * i + 1u]) ? err[f] : LINNE_APIRESULT_OK);
+        if (overall == LINNE_APIRESULT_OK && w->status != (int32_t)LINNE_APIRESULT_OK) overall = (LINNEApiResult)w->status;
+        if (w->num_samples == 0u) continue;
+        if (!resident && nok && w->status == (int32_t)LINNE_APIRESULT_OK)
+            for (c = 0; c < C; c++)
+                memcpy(buffer[c] + w->out_offset, (const int32_t *)dec->h_win_pcm.ptr + (size_t)c * dense_stride + gw[j].dst,
+                       (size_t)w->num_samples * sizeof(int32_t));
+        j++;
+    }
+    free(mark);
+    return overall;
+}
+
+LINNEApiResult LINNEB200_DecodeWindows(struct LINNEDecoder *dec, const uint8_t *data, uint32_t data_size,
+        const struct LINNEB200SeekPoint *points, uint32_t num_points, struct LINNEB200Window *windows, uint32_t num_windows,
+        int32_t **buffer, uint32_t buffer_num_channels, uint32_t buffer_num_samples)
+{
+    uint32_t c;
+    if (dec == NULL || data == NULL || points == NULL || windows == NULL || buffer == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
+    if (!(dec->flags & DEC_FLAG_HEADER_SET)) return LINNE_APIRESULT_PARAMETER_NOT_SET;
+    if (buffer_num_channels < dec->header.num_channels) return LINNE_APIRESULT_INSUFFICIENT_BUFFER;
+    for (c = 0; c < dec->header.num_channels; c++) if (buffer[c] == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
+    return decode_windows(dec, data, NULL, data_size, points, num_points, windows, num_windows, buffer, NULL, buffer_num_samples);
+}
+
+LINNEApiResult LINNEB200_DecodeWindowsResident(struct LINNEDecoder *dec, const uint8_t *d_data, uint32_t data_size,
+        const struct LINNEB200SeekPoint *points, uint32_t num_points, struct LINNEB200Window *windows, uint32_t num_windows,
+        int32_t *d_pcm, uint32_t pcm_stride)
+{
+    if (dec == NULL || d_data == NULL || points == NULL || windows == NULL || d_pcm == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
+    if (!(dec->flags & DEC_FLAG_HEADER_SET)) return LINNE_APIRESULT_PARAMETER_NOT_SET;
+    return decode_windows(dec, NULL, d_data, data_size, points, num_points, windows, num_windows, NULL, d_pcm, pcm_stride);
 }

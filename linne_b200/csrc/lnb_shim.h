@@ -70,6 +70,15 @@ int lnb_shim_encode_pack(LnbDevice *dev, const LnbEncodeBatch *batch, uint32_t o
 int lnb_shim_hop(LnbDevice *dev, const uint8_t *d_image, const LnbHopFile *d_files, uint32_t num_files,
                  LnbBlockDesc *d_table, LnbHopResult *d_results);
 
+/* sample-window decodes (lnb_window.cuh), enqueue only.  seek: one item per block a window needs -- reads the block header
+ * at d_in[j].img_off of d_image, checks it against the index and fills d_out[j] (result code in .status).  gather: copies
+ * every window of d_wins from the scratch planes [C][scratch_stride] to d_dst [C][dst_stride]; `num_items` is the item
+ * count after the last window's item_first (one item per channel and aligned group of four destination samples). */
+int lnb_shim_seek_blocks(LnbDevice *dev, const uint8_t *d_image, const LnbSeekIn *d_in, uint32_t n,
+                         uint32_t channels, uint32_t bits, LnbBlockDesc *d_out);
+int lnb_shim_gather_windows(LnbDevice *dev, const int32_t *d_scratch, uint32_t scratch_stride, const LnbGatherWin *d_wins,
+                            uint32_t num_wins, uint32_t num_items, int32_t *d_dst, uint32_t dst_stride);
+
 /* packed interleaved PCM (WAV data-chunk layout, `bytes` per sample) <-> int32 planes, on the device (enqueue only) */
 int lnb_shim_unpack_pcm(LnbDevice *dev, const uint8_t *d_packed, int32_t *d_pcm, uint32_t pcm_stride,
                         uint32_t frames, uint32_t channels, uint32_t bytes);

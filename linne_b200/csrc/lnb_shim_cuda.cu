@@ -22,6 +22,7 @@
 #include "lnb_scan_v2.cuh"
 #include "lnb_stream_v2.cuh"
 #include "lnb_hop.cuh"
+#include "lnb_window.cuh"
 
 #define LNB_MAX_STAGES 32
 #define LNB_MAX_PENDING 8192
@@ -579,6 +580,23 @@ int lnb_shim_hop(LnbDevice *dev, const uint8_t *d_image, const LnbHopFile *d_fil
     const int slot = ex.begin_stage("hop");
     lnb_hop_kernel<<<num_files, 32, 0, dev->stream>>>(d_image, d_files, num_files, d_table, d_results);
     ex.end_stage(slot);
+    return dev->last_error == cudaSuccess ? 0 : 1;
+}
+
+int lnb_shim_seek_blocks(LnbDevice *dev, const uint8_t *d_image, const LnbSeekIn *d_in, uint32_t n,
+                         uint32_t channels, uint32_t bits, LnbBlockDesc *d_out)
+{
+    bind_device(dev);
+    CudaExec ex{dev};
+    lnb_seek_pipeline(ex, d_image, d_in, n, channels, bits, d_out);
+    return dev->last_error == cudaSuccess ? 0 : 1;
+}
+int lnb_shim_gather_windows(LnbDevice *dev, const int32_t *d_scratch, uint32_t scratch_stride, const LnbGatherWin *d_wins,
+                            uint32_t num_wins, uint32_t num_items, int32_t *d_dst, uint32_t dst_stride)
+{
+    bind_device(dev);
+    CudaExec ex{dev};
+    lnb_gather_windows_pipeline(ex, d_scratch, scratch_stride, d_wins, num_wins, num_items, d_dst, dst_stride);
     return dev->last_error == cudaSuccess ? 0 : 1;
 }
 

@@ -104,6 +104,20 @@ typedef struct LnbHopResult {
     uint32_t overflow;              /* 1: more blocks than table_cap -- the caller falls back to hopping on the host */
 } LnbHopResult;
 
+/* ---- sample-window decodes (lnb_window.cuh) ----
+ * LnbSeekIn: one block a window needs, found through the caller's seek index.  The block header is read at `img_off` of
+ * the batch's image; `span` bytes are there (up to the next indexed block), `remain` bytes of the stream follow the
+ * block's start (the framing checks of scan_blocks use it).  `nsmp` is the index's sample count of the block and
+ * `smp_off` its place in the scratch planes. */
+typedef struct LnbSeekIn {
+    uint32_t img_off, span, remain, nsmp, smp_off;
+} LnbSeekIn;
+/* LnbGatherWin: one window of a gather: `len` samples per channel from scratch sample `src` to destination sample `dst`;
+ * its items (one per aligned group of four destination samples and channel) start at item `item_first`. */
+typedef struct LnbGatherWin {
+    uint32_t src, dst, len, item_first;
+} LnbGatherWin;
+
 /* ---- one encode batch (all pointers are device pointers) ---- */
 typedef struct LnbEncodeBatch {
     LnbStreamCfg cfg;
