@@ -32,7 +32,7 @@ struct LINNEDecoder {
     void *work;
     LnbDevice *dev;
     LnbBuf d_stream, d_blocks, d_params, d_pcm, d_packed;
-    LnbBuf h_blocks;                       /* pinned LnbBlockDesc[] */
+    LnbBuf h_blocks;                       /* pinned LnbBlockDesc[]: the block table of every call */
     LnbBuf h_stream;                       /* pinned copy of a device-resident stream (block hop on the host: fallback only) */
     LnbBuf d_hop_files, d_hop_res, d_hop_table, h_hop;     /* device-side block hop: records, results, table; pinned staging */
     LnbBuf h_pcm;                          /* pinned int32 [C][stage_stride]: PCM staging of DecodeBlock / read-ahead cache */
@@ -55,8 +55,6 @@ struct LINNEDecoder {
     uint32_t turn_index;
     int rank_override;                     /* >= 0: the stream priority rank of a child (its place in the pipeline) instead of the preset's */
     struct LINNEDecoderConfig config;
-    LnbBlockDesc *shard_table;             /* host block table of the sharding hop */
-    uint32_t shard_table_cap;
 };
 #define LNB_MAX_READAHEAD 1024u
 #define LNB_READAHEAD_MAX_SAMPLES (1u << 21)  /* per channel and batch: bounds the pinned PCM cache (8 ch: 64 MiB) */
@@ -135,7 +133,6 @@ void LINNEDecoder_Destroy(struct LINNEDecoder *dec)
     uint32_t k;
     if (dec == NULL) return;
     for (k = 0; k < LNB_MAX_DEVICES; k++) if (dec->child[k]) { LINNEDecoder_Destroy(dec->child[k]); dec->child[k] = NULL; }
-    free(dec->shard_table); dec->shard_table = NULL; dec->shard_table_cap = 0;
     if (dec->dev) {
         lnb_buf_release_device(dec->dev, &dec->d_stream);
         lnb_buf_release_device(dec->dev, &dec->d_blocks);
@@ -182,84 +179,57 @@ LINNEApiResult LINNEDecoder_SetHeader(struct LINNEDecoder *dec, const struct LIN
     return LINNE_APIRESULT_OK;
 }
 
-/* ----------------------------------------------------------------------------------------------
- * Block table: hop over the size fields (serial by nature, a few ns per block).
- * Per block the reference checks, in this order (linne_decoder.c:604-653):
- *   sync (INVALID_FORMAT) -> size (INSUFFICIENT_DATA) -> CRC (DETECT_DATA_CORRUPTION)
- *   -> sample count vs buffer (INSUFFICIENT_BUFFER) -> type (INVALID_FORMAT, :651)
- *   -> raw payload size (INSUFFICIENT_DATA, :383)
- * Sync and size stop the hop; the later ones are recorded as the terminal block's `post_crc_error`
- * because a CRC mismatch (known only after the GPU pass) outranks them.
- * ---------------------------------------------------------------------------------------------- */
-typedef struct {
-    uint32_t num_blocks;          /* blocks entered in the table (the terminal block included if its CRC can be checked) */
-    uint32_t num_decodable;       /* blocks that can be decoded (terminal block with a post-CRC error excluded) */
-    LINNEApiResult framing_error; /* error that ends the stream after num_blocks blocks (or OK) */
-    LINNEApiResult post_crc_error;/* error of block num_decodable (only when num_blocks == num_decodable + 1) */
-    uint32_t total_samples;
-    uint32_t end_offset;
-} BlockScan;
-
-static int scan_blocks(const struct LINNEHeader *h, const uint8_t *data, uint32_t data_size,
-                       uint32_t start_offset, uint32_t max_samples, uint32_t sample_limit, uint32_t block_limit,
-                       LnbBlockDesc *table, uint32_t table_cap, BlockScan *out)
+/* Block table: the hop over the size fields (lnb_framing.h; serial by nature, a few ns per block) of data[off, data_size)
+ * into dec->h_blocks from entry `first` on, the entries before it kept (a call over several streams appends them).  The
+ * table grows until the hop fits.  Byte offsets are relative to `data`. */
+static int hop_host(struct LINNEDecoder *dec, const struct LINNEHeader *h, const uint8_t *data, uint32_t data_size, uint32_t off,
+                    uint32_t room, uint32_t sample_limit, uint32_t block_limit, uint32_t first, LnbHopResult *res)
 {
-    uint32_t off = start_offset, progress = 0, nb = 0;
-    memset(out, 0, sizeof(*out));
-    out->framing_error = LINNE_APIRESULT_OK;
-    out->post_crc_error = LINNE_APIRESULT_OK;
-    while (progress < sample_limit && off < data_size) {
-        const uint8_t *p = data + off;
-        const uint32_t remain = data_size - off;
-        uint32_t size32, type, ns, consumed;
-        LnbBlockDesc *d;
-        if (nb >= table_cap) return 1;                         /* caller grows the table and retries */
-        if (remain < 2 || lnb_rd_be(p, 2) != LNB_SYNC_CODE) {
-            out->framing_error = (remain < 2) ? LINNE_APIRESULT_INSUFFICIENT_DATA : LINNE_APIRESULT_INVALID_FORMAT;
-            break;
+    uint32_t want = block_limit ? block_limit : (uint32_t)((uint64_t)(data_size - off) / 64u + 16u);
+    if (!block_limit && h->num_samples_per_block && sample_limit / h->num_samples_per_block + 16u < want)
+        want = (sample_limit / h->num_samples_per_block + 16u) * 2u;
+    for (;;) {
+        const size_t cap = dec->h_blocks.cap / sizeof(LnbBlockDesc);
+        if (dec->h_blocks.ptr == NULL || cap < (size_t)first + want) {
+            LnbBuf grown = { NULL, 0 };
+            if (lnb_buf_reserve_host(&grown, ((size_t)first + want) * sizeof(LnbBlockDesc))) return 1;
+            if (first) memcpy(grown.ptr, dec->h_blocks.ptr, (size_t)first * sizeof(LnbBlockDesc));
+            lnb_buf_release_host(&dec->h_blocks);
+            dec->h_blocks = grown;
+            continue;
         }
-        if (remain < 6) { out->framing_error = LINNE_APIRESULT_INSUFFICIENT_DATA; break; }
-        size32 = lnb_rd_be(p + 2, 4);
-        if ((uint64_t)size32 + 6u > remain) { out->framing_error = LINNE_APIRESULT_INSUFFICIENT_DATA; break; }
-        if (size32 < 5u) { out->framing_error = LINNE_APIRESULT_INVALID_FORMAT; break; }   /* cannot hold crc+type+count */
-        type = p[8];
-        ns = lnb_rd_be(p + 9, 2);
-        d = &table[nb];
-        memset(d, 0, sizeof(*d));
-        d->smp_off = progress; d->nsmp = ns; d->byte_off = off; d->byte_size = size32 + 6u; d->type = type;
-        nb++;
-        if (ns > max_samples - progress) { out->post_crc_error = LINNE_APIRESULT_INSUFFICIENT_BUFFER; break; }
-        if (type > LNB_BLOCK_RAW) { out->post_crc_error = LINNE_APIRESULT_INVALID_FORMAT; break; }
-        if (type == LNB_BLOCK_RAW) {
-            const uint32_t need = (h->bits_per_sample * ns * h->num_channels) / 8u;
-            if (remain - LNB_BLOCK_HEADER_SIZE < need) { out->post_crc_error = LINNE_APIRESULT_INSUFFICIENT_DATA; break; }
-            consumed = LNB_BLOCK_HEADER_SIZE + (h->bits_per_sample / 8u) * ns * h->num_channels;
-        } else if (type == LNB_BLOCK_SILENT) {
-            consumed = LNB_BLOCK_HEADER_SIZE;
-        } else {
-            consumed = size32 + 6u;                            /* == 11 + ceil(bits/8) for any stream an encoder wrote */
-        }
-        out->num_decodable = nb;
-        progress += ns;
-        off += consumed;
-        if (block_limit && nb >= block_limit) break;
+        lnb_hop_blocks(data, data_size, off, h->num_channels, h->bits_per_sample, room, sample_limit, block_limit,
+                       (LnbBlockDesc *)dec->h_blocks.ptr + first, (uint32_t)(cap - first), 0u, res);
+        if (!res->overflow) return 0;
+        want = (uint32_t)(cap - first) * 2u;
     }
-    out->num_blocks = nb;
-    out->total_samples = progress;
-    out->end_offset = off;
-    return 0;
 }
 
-/* Routing of a decode batch, the same for every caller: compressed blocks go to the fused streaming kernel (unless
- * LINNE_B200_SPLIT_DECODE=1), what is left is counted for the split kernels, the longest block sizes their shared-memory
- * lines, and batches of at least tput_min_blocks blocks take the throughput kernels (eight lanes per block / one per
- * (block, channel) instead of one CTA per block, lnb_tput_v2.cuh).  batch->cfg must be filled in. */
-static void route_batch(const struct LINNEDecoder *dec, LnbDecodeBatch *batch, const LnbBlockDesc *blocks, uint32_t nb,
-                        const int32_t *pcm_base)
+/* the result of a stream whose blocks all pass their CRC check */
+static LINNEApiResult hop_status(const LnbHopResult *r)
+{
+    return (LINNEApiResult)(r->num_blocks > r->num_decodable ? r->post_crc_error : r->framing_error);
+}
+
+/* Reserves the device block table and parameters of `nb` blocks and fills `batch` for them: the handle's stream
+ * parameters and CRC setting, the tables, the pointers and the routing.  The routing is the same for every caller:
+ * compressed blocks go to the fused streaming kernel (unless LINNE_B200_SPLIT_DECODE=1), what is left is counted for the
+ * split kernels, the longest block sizes their shared-memory lines, and batches of at least tput_min_blocks blocks take
+ * the throughput kernels (eight lanes per block / one per (block, channel) instead of one CTA per block,
+ * lnb_tput_v2.cuh). */
+static int setup_batch(struct LINNEDecoder *dec, LnbDecodeBatch *batch, const LnbBlockDesc *blocks, uint32_t nb,
+                       const uint8_t *stream, uint32_t stream_size, int32_t *pcm, uint32_t pcm_stride)
 {
     const char *split = getenv("LINNE_B200_SPLIT_DECODE");
     const uint32_t min_blocks = dec->tput_min_blocks;
     uint32_t i;
+    if (lnb_buf_reserve_device(dec->dev, &dec->d_blocks, (size_t)nb * sizeof(LnbBlockDesc))
+        || lnb_buf_reserve_device(dec->dev, &dec->d_params, (size_t)nb * dec->header.num_channels * sizeof(LnbChanParams)))
+        return 1;
+    lnb_fill_stream_cfg(&batch->cfg, &dec->header);
+    batch->cfg.pcm_stride = pcm_stride;
+    batch->cfg.work_stride = 0;
+    batch->cfg.check_crc = (dec->flags & DEC_FLAG_CHECK_CRC) ? 1u : 0u;
     batch->fused_max_n = (split && *split == '1') ? 0u : lnb_shim_fused_max_n();
     batch->num_plain_blocks = 0;
     batch->max_nsmp = 0;
@@ -269,101 +239,108 @@ static void route_batch(const struct LINNEDecoder *dec, LnbDecodeBatch *batch, c
         if (blocks[i].nsmp > batch->max_nsmp) batch->max_nsmp = blocks[i].nsmp;
     }
     batch->tput = (min_blocks && nb >= min_blocks && batch->fused_max_n
-                   && ((uintptr_t)pcm_base & 15u) == 0u && (batch->cfg.pcm_stride & 3u) == 0u
+                   && ((uintptr_t)pcm & 15u) == 0u && (pcm_stride & 3u) == 0u
                    && lnb_shim_tput_supported(&batch->cfg)) ? 1u : 0u;
+    batch->tab = *lnb_shim_tables(dec->dev);
+    batch->stream = stream;
+    batch->stream_size = stream_size;
+    batch->blocks = (LnbBlockDesc *)dec->d_blocks.ptr;
+    batch->num_blocks = nb;
+    batch->params = (LnbChanParams *)dec->d_params.ptr;
+    batch->pcm = pcm;
+    return 0;
 }
 
-/* shared by DecodeBlock (block_limit >= 1, staged) and DecodeWhole (block_limit = 0) */
-/* Resident mode (d_stream_ext / d_pcm_ext non-NULL): the stream image and/or the PCM planes already
- * live on the device, so the corresponding bulk copy is skipped; `data` (host) is still needed for
- * the block hop.
- * Staged mode (`staged`): the PCM comes back into the handle's pinned planes (dec->h_pcm, stride
- * dec->stage_stride) together with the block table, behind ONE synchronisation; the caller hands samples on
- * from there.  `scan_out` (optional) receives the hop's result; the block table stays in dec->h_blocks. */
-static LINNEApiResult decode_range(struct LINNEDecoder *dec, const uint8_t *data, uint32_t data_size,
-                                   uint32_t start_offset, int32_t **buffer, uint32_t buffer_num_samples,
-                                   uint32_t sample_limit, uint32_t block_limit, int staged,
-                                   uint32_t *consumed_bytes, uint32_t *decoded_samples,
-                                   const uint8_t *d_stream_ext, int32_t *d_pcm_ext, uint32_t pcm_stride_ext,
-                                   BlockScan *scan_out, uint32_t *first_bad_out)
+/* the first block of blocks[from, to) whose CRC failed, or `to` (also when the handle does not check CRCs) */
+static uint32_t first_crc_failure(const struct LINNEDecoder *dec, const LnbBlockDesc *blocks, uint32_t from, uint32_t to)
+{
+    uint32_t i;
+    if (dec->flags & DEC_FLAG_CHECK_CRC)
+        for (i = from; i < to; i++) if (blocks[i].status & LNB_ST_CRC_MISMATCH) return i;
+    return to;
+}
+
+/* One range of a stream for decode_range(), shared by DecodeBlock (block_limit >= 1, staged) and DecodeWhole
+ * (block_limit = 0): the blocks found from data[start_offset] on (header already set), at most block_limit blocks /
+ * sample_limit samples, checked against `room` samples of output.
+ * Resident mode (d_stream / d_pcm non-NULL): the stream image and/or the PCM planes (stride pcm_stride) already live on
+ * the device, so the corresponding bulk copy is skipped; `data` (host) is still needed for the block hop.
+ * Staged mode (`staged`): the PCM comes back into the handle's pinned planes (dec->h_pcm, stride dec->stage_stride)
+ * together with the block table, behind ONE synchronisation; the caller hands samples on from there.  Otherwise the
+ * samples go to the caller's planes `buffer`. */
+typedef struct {
+    const uint8_t *data;
+    uint32_t data_size, start_offset;
+    int32_t **buffer;
+    uint32_t room, sample_limit, block_limit;
+    int staged;
+    const uint8_t *d_stream;
+    int32_t *d_pcm;
+    uint32_t pcm_stride;
+} RangeRequest;
+
+/* What decode_range() found: the hop's result (the block table stays in dec->h_blocks), the first block that failed
+ * (hop.num_blocks: none), the bytes the hop walked over and the samples handed back. */
+typedef struct {
+    LnbHopResult hop;
+    uint32_t first_bad, consumed, decoded;
+} RangeResult;
+
+static LINNEApiResult decode_range(struct LINNEDecoder *dec, const RangeRequest *rq, RangeResult *out)
 {
     const struct LINNEHeader *h = &dec->header;
     const uint32_t C = h->num_channels;
     LnbDecodeBatch batch;
-    BlockScan scan;
+    LnbHopResult scan;
     LnbBlockDesc *blocks;
-    uint32_t guess, first_bad, ok_samples, c, i, used;
+    uint32_t pcm_stride, first_bad, ok_samples, c, i, used;
     size_t padded;
     LINNEApiResult result;
 
-    /* block table in pinned host memory; grow until the hop fits */
-    guess = block_limit ? block_limit : (uint32_t)((uint64_t)(data_size - start_offset) / 64u + 16u);
-    if (!block_limit && h->num_samples_per_block) {
-        const uint32_t by_samples = sample_limit / h->num_samples_per_block + 16u;
-        if (by_samples < guess) guess = by_samples * 2u;
-    }
-    for (;;) {
-        if (lnb_buf_reserve_host(&dec->h_blocks, (size_t)guess * sizeof(LnbBlockDesc))) return LINNE_APIRESULT_NG;
-        blocks = (LnbBlockDesc *)dec->h_blocks.ptr;
-        if (scan_blocks(h, data, data_size, start_offset, buffer_num_samples, sample_limit, block_limit,
-                        blocks, guess, &scan) == 0) break;
-        guess *= 2u;
-    }
-    if (scan_out) *scan_out = scan;
-    if (first_bad_out) *first_bad_out = 0;
-
-    if (consumed_bytes) *consumed_bytes = 0;
-    if (decoded_samples) *decoded_samples = 0;
-    if (scan.num_blocks == 0) return scan.framing_error;      /* OK when there was simply nothing to do */
+    memset(out, 0, sizeof(*out));
+    if (hop_host(dec, h, rq->data, rq->data_size, rq->start_offset, rq->room, rq->sample_limit, rq->block_limit, 0u, &scan))
+        return LINNE_APIRESULT_NG;
+    out->hop = scan;
+    blocks = (LnbBlockDesc *)dec->h_blocks.ptr;
+    if (scan.num_blocks == 0) return (LINNEApiResult)scan.framing_error;    /* OK when there was simply nothing to do */
 
     /* bytes of the image the blocks of this call span: a streaming caller passes everything that is left of its
      * stream with every DecodeBlock (tools/linne_player/linne_player.c:110-121) -- only this much is uploaded */
     used = scan.end_offset;
     for (i = 0; i < scan.num_blocks; i++) {
         const uint64_t end = (uint64_t)blocks[i].byte_off + blocks[i].byte_size;
-        if (end > used) used = (end > data_size) ? data_size : (uint32_t)end;
+        if (end > used) used = (end > rq->data_size) ? rq->data_size : (uint32_t)end;
     }
-    if (!block_limit || d_stream_ext) used = data_size;
+    if (!rq->block_limit || rq->d_stream) used = rq->data_size;
 
     /* device buffers */
     padded = LNB_ROUNDUP((size_t)used + 16u, 16u);
-    lnb_fill_stream_cfg(&batch.cfg, h);
     {   /* the terminal block (post-CRC error) may not fit the PCM planes: park it inside the stride */
         uint32_t worst = scan.total_samples;
         if (scan.num_blocks > scan.num_decodable) worst += blocks[scan.num_blocks - 1].nsmp;
-        batch.cfg.pcm_stride = (uint32_t)LNB_ROUNDUP((size_t)worst + 4u, 4u);
+        pcm_stride = (uint32_t)LNB_ROUNDUP((size_t)worst + 4u, 4u);
     }
-    batch.cfg.work_stride = 0;
-    batch.cfg.check_crc = (dec->flags & DEC_FLAG_CHECK_CRC) ? 1u : 0u;
-    if (d_pcm_ext) batch.cfg.pcm_stride = pcm_stride_ext;
-    if ((!d_stream_ext && lnb_buf_reserve_device(dec->dev, &dec->d_stream, padded))
-        || lnb_buf_reserve_device(dec->dev, &dec->d_blocks, (size_t)scan.num_blocks * sizeof(LnbBlockDesc))
-        || lnb_buf_reserve_device(dec->dev, &dec->d_params, (size_t)scan.num_blocks * C * sizeof(LnbChanParams))
-        || (!d_pcm_ext && lnb_buf_reserve_device(dec->dev, &dec->d_pcm, (size_t)batch.cfg.pcm_stride * C * sizeof(int32_t)))
-        || (staged && lnb_buf_reserve_host(&dec->h_pcm, (size_t)batch.cfg.pcm_stride * C * sizeof(int32_t))))
+    if (rq->d_pcm) pcm_stride = rq->pcm_stride;
+    if ((!rq->d_stream && lnb_buf_reserve_device(dec->dev, &dec->d_stream, padded))
+        || (!rq->d_pcm && lnb_buf_reserve_device(dec->dev, &dec->d_pcm, (size_t)pcm_stride * C * sizeof(int32_t)))
+        || (rq->staged && lnb_buf_reserve_host(&dec->h_pcm, (size_t)pcm_stride * C * sizeof(int32_t))))
         return LINNE_APIRESULT_NG;
 
     /* a terminal block with a post-CRC error takes part in the CRC pass only */
     for (i = scan.num_decodable; i < scan.num_blocks; i++) blocks[i].type = 0xFFu;
-    route_batch(dec, &batch, blocks, scan.num_blocks, d_pcm_ext ? d_pcm_ext : (const int32_t *)dec->d_pcm.ptr);
-
-    batch.tab = *lnb_shim_tables(dec->dev);
-    batch.stream = d_stream_ext ? d_stream_ext : (const uint8_t *)dec->d_stream.ptr;
-    batch.stream_size = used;
-    batch.blocks = (LnbBlockDesc *)dec->d_blocks.ptr;
-    batch.num_blocks = scan.num_blocks;
-    batch.params = (LnbChanParams *)dec->d_params.ptr;
-    batch.pcm = d_pcm_ext ? d_pcm_ext : (int32_t *)dec->d_pcm.ptr;
+    if (setup_batch(dec, &batch, blocks, scan.num_blocks, rq->d_stream ? rq->d_stream : (const uint8_t *)dec->d_stream.ptr, used,
+                    rq->d_pcm ? rq->d_pcm : (int32_t *)dec->d_pcm.ptr, pcm_stride))
+        return LINNE_APIRESULT_NG;
 
     DEC_TRACE(dec, "hopped");
-    if (!d_stream_ext) {
+    if (!rq->d_stream) {
         if (dec->turn) lnb_turnstile_wait(dec->turn, 0, dec->turn_index);
         DEC_TRACE(dec, "upload turn");
         lnb_shim_memset(dec->dev, (uint8_t *)dec->d_stream.ptr + (padded - 16u), 0, 16u);
-        lnb_shim_h2d(dec->dev, dec->d_stream.ptr, data, used);
+        lnb_shim_h2d(dec->dev, dec->d_stream.ptr, rq->data, used);
     }
     lnb_shim_h2d(dec->dev, dec->d_blocks.ptr, blocks, (size_t)scan.num_blocks * sizeof(LnbBlockDesc));
-    if (dec->turn && !d_stream_ext) {                            /* the next range of this device may upload while this one computes */
+    if (dec->turn && !rq->d_stream) {                            /* the next range of this device may upload while this one computes */
         const int bad = lnb_shim_sync(dec->dev);
         lnb_turnstile_pass(dec->turn, 0, dec->turn_index);
         DEC_TRACE(dec, "uploaded");
@@ -372,42 +349,35 @@ static LINNEApiResult decode_range(struct LINNEDecoder *dec, const uint8_t *data
     if (lnb_shim_decode(dec->dev, &batch)) return LINNE_APIRESULT_NG;
     DEC_TRACE(dec, "launched");
     lnb_shim_d2h(dec->dev, blocks, dec->d_blocks.ptr, (size_t)scan.num_blocks * sizeof(LnbBlockDesc));
-    if (staged && scan.total_samples) {
+    if (rq->staged && scan.total_samples) {
         /* pinned planes: the samples travel with the block table, the verdict below decides what is handed on */
-        dec->stage_stride = batch.cfg.pcm_stride;
+        dec->stage_stride = pcm_stride;
         for (c = 0; c < C; c++)
-            lnb_shim_d2h(dec->dev, (int32_t *)dec->h_pcm.ptr + (size_t)c * batch.cfg.pcm_stride,
-                         (int32_t *)dec->d_pcm.ptr + (size_t)c * batch.cfg.pcm_stride,
-                         (size_t)scan.total_samples * sizeof(int32_t));
+            lnb_shim_d2h(dec->dev, (int32_t *)dec->h_pcm.ptr + (size_t)c * pcm_stride,
+                         (int32_t *)dec->d_pcm.ptr + (size_t)c * pcm_stride, (size_t)scan.total_samples * sizeof(int32_t));
     }
     if (lnb_shim_sync(dec->dev)) return LINNE_APIRESULT_NG;
     DEC_TRACE(dec, "kernels done");
 
     /* first block (stream order) whose CRC failed outranks everything after it */
-    first_bad = scan.num_blocks;
-    if (dec->flags & DEC_FLAG_CHECK_CRC)
-        for (i = 0; i < scan.num_blocks; i++) if (blocks[i].status & LNB_ST_CRC_MISMATCH) { first_bad = i; break; }
-
+    first_bad = first_crc_failure(dec, blocks, 0, scan.num_blocks);
     if (first_bad < scan.num_blocks) {
         result = LINNE_APIRESULT_DETECT_DATA_CORRUPTION;
         ok_samples = blocks[first_bad].smp_off;
-    } else if (scan.num_blocks > scan.num_decodable) {
-        result = scan.post_crc_error;
-        ok_samples = scan.total_samples;
-        first_bad = scan.num_decodable;
     } else {
-        result = scan.framing_error;
+        result = hop_status(&scan);
         ok_samples = scan.total_samples;
+        if (scan.num_blocks > scan.num_decodable) first_bad = scan.num_decodable;
     }
-    if (first_bad_out) *first_bad_out = first_bad;
+    out->first_bad = first_bad;
 
     /* hand back every sample the reference would have produced before stopping */
-    if (!d_pcm_ext && !staged) {
+    if (!rq->d_pcm && !rq->staged) {
         int bad;
         if (dec->turn) lnb_turnstile_wait(dec->turn, 1, dec->turn_index);
         DEC_TRACE(dec, "download turn");
         for (c = 0; c < C; c++)
-            lnb_shim_d2h(dec->dev, buffer[c], (int32_t *)dec->d_pcm.ptr + (size_t)c * batch.cfg.pcm_stride,
+            lnb_shim_d2h(dec->dev, rq->buffer[c], (int32_t *)dec->d_pcm.ptr + (size_t)c * pcm_stride,
                          (size_t)ok_samples * sizeof(int32_t));
         bad = lnb_shim_sync(dec->dev);
         if (dec->turn) lnb_turnstile_pass(dec->turn, 1, dec->turn_index);
@@ -415,8 +385,8 @@ static LINNEApiResult decode_range(struct LINNEDecoder *dec, const uint8_t *data
         if (bad) return LINNE_APIRESULT_NG;
     }
 
-    if (consumed_bytes) *consumed_bytes = scan.end_offset - start_offset;
-    if (decoded_samples) *decoded_samples = ok_samples;
+    out->consumed = scan.end_offset - rq->start_offset;
+    out->decoded = ok_samples;
     return result;
 }
 
@@ -450,16 +420,15 @@ static int serve_cached_block(struct LINNEDecoder *dec, const uint8_t *data, uin
 
 static void fill_block_cache(struct LINNEDecoder *dec, const uint8_t *data, uint32_t data_size)
 {
+    const RangeRequest rq = { .data = data, .data_size = data_size, .room = 0xFFFFFFFFu,
+                              .sample_limit = LNB_READAHEAD_MAX_SAMPLES, .block_limit = dec->readahead, .staged = 1 };
     const LnbBlockDesc *blocks;
-    BlockScan scan;
-    uint32_t first_bad = 0, i, n, span;
+    RangeResult r;
+    uint32_t i, n, span;
     dec->ra_count = dec->ra_next = 0;
-    memset(&scan, 0, sizeof(scan));
-    if (decode_range(dec, data, data_size, 0, NULL, 0xFFFFFFFFu, LNB_READAHEAD_MAX_SAMPLES, dec->readahead, 1,
-                     NULL, NULL, NULL, NULL, 0, &scan, &first_bad) == LINNE_APIRESULT_NG) return;
+    if (decode_range(dec, &rq, &r) == LINNE_APIRESULT_NG) return;
     blocks = (const LnbBlockDesc *)dec->h_blocks.ptr;
-    if (blocks == NULL) return;
-    n = (first_bad < scan.num_decodable) ? first_bad : scan.num_decodable;
+    n = (r.first_bad < r.hop.num_decodable) ? r.first_bad : r.hop.num_decodable;
     /* a block whose payload does not end where its size field says is left to the ordinary path */
     for (i = 0; i < n; i++) {
         uint32_t walked = LNB_BLOCK_HEADER_SIZE;
@@ -492,8 +461,11 @@ LINNEApiResult LINNEDecoder_DecodeBlock(struct LINNEDecoder *dec, const uint8_t 
         int32_t **buffer, uint32_t buffer_num_channels, uint32_t buffer_num_samples,
         uint32_t *decode_size, uint32_t *num_decode_samples)
 {
+    const RangeRequest rq = { .data = data, .data_size = data_size, .room = buffer_num_samples, .sample_limit = 0xFFFFFFFFu,
+                              .block_limit = 1, .staged = 1 };
+    RangeResult r;
     LINNEApiResult ret;
-    uint32_t c, ok_samples = 0, consumed = 0;
+    uint32_t c;
     if (dec == NULL || data == NULL || buffer == NULL || decode_size == NULL || num_decode_samples == NULL)
         return LINNE_APIRESULT_INVALID_ARGUMENT;
     if (!(dec->flags & DEC_FLAG_HEADER_SET)) return LINNE_APIRESULT_PARAMETER_NOT_SET;
@@ -509,17 +481,16 @@ LINNEApiResult LINNEDecoder_DecodeBlock(struct LINNEDecoder *dec, const uint8_t 
             return LINNE_APIRESULT_OK;
         dec->ra_count = dec->ra_next = 0;
     }
-    ret = decode_range(dec, data, data_size, 0, NULL, buffer_num_samples, 0xFFFFFFFFu, 1, 1,
-                       &consumed, &ok_samples, NULL, NULL, 0, NULL, NULL);
-    for (c = 0; ok_samples && c < dec->header.num_channels; c++)
-        memcpy(buffer[c], (const int32_t *)dec->h_pcm.ptr + (size_t)c * dec->stage_stride, (size_t)ok_samples * sizeof(int32_t));
+    ret = decode_range(dec, &rq, &r);
+    for (c = 0; r.decoded && c < dec->header.num_channels; c++)
+        memcpy(buffer[c], (const int32_t *)dec->h_pcm.ptr + (size_t)c * dec->stage_stride, (size_t)r.decoded * sizeof(int32_t));
     if (ret == LINNE_APIRESULT_OK) {
         /* the bytes the payload reader walked over (linne_decoder.c:655-661) */
         const LnbBlockDesc *blk = (const LnbBlockDesc *)dec->h_blocks.ptr;
-        consumed = LNB_BLOCK_HEADER_SIZE + blk[0].na;
+        r.consumed = LNB_BLOCK_HEADER_SIZE + blk[0].na;
     }
-    *decode_size = consumed;
-    *num_decode_samples = ok_samples;
+    *decode_size = r.consumed;
+    *num_decode_samples = r.decoded;
     return ret;
 }
 
@@ -558,8 +529,13 @@ static void *dec_shard_main(void *arg)
     lnb_shim_set_device(sh->ordinal);
     sh->decoded = 0;
     if (sh->packed) sh->result = decode_packed_range(sh->child, sh->data, sh->data_size, 0, sh->packed, sh->room, sh->sample_limit, sh->block_limit, &sh->decoded);
-    else sh->result = decode_range(sh->child, sh->data, sh->data_size, 0, sh->planes, sh->room, sh->sample_limit, sh->block_limit, 0,
-                                   NULL, &sh->decoded, NULL, NULL, 0, NULL, NULL);
+    else {
+        const RangeRequest rq = { .data = sh->data, .data_size = sh->data_size, .buffer = sh->planes, .room = sh->room,
+                                  .sample_limit = sh->sample_limit, .block_limit = sh->block_limit };
+        RangeResult r;
+        sh->result = decode_range(sh->child, &rq, &r);
+        sh->decoded = r.decoded;
+    }
     if (sh->child->turn) {                                       /* whatever happened: nobody waits for this range any more */
         lnb_turnstile_pass(sh->child->turn, 0, sh->child->turn_index);
         lnb_turnstile_pass(sh->child->turn, 1, sh->child->turn_index);
@@ -577,25 +553,14 @@ static int decode_whole_sharded(struct LINNEDecoder *dec, const uint8_t *data, u
     struct LnbDecShard sh[LNB_MAX_DEVICES];
     pthread_t th[LNB_MAX_DEVICES];
     LnbTurnstile turn;
-    BlockScan scan;
-    uint32_t guess, G, k, c, started = 0, ndev_used = 1;
+    LnbHopResult scan;
+    const LnbBlockDesc *table;
+    uint32_t G, k, c, started = 0, ndev_used = 1;
     int home, own;
     if (ndev <= 0) return 0;
-    guess = (uint32_t)((uint64_t)(data_size - LINNE_HEADER_SIZE) / 64u + 16u);
-    if (h->num_samples_per_block) {
-        const uint32_t by_samples = h->num_samples / h->num_samples_per_block + 16u;
-        if (by_samples < guess) guess = by_samples * 2u;
-    }
-    for (;;) {
-        if (guess > dec->shard_table_cap) {
-            LnbBlockDesc *p = (LnbBlockDesc *)realloc(dec->shard_table, (size_t)guess * sizeof(LnbBlockDesc));
-            if (!p) return 0;
-            dec->shard_table = p; dec->shard_table_cap = guess;
-        }
-        if (scan_blocks(h, data, data_size, LINNE_HEADER_SIZE, buffer_num_samples, h->num_samples, 0,
-                        dec->shard_table, dec->shard_table_cap, &scan) == 0) break;
-        guess *= 2u;
-    }
+    /* the handle's own block table: the children decode their ranges with tables of their own */
+    if (hop_host(dec, h, data, data_size, LINNE_HEADER_SIZE, buffer_num_samples, h->num_samples, 0u, 0u, &scan)) return 0;
+    table = (const LnbBlockDesc *)dec->h_blocks.ptr;
     /* ranges per requested device (pipelining), devices shared round-robin when fewer are visible than asked for */
     G = lnb_plan_ranges(scan.num_decodable, dec->num_devices > 1u ? dec->num_devices : 1u);
     ndev_used = dec->num_devices > 1u ? (dec->num_devices < (uint32_t)ndev ? dec->num_devices : (uint32_t)ndev) : 1u;
@@ -625,9 +590,9 @@ static int decode_whole_sharded(struct LINNEDecoder *dec, const uint8_t *data, u
         /* contiguous ranges of the decodable blocks; the last range runs to the end of the data and meets whatever ends
          * the stream (framing error, terminal block) exactly as the single-device path does */
         const uint32_t b0 = (uint32_t)((uint64_t)scan.num_decodable * k / G), b1 = (uint32_t)((uint64_t)scan.num_decodable * (k + 1u) / G);
-        const LnbBlockDesc *first = &dec->shard_table[b0];
+        const LnbBlockDesc *first = &table[b0];
         const int last = (k + 1u == G);
-        const uint32_t end_byte = last ? data_size : dec->shard_table[b1].byte_off;
+        const uint32_t end_byte = last ? data_size : table[b1].byte_off;
         memset(&sh[k], 0, sizeof(sh[k]));
         sh[k].child = dec->child[k];
         sh[k].data = data + first->byte_off;
@@ -636,7 +601,7 @@ static int decode_whole_sharded(struct LINNEDecoder *dec, const uint8_t *data, u
         if (packed) sh[k].packed = packed + (size_t)first->smp_off * h->num_channels * (h->bits_per_sample / 8u);
         sh[k].first_sample = first->smp_off;
         sh[k].room = buffer_num_samples - first->smp_off;
-        sh[k].sample_limit = last ? h->num_samples - first->smp_off : dec->shard_table[b1].smp_off - first->smp_off;
+        sh[k].sample_limit = last ? h->num_samples - first->smp_off : table[b1].smp_off - first->smp_off;
         sh[k].block_limit = last ? 0u : b1 - b0;
         sh[k].ordinal = dec->num_devices > 1u ? (int)(k % ndev_used) : own;
         dec->child[k]->turn = &turn; dec->child[k]->turn_index = k;
@@ -659,12 +624,19 @@ static int decode_whole_sharded(struct LINNEDecoder *dec, const uint8_t *data, u
     return 1;
 }
 
+/* several devices, or a stream long enough to pipeline its transfers against its kernels on one */
+static int worth_sharding(const struct LINNEDecoder *dec, uint32_t data_size)
+{
+    return dec->num_devices > 1u || data_size >= (32u << 20);
+}
+
 /* reference linne_decoder.c:671-730 */
 LINNEApiResult LINNEDecoder_DecodeWhole(struct LINNEDecoder *dec, const uint8_t *data, uint32_t data_size,
         int32_t **buffer, uint32_t buffer_num_channels, uint32_t buffer_num_samples)
 {
     struct LINNEHeader header;
     LINNEApiResult ret;
+    RangeResult r;
     uint32_t c;
     if (dec == NULL || data == NULL || buffer == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
     if ((ret = LINNEDecoder_DecodeHeader(data, data_size, &header)) != LINNE_APIRESULT_OK) return ret;
@@ -672,10 +644,12 @@ LINNEApiResult LINNEDecoder_DecodeWhole(struct LINNEDecoder *dec, const uint8_t 
     if (buffer_num_channels < header.num_channels || buffer_num_samples < header.num_samples)
         return LINNE_APIRESULT_INSUFFICIENT_BUFFER;
     for (c = 0; c < header.num_channels; c++) if (buffer[c] == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
-    /* several devices, or a stream long enough to pipeline its transfers against its kernels on one */
-    if ((dec->num_devices > 1u || data_size >= (32u << 20)) && decode_whole_sharded(dec, data, data_size, buffer, NULL, buffer_num_samples, &ret, NULL)) return ret;
-    return decode_range(dec, data, data_size, LINNE_HEADER_SIZE, buffer, buffer_num_samples,
-                        header.num_samples, 0, 0, NULL, NULL, NULL, NULL, 0, NULL, NULL);
+    if (worth_sharding(dec, data_size) && decode_whole_sharded(dec, data, data_size, buffer, NULL, buffer_num_samples, &ret, NULL)) return ret;
+    {
+        const RangeRequest rq = { .data = data, .data_size = data_size, .start_offset = LINNE_HEADER_SIZE, .buffer = buffer,
+                                  .room = buffer_num_samples, .sample_limit = header.num_samples };
+        return decode_range(dec, &rq, &r);
+    }
 }
 
 LnbDevice *lnb_decoder_device(const struct LINNEDecoder *dec) { return dec->dev; }
@@ -699,177 +673,154 @@ LINNEApiResult LINNEB200_DecodeWholeResident(struct LINNEDecoder *dec, const uin
 {
     struct LINNEHeader header;
     LINNEApiResult ret;
+    RangeResult r;
     if (dec == NULL || d_data == NULL || d_pcm == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
     if (data == NULL) {
         /* no host copy supplied: the hop over the size fields runs on the device (one stream of a corpus batch) */
-        struct LINNEB200FileDesc one;
+        struct LINNEB200FileDesc one = { .num_samples = buffer_num_samples, .out_size = data_size };
         if (pcm_stride < buffer_num_samples) return LINNE_APIRESULT_INSUFFICIENT_BUFFER;
-        one.first_sample = 0; one.num_samples = buffer_num_samples; one.out_offset = 0; one.out_size = data_size; one.status = 0;
-        (void)header;
         return decode_files(dec, NULL, d_data, data_size, &one, 1, d_pcm, pcm_stride, buffer_num_channels);
     }
     if ((ret = LINNEDecoder_DecodeHeader(data, data_size, &header)) != LINNE_APIRESULT_OK) return ret;
     if ((ret = LINNEDecoder_SetHeader(dec, &header)) != LINNE_APIRESULT_OK) return ret;
     if (buffer_num_channels < header.num_channels || buffer_num_samples < header.num_samples
         || pcm_stride < buffer_num_samples) return LINNE_APIRESULT_INSUFFICIENT_BUFFER;
-    return decode_range(dec, data, data_size, LINNE_HEADER_SIZE, NULL, buffer_num_samples,
-                        header.num_samples, 0, 0, NULL, NULL, d_data, d_pcm, pcm_stride, NULL, NULL);
+    {
+        const RangeRequest rq = { .data = data, .data_size = data_size, .start_offset = LINNE_HEADER_SIZE,
+                                  .room = buffer_num_samples, .sample_limit = header.num_samples,
+                                  .d_stream = d_data, .d_pcm = d_pcm, .pcm_stride = pcm_stride };
+        return decode_range(dec, &rq, &r);
+    }
+}
+
+/* The hop over the streams `files` of the device image d_data, run where the image is (lnb_hop.cuh): what comes back is
+ * a result record per stream (with its 30 header bytes) in *hr and the filled table slices, one after the other in
+ * dec->h_blocks -- not the image.  A stream of tiny blocks overflows its slice: then the image comes to the host once
+ * (dec->h_stream) for hop_host() and *hr is NULL.  Returns nonzero on a device error. */
+static int hop_device(struct LINNEDecoder *dec, const uint8_t *d_data, uint32_t data_size,
+                      const struct LINNEB200FileDesc *files, uint32_t num_files, const LnbHopResult **hr_out)
+{
+    LnbHopFile *hf;
+    LnbHopResult *hr;
+    uint32_t i, total_cap = 0, nb = 0;
+    *hr_out = NULL;
+    /* table slices: a conforming stream has one block per num_samples_per_block frames; the frames the caller gave
+     * room for bound that from above for any block size >= 256 (smaller: the hop reports the overflow) */
+    for (i = 0; i < num_files; i++) total_cap += files[i].num_samples / 256u + 64u;
+    if (lnb_buf_reserve_host(&dec->h_hop, (size_t)num_files * (sizeof(LnbHopFile) + sizeof(LnbHopResult)))
+        || lnb_buf_reserve_device(dec->dev, &dec->d_hop_files, (size_t)num_files * sizeof(LnbHopFile))
+        || lnb_buf_reserve_device(dec->dev, &dec->d_hop_res, (size_t)num_files * sizeof(LnbHopResult))
+        || lnb_buf_reserve_device(dec->dev, &dec->d_hop_table, (size_t)total_cap * sizeof(LnbBlockDesc))) return 1;
+    hf = (LnbHopFile *)dec->h_hop.ptr;
+    hr = (LnbHopResult *)(hf + num_files);
+    total_cap = 0;
+    for (i = 0; i < num_files; i++) {
+        hf[i].offset = files[i].out_offset; hf[i].size = files[i].out_size; hf[i].room_samples = files[i].num_samples;
+        hf[i].table_first = total_cap; hf[i].table_cap = files[i].num_samples / 256u + 64u;
+        total_cap += hf[i].table_cap;
+    }
+    lnb_shim_h2d(dec->dev, dec->d_hop_files.ptr, hf, (size_t)num_files * sizeof(LnbHopFile));
+    if (lnb_shim_hop(dec->dev, d_data, (const LnbHopFile *)dec->d_hop_files.ptr, num_files,
+                     (LnbBlockDesc *)dec->d_hop_table.ptr, (LnbHopResult *)dec->d_hop_res.ptr)) return 1;
+    lnb_shim_d2h(dec->dev, hr, dec->d_hop_res.ptr, (size_t)num_files * sizeof(LnbHopResult));
+    if (lnb_shim_sync(dec->dev)) return 1;
+    for (i = 0; i < num_files; i++) {
+        if (hr[i].overflow) {
+            if (lnb_buf_reserve_host(&dec->h_stream, (size_t)data_size + 16u)) return 1;
+            lnb_shim_d2h(dec->dev, dec->h_stream.ptr, d_data, data_size);
+            return lnb_shim_sync(dec->dev);
+        }
+        nb += hr[i].num_blocks;
+    }
+    /* only the slices that were filled travel */
+    if (lnb_buf_reserve_host(&dec->h_blocks, (size_t)nb * sizeof(LnbBlockDesc))) return 1;
+    for (i = 0, nb = 0; i < num_files; i++) {
+        if (hr[i].num_blocks) lnb_shim_d2h(dec->dev, (LnbBlockDesc *)dec->h_blocks.ptr + nb, (LnbBlockDesc *)dec->d_hop_table.ptr + hf[i].table_first,
+                                           (size_t)hr[i].num_blocks * sizeof(LnbBlockDesc));
+        nb += hr[i].num_blocks;
+    }
+    if (lnb_shim_sync(dec->dev)) return 1;
+    *hr_out = hr;
+    return 0;
+}
+
+/* one set of stream parameters per batch */
+static int same_stream_params(const struct LINNEHeader *h0, const struct LINNEHeader *h1)
+{
+    return h1->num_channels == h0->num_channels && h1->bits_per_sample == h0->bits_per_sample && h1->preset == h0->preset
+        && h1->num_samples_per_block == h0->num_samples_per_block && h1->ch_process_method == h0->ch_process_method
+        && h1->format_version == h0->format_version && h1->codec_version == h0->codec_version;
 }
 
 /* Several streams per call (corpus batches, SURVEY 8e): the streams sit one after the other in the device image
  * `d_data` (files[i].out_offset / out_size), all with the same stream parameters; the blocks of all of them go
- * through the kernels as ONE batch and every file's PCM lands at files[i].first_sample of the planes. */
+ * through the kernels as ONE batch and every file's PCM lands at files[i].first_sample of the planes.  Without a host
+ * copy of the image (`host_image`) the hop runs on the device. */
 static LINNEApiResult decode_files(struct LINNEDecoder *dec, const uint8_t *host_image, const uint8_t *d_data, uint32_t data_size,
         struct LINNEB200FileDesc *files, uint32_t num_files, int32_t *d_pcm, uint32_t pcm_stride, uint32_t max_channels)
 {
     struct LINNEHeader h0, h1;
     LnbDecodeBatch batch;
     LnbBlockDesc *blocks;
-    const uint8_t *img;
+    const LnbHopResult *hr = NULL;
+    const uint8_t *img = host_image;
     LINNEApiResult ret, overall = LINNE_APIRESULT_OK;
-    uint32_t i, k, nb = 0, cap, C = 0;
+    uint32_t i, k, nb = 0, slice = 0;
     uint32_t *first_block;
-    int hopped = 0;
     if (dec == NULL || d_data == NULL || files == NULL || num_files == 0 || d_pcm == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
     for (i = 0; i < num_files; i++) {
         if ((uint64_t)files[i].out_offset + files[i].out_size > data_size
             || (uint64_t)files[i].first_sample + files[i].num_samples > pcm_stride) return LINNE_APIRESULT_INVALID_ARGUMENT;
         files[i].status = (int32_t)LINNE_APIRESULT_OK;
     }
-    img = host_image;
     if (!(first_block = (uint32_t *)malloc(((size_t)num_files + 1u) * sizeof(uint32_t)))) return LINNE_APIRESULT_NG;
     if (!host_image) {
-        /* The image is in HBM only: the hop over the size fields runs there (lnb_hop.cuh).  What comes back is a result
-         * record per stream (with its 30 header bytes) and the block table -- not the image. */
-        LnbHopFile *hf;
-        LnbHopResult *hr;
-        LnbBlockDesc *ht;
-        uint32_t total_cap = 0;
-        size_t staging;
-        int fallback = 0;
-        /* table slices: a conforming stream has one block per num_samples_per_block frames; the frames the caller gave
-         * room for bound that from above for any block size >= 256 (smaller: the hop reports the overflow) */
-        for (i = 0; i < num_files; i++) total_cap += files[i].num_samples / 256u + 64u;
-        staging = (size_t)num_files * (sizeof(LnbHopFile) + sizeof(LnbHopResult)) + (size_t)total_cap * sizeof(LnbBlockDesc);
-        if (lnb_buf_reserve_host(&dec->h_hop, staging)
-            || lnb_buf_reserve_device(dec->dev, &dec->d_hop_files, (size_t)num_files * sizeof(LnbHopFile))
-            || lnb_buf_reserve_device(dec->dev, &dec->d_hop_res, (size_t)num_files * sizeof(LnbHopResult))
-            || lnb_buf_reserve_device(dec->dev, &dec->d_hop_table, (size_t)total_cap * sizeof(LnbBlockDesc))
-            || lnb_buf_reserve_host(&dec->h_blocks, (size_t)total_cap * sizeof(LnbBlockDesc))) { free(first_block); return LINNE_APIRESULT_NG; }
-        hf = (LnbHopFile *)dec->h_hop.ptr;
-        hr = (LnbHopResult *)(hf + num_files);
-        ht = (LnbBlockDesc *)(hr + num_files);
-        total_cap = 0;
-        for (i = 0; i < num_files; i++) {
-            hf[i].offset = files[i].out_offset; hf[i].size = files[i].out_size; hf[i].room_samples = files[i].num_samples;
-            hf[i].table_first = total_cap; hf[i].table_cap = files[i].num_samples / 256u + 64u;
-            total_cap += hf[i].table_cap;
-        }
-        lnb_shim_h2d(dec->dev, dec->d_hop_files.ptr, hf, (size_t)num_files * sizeof(LnbHopFile));
-        if (lnb_shim_hop(dec->dev, d_data, (const LnbHopFile *)dec->d_hop_files.ptr, num_files,
-                         (LnbBlockDesc *)dec->d_hop_table.ptr, (LnbHopResult *)dec->d_hop_res.ptr)) { free(first_block); return LINNE_APIRESULT_NG; }
-        lnb_shim_d2h(dec->dev, hr, dec->d_hop_res.ptr, (size_t)num_files * sizeof(LnbHopResult));
-        if (lnb_shim_sync(dec->dev)) { free(first_block); return LINNE_APIRESULT_NG; }
-        for (i = 0; i < num_files; i++) if (hr[i].overflow) fallback = 1;
-        if (!fallback) {
-            /* only the slices that were filled travel */
-            for (i = 0; i < num_files; i++)
-                if (hr[i].num_blocks) lnb_shim_d2h(dec->dev, ht + hf[i].table_first, (LnbBlockDesc *)dec->d_hop_table.ptr + hf[i].table_first,
-                                                   (size_t)hr[i].num_blocks * sizeof(LnbBlockDesc));
-            if (lnb_shim_sync(dec->dev)) { free(first_block); return LINNE_APIRESULT_NG; }
-            if ((ret = LINNEDecoder_DecodeHeader(hr[0].header, files[0].out_size < 32u ? files[0].out_size : 32u, &h0)) != LINNE_APIRESULT_OK
-                || (ret = LINNEDecoder_SetHeader(dec, &h0)) != LINNE_APIRESULT_OK) { free(first_block); return ret; }
-            C = h0.num_channels;
-            if (max_channels && max_channels < C) { free(first_block); return LINNE_APIRESULT_INSUFFICIENT_BUFFER; }
-            blocks = (LnbBlockDesc *)dec->h_blocks.ptr;
-            for (i = 0; i < num_files; i++) {
-                first_block[i] = nb;
-                ret = LINNEDecoder_DecodeHeader(hr[i].header, files[i].out_size < 32u ? files[i].out_size : 32u, &h1);
-                if (ret == LINNE_APIRESULT_OK
-                    && (h1.num_channels != h0.num_channels || h1.bits_per_sample != h0.bits_per_sample || h1.preset != h0.preset
-                        || h1.num_samples_per_block != h0.num_samples_per_block || h1.ch_process_method != h0.ch_process_method
-                        || h1.format_version != h0.format_version || h1.codec_version != h0.codec_version))
-                    ret = LINNE_APIRESULT_INVALID_FORMAT;                     /* one set of stream parameters per batch */
-                if (ret == LINNE_APIRESULT_OK && files[i].num_samples < h1.num_samples) ret = LINNE_APIRESULT_INSUFFICIENT_BUFFER;
-                if (ret != LINNE_APIRESULT_OK) { files[i].status = (int32_t)ret; continue; }
-                memcpy(blocks + nb, ht + hf[i].table_first, (size_t)hr[i].num_blocks * sizeof(LnbBlockDesc));
-                for (k = 0; k < hr[i].num_blocks; k++) blocks[nb + k].smp_off += files[i].first_sample;
-                for (k = hr[i].num_decodable; k < hr[i].num_blocks; k++) blocks[nb + k].type = 0xFFu;    /* CRC pass only */
-                if (hr[i].num_blocks > hr[i].num_decodable) files[i].status = (int32_t)hr[i].post_crc_error;
-                else files[i].status = (int32_t)hr[i].framing_error;
-                nb += hr[i].num_blocks;
-            }
-            hopped = 1;
-        } else {
-            /* a stream of tiny blocks: the image comes to the host once and the hop runs there */
-            if (lnb_buf_reserve_host(&dec->h_stream, (size_t)data_size + 16u)) { free(first_block); return LINNE_APIRESULT_NG; }
-            lnb_shim_d2h(dec->dev, dec->h_stream.ptr, d_data, data_size);
-            if (lnb_shim_sync(dec->dev)) { free(first_block); return LINNE_APIRESULT_NG; }
-            img = (const uint8_t *)dec->h_stream.ptr;
-        }
+        if (hop_device(dec, d_data, data_size, files, num_files, &hr)) { overall = LINNE_APIRESULT_NG; goto done; }
+        if (!hr) img = (const uint8_t *)dec->h_stream.ptr;
     }
-    if (!hopped) {
-    if ((ret = LINNEDecoder_DecodeHeader(img + files[0].out_offset, files[0].out_size, &h0)) != LINNE_APIRESULT_OK) { free(first_block); return ret; }
-    if ((ret = LINNEDecoder_SetHeader(dec, &h0)) != LINNE_APIRESULT_OK) { free(first_block); return ret; }
-    C = h0.num_channels;
-    if (max_channels && max_channels < C) { free(first_block); return LINNE_APIRESULT_INSUFFICIENT_BUFFER; }
+    if ((overall = LINNEDecoder_DecodeHeader(hr ? hr[0].header : img + files[0].out_offset, files[0].out_size, &h0)) != LINNE_APIRESULT_OK
+        || (overall = LINNEDecoder_SetHeader(dec, &h0)) != LINNE_APIRESULT_OK) goto done;
+    if (max_channels && max_channels < h0.num_channels) { overall = LINNE_APIRESULT_INSUFFICIENT_BUFFER; goto done; }
 
-    cap = 64u;
-    for (i = 0; i < num_files; i++) cap += files[i].out_size / 64u + 16u;
-    if (lnb_buf_reserve_host(&dec->h_blocks, (size_t)cap * sizeof(LnbBlockDesc))) { free(first_block); return LINNE_APIRESULT_NG; }
-    blocks = (LnbBlockDesc *)dec->h_blocks.ptr;
     for (i = 0; i < num_files; i++) {
-        BlockScan scan;
+        LnbHopResult res;
         first_block[i] = nb;
-        ret = LINNEDecoder_DecodeHeader(img + files[i].out_offset, files[i].out_size, &h1);
-        if (ret == LINNE_APIRESULT_OK
-            && (h1.num_channels != h0.num_channels || h1.bits_per_sample != h0.bits_per_sample || h1.preset != h0.preset
-                || h1.num_samples_per_block != h0.num_samples_per_block || h1.ch_process_method != h0.ch_process_method
-                || h1.format_version != h0.format_version || h1.codec_version != h0.codec_version))
-            ret = LINNE_APIRESULT_INVALID_FORMAT;                     /* one set of stream parameters per batch */
+        ret = LINNEDecoder_DecodeHeader(hr ? hr[i].header : img + files[i].out_offset, files[i].out_size, &h1);
+        if (ret == LINNE_APIRESULT_OK && !same_stream_params(&h0, &h1)) ret = LINNE_APIRESULT_INVALID_FORMAT;
         if (ret == LINNE_APIRESULT_OK && files[i].num_samples < h1.num_samples) ret = LINNE_APIRESULT_INSUFFICIENT_BUFFER;
+        if (hr) {                                   /* the device hop's slices lie back to back: a rejected stream's closes up */
+            res = hr[i];
+            slice += res.num_blocks;
+            if (ret == LINNE_APIRESULT_OK && slice - res.num_blocks != nb)
+                memmove((LnbBlockDesc *)dec->h_blocks.ptr + nb, (LnbBlockDesc *)dec->h_blocks.ptr + (slice - res.num_blocks),
+                        (size_t)res.num_blocks * sizeof(LnbBlockDesc));
+        }
         if (ret != LINNE_APIRESULT_OK) { files[i].status = (int32_t)ret; continue; }
         /* offsets relative to the image; a file's hop cannot run into its neighbour */
-        if (scan_blocks(&h1, img, files[i].out_offset + files[i].out_size, files[i].out_offset + LINNE_HEADER_SIZE,
-                        files[i].num_samples, h1.num_samples, 0, blocks + nb, cap - nb, &scan)) {
-            free(first_block);
-            return LINNE_APIRESULT_NG;                                /* the table bound above covers every legal stream */
-        }
-        for (k = 0; k < scan.num_blocks; k++) blocks[nb + k].smp_off += files[i].first_sample;
-        for (k = scan.num_decodable; k < scan.num_blocks; k++) blocks[nb + k].type = 0xFFu;    /* CRC pass only */
-        if (scan.num_blocks > scan.num_decodable) files[i].status = (int32_t)scan.post_crc_error;
-        else files[i].status = (int32_t)scan.framing_error;
-        nb += scan.num_blocks;
-    }
+        if (!hr && hop_host(dec, &h1, img, files[i].out_offset + files[i].out_size, files[i].out_offset + LINNE_HEADER_SIZE,
+                            files[i].num_samples, h1.num_samples, 0u, nb, &res)) { overall = LINNE_APIRESULT_NG; goto done; }
+        blocks = (LnbBlockDesc *)dec->h_blocks.ptr + nb;
+        for (k = 0; k < res.num_blocks; k++) blocks[k].smp_off += files[i].first_sample;
+        for (k = res.num_decodable; k < res.num_blocks; k++) blocks[k].type = 0xFFu;    /* CRC pass only */
+        files[i].status = (int32_t)hop_status(&res);
+        nb += res.num_blocks;
     }
     first_block[num_files] = nb;
 
+    blocks = (LnbBlockDesc *)dec->h_blocks.ptr;
     if (nb) {
-        lnb_fill_stream_cfg(&batch.cfg, &h0);
-        batch.cfg.pcm_stride = pcm_stride;
-        batch.cfg.work_stride = 0;
-        batch.cfg.check_crc = (dec->flags & DEC_FLAG_CHECK_CRC) ? 1u : 0u;
-        if (lnb_buf_reserve_device(dec->dev, &dec->d_blocks, (size_t)nb * sizeof(LnbBlockDesc))
-            || lnb_buf_reserve_device(dec->dev, &dec->d_params, (size_t)nb * C * sizeof(LnbChanParams))) { free(first_block); return LINNE_APIRESULT_NG; }
-        route_batch(dec, &batch, blocks, nb, d_pcm);
-        batch.tab = *lnb_shim_tables(dec->dev);
-        batch.stream = d_data;
-        batch.stream_size = data_size;
-        batch.blocks = (LnbBlockDesc *)dec->d_blocks.ptr;
-        batch.num_blocks = nb;
-        batch.params = (LnbChanParams *)dec->d_params.ptr;
-        batch.pcm = d_pcm;
+        if (setup_batch(dec, &batch, blocks, nb, d_data, data_size, d_pcm, pcm_stride)) { overall = LINNE_APIRESULT_NG; goto done; }
         lnb_shim_h2d(dec->dev, dec->d_blocks.ptr, blocks, (size_t)nb * sizeof(LnbBlockDesc));
-        if (lnb_shim_decode(dec->dev, &batch)) { free(first_block); return LINNE_APIRESULT_NG; }
+        if (lnb_shim_decode(dec->dev, &batch)) { overall = LINNE_APIRESULT_NG; goto done; }
         lnb_shim_d2h(dec->dev, blocks, dec->d_blocks.ptr, (size_t)nb * sizeof(LnbBlockDesc));
-        if (lnb_shim_sync(dec->dev)) { free(first_block); return LINNE_APIRESULT_NG; }
+        if (lnb_shim_sync(dec->dev)) { overall = LINNE_APIRESULT_NG; goto done; }
     }
     for (i = 0; i < num_files; i++) {
-        if (dec->flags & DEC_FLAG_CHECK_CRC)
-            for (k = first_block[i]; k < first_block[i + 1u]; k++)
-                if (blocks[k].status & LNB_ST_CRC_MISMATCH) { files[i].status = (int32_t)LINNE_APIRESULT_DETECT_DATA_CORRUPTION; break; }
+        if (first_crc_failure(dec, blocks, first_block[i], first_block[i + 1u]) < first_block[i + 1u])
+            files[i].status = (int32_t)LINNE_APIRESULT_DETECT_DATA_CORRUPTION;
         if (overall == LINNE_APIRESULT_OK && files[i].status != (int32_t)LINNE_APIRESULT_OK) overall = (LINNEApiResult)files[i].status;
     }
+done:
     free(first_block);
     return overall;
 }
@@ -928,8 +879,14 @@ static LINNEApiResult decode_packed_range(struct LINNEDecoder *dec, const uint8_
     if (lnb_buf_reserve_device(dec->dev, &dec->d_pcm, stride * h->num_channels * sizeof(int32_t))
         || lnb_buf_reserve_device(dec->dev, &dec->d_packed, (size_t)frames * h->num_channels * bytes + 16u))
         return LINNE_APIRESULT_NG;
-    ret = decode_range(dec, data, data_size, start_offset, NULL, room_frames, sample_limit, block_limit, 0,
-                       NULL, &decoded, NULL, (int32_t *)dec->d_pcm.ptr, (uint32_t)stride, NULL, NULL);
+    {
+        const RangeRequest rq = { .data = data, .data_size = data_size, .start_offset = start_offset, .room = room_frames,
+                                  .sample_limit = sample_limit, .block_limit = block_limit,
+                                  .d_pcm = (int32_t *)dec->d_pcm.ptr, .pcm_stride = (uint32_t)stride };
+        RangeResult r;
+        ret = decode_range(dec, &rq, &r);
+        decoded = r.decoded;
+    }
     if (decoded) {          /* every sample the reference would have produced before stopping */
         if (lnb_shim_pack_pcm(dec->dev, (const int32_t *)dec->d_pcm.ptr, (uint8_t *)dec->d_packed.ptr, (uint32_t)stride,
                               decoded, h->num_channels, bytes)) return LINNE_APIRESULT_NG;
@@ -961,9 +918,7 @@ LINNEApiResult LINNEB200_DecodeWholePacked(struct LINNEDecoder *dec, const uint8
     if (pcm_capacity_frames < header.num_samples) return LINNE_APIRESULT_INSUFFICIENT_BUFFER;
     bytes = header.bits_per_sample / 8u;
     if (bytes == 0 || bytes > 4u || (header.bits_per_sample % 8u) != 0u) return LINNE_APIRESULT_INVALID_FORMAT;
-    /* several devices, or a stream long enough to pipeline its transfers against its kernels on one */
-    if ((dec->num_devices > 1u || data_size >= (32u << 20))
-        && decode_whole_sharded(dec, data, data_size, NULL, pcm, header.num_samples, &ret, &decoded)) {
+    if (worth_sharding(dec, data_size) && decode_whole_sharded(dec, data, data_size, NULL, pcm, header.num_samples, &ret, &decoded)) {
         *num_frames = decoded;
         return ret;
     }
@@ -981,8 +936,9 @@ LINNEApiResult LINNEB200_DecoderBuildIndex(struct LINNEDecoder *dec, const uint8
 {
     struct LINNEHeader h;
     const LnbBlockDesc *table;
+    const LnbHopResult *hr = NULL;
+    LnbHopResult scan;
     LINNEApiResult ret;
-    BlockScan scan;
     uint32_t i, n;
     if (dec == NULL || num_points == NULL || (data == NULL && d_data == NULL) || (points == NULL && capacity)) return LINNE_APIRESULT_INVALID_ARGUMENT;
     *num_points = 0;
@@ -1000,54 +956,21 @@ LINNEApiResult LINNEB200_DecoderBuildIndex(struct LINNEDecoder *dec, const uint8
     }
     if ((ret = LINNEDecoder_SetHeader(dec, &h)) != LINNE_APIRESULT_OK) return ret;
 
-    memset(&scan, 0, sizeof(scan));
     if (data == NULL) {
-        /* the device hop of one stream (lnb_hop.cuh), as DecodeWholeResident without a host copy runs it */
-        LnbHopFile *hf;
-        LnbHopResult *hr;
-        const uint32_t cap = h.num_samples / 256u + 64u;
-        if (lnb_buf_reserve_host(&dec->h_hop, sizeof(LnbHopFile) + sizeof(LnbHopResult))
-            || lnb_buf_reserve_device(dec->dev, &dec->d_hop_files, sizeof(LnbHopFile))
-            || lnb_buf_reserve_device(dec->dev, &dec->d_hop_res, sizeof(LnbHopResult))
-            || lnb_buf_reserve_device(dec->dev, &dec->d_hop_table, (size_t)cap * sizeof(LnbBlockDesc))
-            || lnb_buf_reserve_host(&dec->h_blocks, (size_t)cap * sizeof(LnbBlockDesc))) return LINNE_APIRESULT_NG;
-        hf = (LnbHopFile *)dec->h_hop.ptr;
-        hr = (LnbHopResult *)(hf + 1);
-        hf->offset = 0; hf->size = data_size; hf->room_samples = h.num_samples; hf->table_first = 0; hf->table_cap = cap;
-        lnb_shim_h2d(dec->dev, dec->d_hop_files.ptr, hf, sizeof(LnbHopFile));
-        if (lnb_shim_hop(dec->dev, d_data, (const LnbHopFile *)dec->d_hop_files.ptr, 1u,
-                         (LnbBlockDesc *)dec->d_hop_table.ptr, (LnbHopResult *)dec->d_hop_res.ptr)) return LINNE_APIRESULT_NG;
-        lnb_shim_d2h(dec->dev, hr, dec->d_hop_res.ptr, sizeof(LnbHopResult));
-        if (lnb_shim_sync(dec->dev)) return LINNE_APIRESULT_NG;
-        if (!hr->overflow) {
-            lnb_shim_d2h(dec->dev, dec->h_blocks.ptr, dec->d_hop_table.ptr, (size_t)hr->num_blocks * sizeof(LnbBlockDesc));
-            if (lnb_shim_sync(dec->dev)) return LINNE_APIRESULT_NG;
-            scan.num_blocks = hr->num_blocks; scan.num_decodable = hr->num_decodable;
-            scan.framing_error = (LINNEApiResult)hr->framing_error; scan.post_crc_error = (LINNEApiResult)hr->post_crc_error;
-        } else {
-            /* a stream of tiny blocks: the image comes to the host once and the hop runs there (as in decode_files) */
-            if (lnb_buf_reserve_host(&dec->h_stream, (size_t)data_size + 16u)) return LINNE_APIRESULT_NG;
-            lnb_shim_d2h(dec->dev, dec->h_stream.ptr, d_data, data_size);
-            if (lnb_shim_sync(dec->dev)) return LINNE_APIRESULT_NG;
-            data = (const uint8_t *)dec->h_stream.ptr;
-        }
+        /* the device hop of one stream, as DecodeWholeResident without a host copy runs it */
+        const struct LINNEB200FileDesc one = { .num_samples = h.num_samples, .out_size = data_size };
+        if (hop_device(dec, d_data, data_size, &one, 1u, &hr)) return LINNE_APIRESULT_NG;
+        if (hr) scan = hr[0];
+        else data = (const uint8_t *)dec->h_stream.ptr;
     }
-    if (data != NULL) {
-        uint32_t guess = h.num_samples_per_block ? h.num_samples / h.num_samples_per_block * 2u + 32u : data_size / 64u + 16u;
-        for (;;) {
-            if (lnb_buf_reserve_host(&dec->h_blocks, (size_t)guess * sizeof(LnbBlockDesc))) return LINNE_APIRESULT_NG;
-            if (scan_blocks(&h, data, data_size, LINNE_HEADER_SIZE, h.num_samples, h.num_samples, 0,
-                            (LnbBlockDesc *)dec->h_blocks.ptr, guess, &scan) == 0) break;
-            guess *= 2u;
-        }
-    }
+    if (!hr && hop_host(dec, &h, data, data_size, LINNE_HEADER_SIZE, h.num_samples, h.num_samples, 0u, 0u, &scan)) return LINNE_APIRESULT_NG;
     /* the blocks a DecodeWhole would decode; the result is what its hop reports for the stream's framing */
     table = (const LnbBlockDesc *)dec->h_blocks.ptr;
     n = scan.num_decodable;
     for (i = 0; i < n && i < capacity; i++) { points[i].first_sample = table[i].smp_off; points[i].byte_offset = table[i].byte_off; }
     *num_points = n;
     if (n > capacity) return LINNE_APIRESULT_INSUFFICIENT_BUFFER;
-    return (scan.num_blocks > scan.num_decodable) ? scan.post_crc_error : scan.framing_error;
+    return hop_status(&scan);
 }
 
 /* index of the block that holds sample s: the last point whose first sample is <= s */
@@ -1107,7 +1030,7 @@ static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *da
     }
     win_bytes = LNB_ROUNDUP((size_t)N * sizeof(LnbSeekIn), 16u);
     if (lnb_buf_reserve_host(&dec->h_win, win_bytes + (size_t)num_windows * sizeof(LnbGatherWin))
-        || lnb_buf_reserve_host(&dec->h_blocks, (size_t)N * sizeof(LnbBlockDesc))) { free(mark); return LINNE_APIRESULT_NG; }
+        || lnb_buf_reserve_host(&dec->h_blocks, (size_t)N * sizeof(LnbBlockDesc))) { overall = LINNE_APIRESULT_NG; goto done; }
     seek = (LnbSeekIn *)dec->h_win.ptr;
     gw = (LnbGatherWin *)((uint8_t *)dec->h_win.ptr + win_bytes);
     blocks = (LnbBlockDesc *)dec->h_blocks.ptr;
@@ -1155,7 +1078,7 @@ static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *da
         ngw++;
     }
     dense_stride = (uint32_t)LNB_ROUNDUP(dense, 4u);
-    if (items > 0xFFFFFFFFull || dense > 0xFFFFFFF0ull) { free(mark); return LINNE_APIRESULT_NG; }   /* more than 2^32 items */
+    if (items > 0xFFFFFFFFull || dense > 0xFFFFFFF0ull) { overall = LINNE_APIRESULT_NG; goto done; }   /* more than 2^32 items */
 
     if (nneed) {
         const uint8_t *image = d_data;
@@ -1164,7 +1087,7 @@ static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *da
         if (data) {
             const size_t padded = LNB_ROUNDUP((size_t)img_bytes + 16u, 16u);
             uint8_t *stage;
-            if (lnb_buf_reserve_host(&dec->h_win_img, padded) || lnb_buf_reserve_device(dec->dev, &dec->d_stream, padded)) { free(mark); return LINNE_APIRESULT_NG; }
+            if (lnb_buf_reserve_host(&dec->h_win_img, padded) || lnb_buf_reserve_device(dec->dev, &dec->d_stream, padded)) { overall = LINNE_APIRESULT_NG; goto done; }
             stage = (uint8_t *)dec->h_win_img.ptr;
             for (j = 0; j < nneed; ) {
                 const uint32_t src = data_size - seek[j].remain, dst = seek[j].img_off;
@@ -1180,15 +1103,14 @@ static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *da
         /* ---- seek: the block table, built in parallel from the index; back to the host for routing and status ---- */
         if (lnb_buf_reserve_device(dec->dev, &dec->d_win, win_bytes + (size_t)num_windows * sizeof(LnbGatherWin))
             || lnb_buf_reserve_device(dec->dev, &dec->d_blocks, (size_t)nneed * sizeof(LnbBlockDesc))
-            || lnb_buf_reserve_device(dec->dev, &dec->d_params, (size_t)nneed * C * sizeof(LnbChanParams))
             || lnb_buf_reserve_device(dec->dev, &dec->d_pcm, (size_t)stride * C * sizeof(int32_t))
             || (!resident && ngw && lnb_buf_reserve_device(dec->dev, &dec->d_packed, (size_t)dense_stride * C * sizeof(int32_t)))
-            || (!resident && ngw && lnb_buf_reserve_host(&dec->h_win_pcm, (size_t)dense_stride * C * sizeof(int32_t)))) { free(mark); return LINNE_APIRESULT_NG; }
+            || (!resident && ngw && lnb_buf_reserve_host(&dec->h_win_pcm, (size_t)dense_stride * C * sizeof(int32_t)))) { overall = LINNE_APIRESULT_NG; goto done; }
         lnb_shim_h2d(dec->dev, dec->d_win.ptr, dec->h_win.ptr, win_bytes + (size_t)ngw * sizeof(LnbGatherWin));
         if (lnb_shim_seek_blocks(dec->dev, image, (const LnbSeekIn *)dec->d_win.ptr, nneed, C, h->bits_per_sample, (LnbBlockDesc *)dec->d_blocks.ptr))
-            { free(mark); return LINNE_APIRESULT_NG; }
+            { overall = LINNE_APIRESULT_NG; goto done; }
         lnb_shim_d2h(dec->dev, blocks, dec->d_blocks.ptr, (size_t)nneed * sizeof(LnbBlockDesc));
-        if (lnb_shim_sync(dec->dev)) { free(mark); return LINNE_APIRESULT_NG; }
+        if (lnb_shim_sync(dec->dev)) { overall = LINNE_APIRESULT_NG; goto done; }
         /* blocks whose framing failed are neither CRC-checked nor decoded: the batch holds the others */
         {
             int32_t depth = 0;
@@ -1202,31 +1124,19 @@ static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *da
         }
         /* ---- decode of the needed blocks into the scratch planes, then the gather of every window ---- */
         if (nok) {
-            lnb_fill_stream_cfg(&batch.cfg, h);
-            batch.cfg.pcm_stride = stride;
-            batch.cfg.work_stride = 0;
-            batch.cfg.check_crc = (dec->flags & DEC_FLAG_CHECK_CRC) ? 1u : 0u;
-            route_batch(dec, &batch, blocks, nok, (const int32_t *)dec->d_pcm.ptr);
-            batch.tab = *lnb_shim_tables(dec->dev);
-            batch.stream = image;
-            batch.stream_size = image_size;
-            batch.blocks = (LnbBlockDesc *)dec->d_blocks.ptr;
-            batch.num_blocks = nok;
-            batch.params = (LnbChanParams *)dec->d_params.ptr;
-            batch.pcm = (int32_t *)dec->d_pcm.ptr;
+            if (setup_batch(dec, &batch, blocks, nok, image, image_size, (int32_t *)dec->d_pcm.ptr, stride)) { overall = LINNE_APIRESULT_NG; goto done; }
             lnb_shim_h2d(dec->dev, dec->d_blocks.ptr, blocks, (size_t)nok * sizeof(LnbBlockDesc));
-            if (lnb_shim_decode(dec->dev, &batch)) { free(mark); return LINNE_APIRESULT_NG; }
+            if (lnb_shim_decode(dec->dev, &batch)) { overall = LINNE_APIRESULT_NG; goto done; }
             lnb_shim_d2h(dec->dev, blocks, dec->d_blocks.ptr, (size_t)nok * sizeof(LnbBlockDesc));
             if (lnb_shim_gather_windows(dec->dev, (const int32_t *)dec->d_pcm.ptr, stride, (const LnbGatherWin *)((uint8_t *)dec->d_win.ptr + win_bytes),
                                         ngw, (uint32_t)items, resident ? d_pcm : (int32_t *)dec->d_packed.ptr, resident ? out_stride : dense_stride))
-                { free(mark); return LINNE_APIRESULT_NG; }
+                { overall = LINNE_APIRESULT_NG; goto done; }
             if (!resident && ngw)
                 for (c = 0; c < C; c++)
                     lnb_shim_d2h(dec->dev, (int32_t *)dec->h_win_pcm.ptr + (size_t)c * dense_stride,
                                  (const int32_t *)dec->d_packed.ptr + (size_t)c * dense_stride, (size_t)dense * sizeof(int32_t));
-            if (lnb_shim_sync(dec->dev)) { free(mark); return LINNE_APIRESULT_NG; }
-            if (dec->flags & DEC_FLAG_CHECK_CRC)
-                for (j = 0; j < nok; j++) if (blocks[j].status & LNB_ST_CRC_MISMATCH) err[ok_block[j]] = LINNE_APIRESULT_DETECT_DATA_CORRUPTION;
+            if (lnb_shim_sync(dec->dev)) { overall = LINNE_APIRESULT_NG; goto done; }
+            for (j = 0; (j = first_crc_failure(dec, blocks, j, nok)) < nok; j++) err[ok_block[j]] = LINNE_APIRESULT_DETECT_DATA_CORRUPTION;
         }
     }
 
@@ -1244,6 +1154,7 @@ static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *da
                        (size_t)w->num_samples * sizeof(int32_t));
         j++;
     }
+done:
     free(mark);
     return overall;
 }

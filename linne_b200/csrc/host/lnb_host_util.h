@@ -6,6 +6,7 @@
 #include <stddef.h>
 #include "linne.h"
 #include "lnb_shim.h"
+#include "lnb_framing.h"
 
 #define LNB_ALIGNMENT 16
 #define LNB_MAX_DEVICES 16                 /* block ranges (devices) one handle shards a whole-stream call over */
@@ -24,8 +25,6 @@ LINNEApiResult lnb_header_check_for_encode(const struct LINNEHeader *h);
 int  lnb_header_fields_valid(const struct LINNEHeader *h);  /* decoder-side validation */
 void lnb_header_write(const struct LINNEHeader *h, uint8_t *dst);
 void lnb_header_read(const uint8_t *src, struct LINNEHeader *h);
-
-static inline uint32_t lnb_rd_be(const uint8_t *p, int n) { uint32_t v = 0; int i; for (i = 0; i < n; i++) v = (v << 8) | p[i]; return v; }
 
 void lnb_fill_stream_cfg(LnbStreamCfg *cfg, const struct LINNEHeader *h);
 

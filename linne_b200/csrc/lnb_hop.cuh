@@ -5,70 +5,22 @@
  * corpus decodes) the host used to copy the whole image back (38 MB per six-minute file) just to read those 11 bytes
  * per block.  Here one lane per file follows the chain where the image is -- a dependent load per block, served from
  * L2 when an encoder has just written the image -- and fills the block table; only the table (32 bytes per block)
- * and a result record per file travel to the host.  The checks and their order are those of scan_blocks() in
- * csrc/host/linne_decoder_host.c (reference linne_decoder.c:604-653, :383).
+ * and a result record per file travel to the host.  The checks and the loop are those of the host hop
+ * (lnb_framing.h).
  */
 #pragma once
 #include "lnb_common.cuh"
-
-/* result codes as in include/linne.h (LINNEApiResult) */
-#define LNB_HOP_OK                  0u
-#define LNB_HOP_INVALID_FORMAT      2u
-#define LNB_HOP_INSUFFICIENT_BUFFER 3u
-#define LNB_HOP_INSUFFICIENT_DATA   4u
-
-LNB_HD uint32_t lnb_hop_be(const uint8_t *p, int n) { uint32_t v = 0; for (int i = 0; i < n; i++) v = (v << 8) | p[i]; return v; }
+#include "lnb_framing.h"
 
 LNB_HD void lnb_hop_file(const uint8_t *image, const LnbHopFile &f, LnbBlockDesc *table, LnbHopResult &out)
 {
     const uint8_t *data = image + f.offset;
-    const uint32_t data_size = f.size;
-    for (uint32_t i = 0; i < 32u; i++) out.header[i] = (i < data_size && i < LNB_HEADER_SIZE) ? data[i] : (uint8_t)0;
-    out.num_blocks = out.num_decodable = out.total_samples = 0u;
-    out.framing_error = out.post_crc_error = LNB_HOP_OK;
-    out.end_offset = LNB_HEADER_SIZE;
-    out.overflow = 0u;
-    if (data_size < LNB_HEADER_SIZE || data[0] != 'I' || data[1] != 'B' || data[2] != 'R' || data[3] != 'A') return;   /* the host looks at the header */
-    const uint32_t channels = lnb_hop_be(data + 12, 2), sample_limit = lnb_hop_be(data + 14, 4), bits = lnb_hop_be(data + 22, 2);
-    const uint32_t max_samples = f.room_samples;
-    uint32_t off = LNB_HEADER_SIZE, progress = 0, nb = 0;
-    while (progress < sample_limit && off < data_size) {
-        const uint8_t *p = data + off;
-        const uint32_t remain = data_size - off;
-        if (nb >= f.table_cap) { out.overflow = 1u; break; }
-        if (remain < 2u || lnb_hop_be(p, 2) != LNB_SYNC_CODE) {
-            out.framing_error = (remain < 2u) ? LNB_HOP_INSUFFICIENT_DATA : LNB_HOP_INVALID_FORMAT;
-            break;
-        }
-        if (remain < 6u) { out.framing_error = LNB_HOP_INSUFFICIENT_DATA; break; }
-        const uint32_t size32 = lnb_hop_be(p + 2, 4);
-        if ((uint64_t)size32 + 6u > remain) { out.framing_error = LNB_HOP_INSUFFICIENT_DATA; break; }
-        if (size32 < 5u) { out.framing_error = LNB_HOP_INVALID_FORMAT; break; }
-        const uint32_t type = p[8], ns = lnb_hop_be(p + 9, 2);
-        LnbBlockDesc d;
-        d.smp_off = progress; d.nsmp = ns; d.byte_off = f.offset + off; d.byte_size = size32 + 6u; d.type = type;
-        d.na = 0; d.status = 0; d.crc = 0;
-        table[nb] = d;
-        nb++;
-        if (ns > max_samples - progress) { out.post_crc_error = LNB_HOP_INSUFFICIENT_BUFFER; break; }
-        if (type > LNB_BLOCK_RAW) { out.post_crc_error = LNB_HOP_INVALID_FORMAT; break; }
-        uint32_t consumed;
-        if (type == LNB_BLOCK_RAW) {
-            const uint32_t need = (bits * ns * channels) / 8u;
-            if (remain - LNB_BLOCK_HEADER_SIZE < need) { out.post_crc_error = LNB_HOP_INSUFFICIENT_DATA; break; }
-            consumed = LNB_BLOCK_HEADER_SIZE + (bits / 8u) * ns * channels;
-        } else if (type == LNB_BLOCK_SILENT) {
-            consumed = LNB_BLOCK_HEADER_SIZE;
-        } else {
-            consumed = size32 + 6u;
-        }
-        out.num_decodable = nb;
-        progress += ns;
-        off += consumed;
+    uint32_t channels = 0, sample_limit = 0, bits = 0;             /* no header: nothing to hop, the host looks at it */
+    for (uint32_t i = 0; i < 32u; i++) out.header[i] = (i < f.size && i < LNB_HEADER_SIZE) ? data[i] : (uint8_t)0;
+    if (f.size >= LNB_HEADER_SIZE && data[0] == 'I' && data[1] == 'B' && data[2] == 'R' && data[3] == 'A') {
+        channels = lnb_rd_be(data + 12, 2); sample_limit = lnb_rd_be(data + 14, 4); bits = lnb_rd_be(data + 22, 2);
     }
-    out.num_blocks = nb;
-    out.total_samples = progress;
-    out.end_offset = off;
+    lnb_hop_blocks(data, f.size, LNB_HEADER_SIZE, channels, bits, f.room_samples, sample_limit, 0u, table, f.table_cap, f.offset, &out);
 }
 
 #if defined(__CUDACC__)

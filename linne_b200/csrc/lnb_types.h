@@ -92,22 +92,22 @@ typedef struct LnbDecodeBatch {
                                      * checks it against the caller's buffer only, linne_decoder.c:632-635) */
 } LnbDecodeBatch;
 
-/* ---- the device-side hop over block size fields (lnb_hop.cuh): one record per stream of the image ---- */
+/* ---- the hop over block size fields (lnb_framing.h; on the device lnb_hop.cuh): one record per stream of the image ---- */
 typedef struct LnbHopFile {
     uint32_t offset, size;          /* the stream inside the image */
     uint32_t room_samples;          /* frames the destination planes hold for it */
     uint32_t table_first, table_cap;/* its slice of the block table */
 } LnbHopFile;
 typedef struct LnbHopResult {
-    uint8_t  header[32];            /* the stream's 30 header bytes (for the host's header checks) */
+    uint8_t  header[32];            /* device hop: the stream's 30 header bytes (for the host's header checks) */
     uint32_t num_blocks, num_decodable, framing_error, post_crc_error, total_samples, end_offset;
-    uint32_t overflow;              /* 1: more blocks than table_cap -- the caller falls back to hopping on the host */
+    uint32_t overflow;              /* 1: more blocks than table_cap (the host hop grows its table; a device hop falls back to it) */
 } LnbHopResult;
 
 /* ---- sample-window decodes (lnb_window.cuh) ----
  * LnbSeekIn: one block a window needs, found through the caller's seek index.  The block header is read at `img_off` of
  * the batch's image; `span` bytes are there (up to the next indexed block), `remain` bytes of the stream follow the
- * block's start (the framing checks of scan_blocks use it).  `nsmp` is the index's sample count of the block and
+ * block's start (the framing checks of lnb_framing.h use it).  `nsmp` is the index's sample count of the block and
  * `smp_off` its place in the scratch planes. */
 typedef struct LnbSeekIn {
     uint32_t img_off, span, remain, nsmp, smp_off;

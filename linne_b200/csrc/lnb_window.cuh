@@ -6,16 +6,16 @@
  * through the executor like the packed-PCM conversions:
  *
  *   seek           item = needed block: reads the 11-byte block header at the indexed offset (never past the indexed
- *                  span) and fills the batch's LnbBlockDesc.  The checks and their order are those of scan_blocks() in
- *                  csrc/host/linne_decoder_host.c / lnb_hop_file(), plus the two the index adds: the block may not run
- *                  past the next indexed block, and its sample count must be the index's.  The result code (include/
- *                  linne.h numbering) is left in LnbBlockDesc.status; the host clears it before the decode.
+ *                  span) and fills the batch's LnbBlockDesc.  The checks and their order are those of lnb_framing.h,
+ *                  plus the two the index adds: the block may not run past the next indexed block, and its sample
+ *                  count must be the index's.  The result code (include/linne.h numbering) is left in
+ *                  LnbBlockDesc.status; the host clears it before the decode.
  *   window_gather  item = (window, channel, aligned group of four destination samples): coalesced copy from the
  *                  scratch planes to the window's place, 16-byte loads and stores where both sides are aligned.
  */
 #pragma once
 #include "lnb_common.cuh"
-#include "lnb_hop.cuh"
+#include "lnb_framing.h"
 
 struct LnbItemSeek {
     const uint8_t *image;           /* the batch's stream image (the caller's device image or the staged blocks) */
@@ -31,27 +31,16 @@ struct LnbItemSeek {
         LnbBlockDesc d;
         d.smp_off = s.smp_off; d.nsmp = s.nsmp; d.byte_off = s.img_off; d.byte_size = 0; d.type = 0xFFu;
         d.na = 0; d.crc = 0;
-        uint32_t err = LNB_HOP_OK;
-        const uint32_t remain = s.remain;
-        if (remain < 2u || lnb_hop_be(h, 2) != LNB_SYNC_CODE) {
-            err = (remain < 2u) ? LNB_HOP_INSUFFICIENT_DATA : LNB_HOP_INVALID_FORMAT;
-        } else if (remain < 6u) {
-            err = LNB_HOP_INSUFFICIENT_DATA;
-        } else {
-            const uint32_t size32 = lnb_hop_be(h + 2, 4);
-            if ((uint64_t)size32 + 6u > remain) err = LNB_HOP_INSUFFICIENT_DATA;
-            else if (size32 < 5u) err = LNB_HOP_INVALID_FORMAT;
-            else {
-                const uint32_t type = h[8], ns = lnb_hop_be(h + 9, 2);
-                d.byte_size = size32 + 6u;
-                d.type = type;
-                if (d.byte_size > s.span || ns != s.nsmp || type > LNB_BLOCK_RAW) err = LNB_HOP_INVALID_FORMAT;
-                else if (type == LNB_BLOCK_RAW) {
-                    const uint64_t need = ((uint64_t)bits * ns * channels) / 8u;
-                    if ((uint64_t)remain - LNB_BLOCK_HEADER_SIZE < need) err = LNB_HOP_INSUFFICIENT_DATA;
-                    else if (LNB_BLOCK_HEADER_SIZE + (uint64_t)(bits / 8u) * ns * channels > s.span) err = LNB_HOP_INVALID_FORMAT;
-                }
-            }
+        uint32_t size32 = 0;
+        uint32_t err = lnb_block_frame(h, s.remain, &size32);
+        if (err == LNB_HOP_OK) {
+            const uint32_t type = h[8], ns = lnb_rd_be(h + 9, 2);
+            d.byte_size = size32 + 6u;
+            d.type = type;
+            if (d.byte_size > s.span || ns != s.nsmp) err = LNB_HOP_INVALID_FORMAT;       /* the index's two checks */
+            else err = lnb_block_body(type, ns, s.remain, channels, bits);
+            if (err == LNB_HOP_OK && type == LNB_BLOCK_RAW && LNB_BLOCK_HEADER_SIZE + (uint64_t)(bits / 8u) * ns * channels > s.span)
+                err = LNB_HOP_INVALID_FORMAT;                                             /* a raw payload past the span */
         }
         if (err != LNB_HOP_OK) d.type = 0xFFu;
         d.status = err;
