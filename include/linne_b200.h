@@ -128,6 +128,20 @@ LINNEApiResult LINNEB200_DecodeWindowsResident(struct LINNEDecoder *decoder, con
         const struct LINNEB200SeekPoint *points, uint32_t num_points, struct LINNEB200Window *windows, uint32_t num_windows,
         int32_t *d_pcm, uint32_t pcm_stride);
 
+/* DecodeWindowsPacked is DecodeWindows with the output of DecodeWholePacked: window w writes frames [first_sample,
+ * first_sample + num_samples) as interleaved little-endian samples (the bytes of a WAV data chunk, see the packed PCM
+ * entry points below) at byte out_offset * F of `pcm`, F = num_channels * bits_per_sample / 8.  On success these bytes
+ * equal the same frames of DecodeWholePacked's output.  The samples are converted on the device, come down as bits/8
+ * bytes per sample in one transfer and are copied with one memcpy per window.
+ *
+ * Rejected as DecodeWindows is, with the same codes (nothing written, no status set), except that the output range of a
+ * window must end at or before pcm_capacity_frames (else INVALID_ARGUMENT), and a header whose bits_per_sample is not 8,
+ * 16, 24 or 32 gives INVALID_FORMAT.  Statuses and the result as in DecodeWindows.  The bytes of a failed window, and
+ * every byte of `pcm` outside the windows, are left as they were. */
+LINNEApiResult LINNEB200_DecodeWindowsPacked(struct LINNEDecoder *decoder, const uint8_t *data, uint32_t data_size,
+        const struct LINNEB200SeekPoint *points, uint32_t num_points, struct LINNEB200Window *windows, uint32_t num_windows,
+        uint8_t *pcm, uint32_t pcm_capacity_frames);
+
 /* ---- packed PCM entry points (SURVEY 8f.2) ------------------------------------------------------------
  * `pcm` = interleaved little-endian samples exactly as in a WAV data chunk (8-bit unsigned with a bias of 128,
  * 16/24/32-bit signed; bits per sample = the encoder's parameter / the stream header).  The conversion to and

@@ -222,9 +222,9 @@ class LinneApi:
             raise RuntimeError(f"BuildIndex rc={rc}")
         return arr
 
-    def decode_windows(self, data: bytes, starts, lengths, index=None, check_crc=1, return_code=False):
-        """Samples [starts[w], starts[w] + lengths[w]) of every channel -> list of int32 [C][len] arrays
-        (LINNEB200_DecodeWindows); with return_code: (rc, arrays, per-window statuses)."""
+    def _windows(self, data: bytes, starts, lengths, index, check_crc, return_code, what, call):
+        """Shared by decode_windows and decode_windows_packed: the handle, the index (built when none is given) and the
+        windows laid out back to back.  `call(dec, hdr, pts, npts, wins, num_windows, offs)` -> (rc, results)."""
         starts, lengths = [int(s) for s in starts], [int(n) for n in lengths]
         if len(starts) != len(lengths):
             raise ValueError("starts and lengths differ in length")
@@ -233,8 +233,7 @@ class LinneApi:
             if return_code:
                 return rc, [], []
             raise RuntimeError(f"DecodeHeader rc={rc}")
-        nch = hdr.num_channels
-        dec = self._open_decoder(nch, check_crc)
+        dec = self._open_decoder(hdr.num_channels, check_crc)
         try:
             if index is None:
                 rc, index = self._build_index(dec, data)
@@ -248,21 +247,42 @@ class LinneApi:
                     raise RuntimeError(f"SetHeader rc={rc}")
             pts, npts = index_points(index)
             offs = np.concatenate([[0], np.cumsum(lengths, dtype=np.int64)]).astype(np.int64)
-            total = int(offs[-1])
-            out = np.zeros((max(nch, 1), max(total, 1)), dtype=np.int32)
             wins = (Window * max(1, len(starts)))(*[Window(s, n, int(o), 0) for s, n, o in zip(starts, lengths, offs)])
-            buf = np.frombuffer(data, dtype=np.uint8)
-            rc = self.lib.LINNEB200_DecodeWindows(dec, buf.ctypes.data_as(C.POINTER(C.c_uint8)), len(data), pts, npts,
-                                                  wins, len(starts), _chan_ptrs(out), nch, out.shape[1])
-            res = [out[:, offs[w]:offs[w + 1]] for w in range(len(starts))]
+            rc, res = call(dec, hdr, pts, npts, wins, len(starts), offs)
             status = [int(wins[w].status) for w in range(len(starts))]
             if return_code:
                 return rc, res, status
             if rc != OK:
-                raise RuntimeError(f"DecodeWindows rc={rc} (statuses {status})")
+                raise RuntimeError(f"{what} rc={rc} (statuses {status})")
             return res
         finally:
             self.lib.LINNEDecoder_Destroy(dec)
+
+    def decode_windows(self, data: bytes, starts, lengths, index=None, check_crc=1, return_code=False):
+        """Samples [starts[w], starts[w] + lengths[w]) of every channel -> list of int32 [C][len] arrays
+        (LINNEB200_DecodeWindows); with return_code: (rc, arrays, per-window statuses)."""
+        def call(dec, hdr, pts, npts, wins, nw, offs):
+            nch = hdr.num_channels
+            out = np.zeros((max(nch, 1), max(int(offs[-1]), 1)), dtype=np.int32)
+            buf = np.frombuffer(data, dtype=np.uint8)
+            rc = self.lib.LINNEB200_DecodeWindows(dec, buf.ctypes.data_as(C.POINTER(C.c_uint8)), len(data), pts, npts,
+                                                  wins, nw, _chan_ptrs(out), nch, out.shape[1])
+            return rc, [out[:, offs[w]:offs[w + 1]] for w in range(nw)]
+        return self._windows(data, starts, lengths, index, check_crc, return_code, "DecodeWindows", call)
+
+    def decode_windows_packed(self, data: bytes, starts, lengths, index=None, check_crc=1, return_code=False):
+        """Frames [starts[w], starts[w] + lengths[w]) -> list of bytes, each the window's WAV data-chunk bytes
+        (interleaved little-endian samples, LINNEB200_DecodeWindowsPacked); with return_code: (rc, list, statuses)."""
+        def call(dec, hdr, pts, npts, wins, nw, offs):
+            frame = hdr.num_channels * (hdr.bits_per_sample // 8)
+            total = int(offs[-1])
+            out = np.zeros(max(total * frame, 1), dtype=np.uint8)
+            buf = np.frombuffer(data, dtype=np.uint8)
+            u8p = C.POINTER(C.c_uint8)
+            rc = self.lib.LINNEB200_DecodeWindowsPacked(dec, buf.ctypes.data_as(u8p), len(data), pts, npts, wins, nw,
+                                                        out.ctypes.data_as(u8p), total)
+            return rc, [out[offs[w] * frame:offs[w + 1] * frame].tobytes() for w in range(nw)]
+        return self._windows(data, starts, lengths, index, check_crc, return_code, "DecodeWindowsPacked", call)
 
 
 def bind_ext_api(lib):
@@ -322,6 +342,9 @@ def bind_ext_api(lib):
     lib.LINNEB200_DecodeWindowsResident.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(SeekPoint), C.c_uint32,
                                                     C.POINTER(Window), C.c_uint32, C.c_void_p, C.c_uint32]
     lib.LINNEB200_DecodeWindowsResident.restype = C.c_int
+    lib.LINNEB200_DecodeWindowsPacked.argtypes = [C.c_void_p, u8p, C.c_uint32, C.POINTER(SeekPoint), C.c_uint32, C.POINTER(Window),
+                                                  C.c_uint32, u8p, C.c_uint32]
+    lib.LINNEB200_DecodeWindowsPacked.restype = C.c_int
     lib.LINNEB200_DecoderSetReadahead.argtypes = [C.c_void_p, C.c_uint32]
     lib.LINNEB200_DecoderSetThroughputBlocks.argtypes = [C.c_void_p, C.c_uint32]
     lib.LINNEB200_EncoderSetDevices.argtypes = [C.c_void_p, C.c_uint32]

@@ -984,15 +984,18 @@ static uint32_t find_block(const struct LINNEB200SeekPoint *points, uint32_t num
     return lo;
 }
 
-/* Shared by DecodeWindows (host image `data`, PCM into the caller's planes `buffer`) and DecodeWindowsResident (device
- * image `d_data`, PCM into the device planes `d_pcm`); `out_stride` = samples per output plane. */
+/* Shared by DecodeWindows (host image `data`, PCM into the caller's planes `buffer`), DecodeWindowsPacked (host image,
+ * packed interleaved PCM into `packed`) and DecodeWindowsResident (device image `d_data`, PCM into the device planes
+ * `d_pcm`); `out_stride` = samples per output plane, or frames of `packed`.  Host outputs are gathered densely into
+ * d_packed (planes [C][dense_stride], or packed frames), come down in one piece and are copied per window. */
 static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *data, const uint8_t *d_data, uint32_t data_size,
         const struct LINNEB200SeekPoint *points, uint32_t num_points, struct LINNEB200Window *windows, uint32_t num_windows,
-        int32_t **buffer, int32_t *d_pcm, uint32_t out_stride)
+        int32_t **buffer, int32_t *d_pcm, uint8_t *packed, uint32_t out_stride)
 {
     const struct LINNEHeader *h = &dec->header;
-    const uint32_t C = h->num_channels, N = num_points;
+    const uint32_t C = h->num_channels, N = num_points, bytes = h->bits_per_sample / 8u;
     const int resident = (d_pcm != NULL);
+    const size_t frame = packed ? (size_t)C * bytes : (size_t)C * sizeof(int32_t);   /* bytes per frame of the dense gather */
     LnbDecodeBatch batch;
     LnbSeekIn *seek;
     LnbGatherWin *gw;
@@ -1073,7 +1076,7 @@ static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *da
         gw[ngw].dst = dst;
         gw[ngw].len = w->num_samples;
         gw[ngw].item_first = (uint32_t)items;
-        items += (uint64_t)(((dst + w->num_samples + 3u) >> 2) - (dst >> 2)) * C;
+        items += (uint64_t)(((dst + w->num_samples + 3u) >> 2) - (dst >> 2)) * (packed ? 1u : C);   /* packed: one item per group */
         dense += w->num_samples;
         ngw++;
     }
@@ -1104,8 +1107,8 @@ static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *da
         if (lnb_buf_reserve_device(dec->dev, &dec->d_win, win_bytes + (size_t)num_windows * sizeof(LnbGatherWin))
             || lnb_buf_reserve_device(dec->dev, &dec->d_blocks, (size_t)nneed * sizeof(LnbBlockDesc))
             || lnb_buf_reserve_device(dec->dev, &dec->d_pcm, (size_t)stride * C * sizeof(int32_t))
-            || (!resident && ngw && lnb_buf_reserve_device(dec->dev, &dec->d_packed, (size_t)dense_stride * C * sizeof(int32_t)))
-            || (!resident && ngw && lnb_buf_reserve_host(&dec->h_win_pcm, (size_t)dense_stride * C * sizeof(int32_t)))) { overall = LINNE_APIRESULT_NG; goto done; }
+            || (!resident && ngw && lnb_buf_reserve_device(dec->dev, &dec->d_packed, (size_t)dense_stride * frame))
+            || (!resident && ngw && lnb_buf_reserve_host(&dec->h_win_pcm, (size_t)dense_stride * frame))) { overall = LINNE_APIRESULT_NG; goto done; }
         lnb_shim_h2d(dec->dev, dec->d_win.ptr, dec->h_win.ptr, win_bytes + (size_t)ngw * sizeof(LnbGatherWin));
         if (lnb_shim_seek_blocks(dec->dev, image, (const LnbSeekIn *)dec->d_win.ptr, nneed, C, h->bits_per_sample, (LnbBlockDesc *)dec->d_blocks.ptr))
             { overall = LINNE_APIRESULT_NG; goto done; }
@@ -1128,10 +1131,15 @@ static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *da
             lnb_shim_h2d(dec->dev, dec->d_blocks.ptr, blocks, (size_t)nok * sizeof(LnbBlockDesc));
             if (lnb_shim_decode(dec->dev, &batch)) { overall = LINNE_APIRESULT_NG; goto done; }
             lnb_shim_d2h(dec->dev, blocks, dec->d_blocks.ptr, (size_t)nok * sizeof(LnbBlockDesc));
-            if (lnb_shim_gather_windows(dec->dev, (const int32_t *)dec->d_pcm.ptr, stride, (const LnbGatherWin *)((uint8_t *)dec->d_win.ptr + win_bytes),
-                                        ngw, (uint32_t)items, resident ? d_pcm : (int32_t *)dec->d_packed.ptr, resident ? out_stride : dense_stride))
+            const LnbGatherWin *d_gw = (const LnbGatherWin *)((uint8_t *)dec->d_win.ptr + win_bytes);
+            if (packed ? lnb_shim_gather_windows_packed(dec->dev, (const int32_t *)dec->d_pcm.ptr, stride, d_gw, ngw, (uint32_t)items,
+                                                        (uint8_t *)dec->d_packed.ptr, C, bytes)
+                       : lnb_shim_gather_windows(dec->dev, (const int32_t *)dec->d_pcm.ptr, stride, d_gw, ngw, (uint32_t)items,
+                                                 resident ? d_pcm : (int32_t *)dec->d_packed.ptr, resident ? out_stride : dense_stride))
                 { overall = LINNE_APIRESULT_NG; goto done; }
-            if (!resident && ngw)
+            if (packed && ngw)
+                lnb_shim_d2h(dec->dev, dec->h_win_pcm.ptr, dec->d_packed.ptr, (size_t)dense * frame);
+            else if (!resident && ngw)
                 for (c = 0; c < C; c++)
                     lnb_shim_d2h(dec->dev, (int32_t *)dec->h_win_pcm.ptr + (size_t)c * dense_stride,
                                  (const int32_t *)dec->d_packed.ptr + (size_t)c * dense_stride, (size_t)dense * sizeof(int32_t));
@@ -1148,7 +1156,10 @@ static LINNEApiResult decode_windows(struct LINNEDecoder *dec, const uint8_t *da
         w->status = (int32_t)((w->num_samples && f <= wk[2u * i + 1u]) ? err[f] : LINNE_APIRESULT_OK);
         if (overall == LINNE_APIRESULT_OK && w->status != (int32_t)LINNE_APIRESULT_OK) overall = (LINNEApiResult)w->status;
         if (w->num_samples == 0u) continue;
-        if (!resident && nok && w->status == (int32_t)LINNE_APIRESULT_OK)
+        if (packed && nok && w->status == (int32_t)LINNE_APIRESULT_OK)
+            memcpy(packed + (size_t)w->out_offset * frame, (const uint8_t *)dec->h_win_pcm.ptr + (size_t)gw[j].dst * frame,
+                   (size_t)w->num_samples * frame);
+        else if (!resident && nok && w->status == (int32_t)LINNE_APIRESULT_OK)
             for (c = 0; c < C; c++)
                 memcpy(buffer[c] + w->out_offset, (const int32_t *)dec->h_win_pcm.ptr + (size_t)c * dense_stride + gw[j].dst,
                        (size_t)w->num_samples * sizeof(int32_t));
@@ -1168,7 +1179,19 @@ LINNEApiResult LINNEB200_DecodeWindows(struct LINNEDecoder *dec, const uint8_t *
     if (!(dec->flags & DEC_FLAG_HEADER_SET)) return LINNE_APIRESULT_PARAMETER_NOT_SET;
     if (buffer_num_channels < dec->header.num_channels) return LINNE_APIRESULT_INSUFFICIENT_BUFFER;
     for (c = 0; c < dec->header.num_channels; c++) if (buffer[c] == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
-    return decode_windows(dec, data, NULL, data_size, points, num_points, windows, num_windows, buffer, NULL, buffer_num_samples);
+    return decode_windows(dec, data, NULL, data_size, points, num_points, windows, num_windows, buffer, NULL, NULL, buffer_num_samples);
+}
+
+LINNEApiResult LINNEB200_DecodeWindowsPacked(struct LINNEDecoder *dec, const uint8_t *data, uint32_t data_size,
+        const struct LINNEB200SeekPoint *points, uint32_t num_points, struct LINNEB200Window *windows, uint32_t num_windows,
+        uint8_t *pcm, uint32_t pcm_capacity_frames)
+{
+    uint32_t bits;
+    if (dec == NULL || data == NULL || points == NULL || windows == NULL || pcm == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
+    if (!(dec->flags & DEC_FLAG_HEADER_SET)) return LINNE_APIRESULT_PARAMETER_NOT_SET;
+    bits = dec->header.bits_per_sample;
+    if (bits != 8u && bits != 16u && bits != 24u && bits != 32u) return LINNE_APIRESULT_INVALID_FORMAT;
+    return decode_windows(dec, data, NULL, data_size, points, num_points, windows, num_windows, NULL, NULL, pcm, pcm_capacity_frames);
 }
 
 LINNEApiResult LINNEB200_DecodeWindowsResident(struct LINNEDecoder *dec, const uint8_t *d_data, uint32_t data_size,
@@ -1177,5 +1200,5 @@ LINNEApiResult LINNEB200_DecodeWindowsResident(struct LINNEDecoder *dec, const u
 {
     if (dec == NULL || d_data == NULL || points == NULL || windows == NULL || d_pcm == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
     if (!(dec->flags & DEC_FLAG_HEADER_SET)) return LINNE_APIRESULT_PARAMETER_NOT_SET;
-    return decode_windows(dec, NULL, d_data, data_size, points, num_points, windows, num_windows, NULL, d_pcm, pcm_stride);
+    return decode_windows(dec, NULL, d_data, data_size, points, num_points, windows, num_windows, NULL, d_pcm, NULL, pcm_stride);
 }

@@ -23,6 +23,13 @@
 LNB_HD uint32_t lnb_zz_enc(int32_t s) { return ((uint32_t)s << 1) ^ (uint32_t)(s >> 31); }
 LNB_HD int32_t lnb_zz_dec(uint32_t u) { return (int32_t)(u >> 1) ^ -(int32_t)(u & 1u); }
 
+/* A sample as the `bytes` (1..4) bytes of a WAV data chunk, little-endian in the low bytes of the result: 8-bit is
+ * unsigned with a bias of 128, 16/24/32-bit two's complement (reference libs/wav/src/wav.c:665-700). */
+LNB_HD uint32_t lnb_wav_sample(int32_t v, uint32_t bytes)
+{
+    return bytes == 1u ? (uint32_t)(v + 128) & 0xFFu : (uint32_t)v & (0xFFFFFFFFu >> (32u - 8u * bytes));
+}
+
 LNB_HD uint32_t lnb_clz32(uint32_t x)
 {
 #if defined(__CUDA_ARCH__)

@@ -151,9 +151,8 @@ struct LnbItemPackPcm {
     {
         uint8_t *p = packed + (size_t)i * channels * bytes;
         for (uint32_t c = 0; c < channels; c++, p += bytes) {
-            const int32_t v = pcm[(size_t)c * stride + i];
-            if (bytes == 1u) p[0] = (uint8_t)((v + 128) & 0xFF);
-            else for (uint32_t k = 0; k < bytes; k++) p[k] = (uint8_t)((uint32_t)v >> (8u * k));
+            const uint32_t u = lnb_wav_sample(pcm[(size_t)c * stride + i], bytes);
+            for (uint32_t k = 0; k < bytes; k++) p[k] = (uint8_t)(u >> (8u * k));
         }
     }
 };

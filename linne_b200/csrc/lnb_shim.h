@@ -78,6 +78,11 @@ int lnb_shim_seek_blocks(LnbDevice *dev, const uint8_t *d_image, const LnbSeekIn
                          uint32_t channels, uint32_t bits, LnbBlockDesc *d_out);
 int lnb_shim_gather_windows(LnbDevice *dev, const int32_t *d_scratch, uint32_t scratch_stride, const LnbGatherWin *d_wins,
                             uint32_t num_wins, uint32_t num_items, int32_t *d_dst, uint32_t dst_stride);
+/* the same windows as packed interleaved PCM (WAV data-chunk layout, `bytes` per sample) into the dense staging buffer
+ * d_dst: window w at byte d_wins[w].dst * channels * bytes, every dst a multiple of 4; one item per aligned group of
+ * four frames; d_dst has room for every window rounded up to whole groups. */
+int lnb_shim_gather_windows_packed(LnbDevice *dev, const int32_t *d_scratch, uint32_t scratch_stride, const LnbGatherWin *d_wins,
+                                   uint32_t num_wins, uint32_t num_items, uint8_t *d_dst, uint32_t channels, uint32_t bytes);
 
 /* packed interleaved PCM (WAV data-chunk layout, `bytes` per sample) <-> int32 planes, on the device (enqueue only) */
 int lnb_shim_unpack_pcm(LnbDevice *dev, const uint8_t *d_packed, int32_t *d_pcm, uint32_t pcm_stride,

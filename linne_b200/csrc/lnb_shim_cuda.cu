@@ -599,6 +599,14 @@ int lnb_shim_gather_windows(LnbDevice *dev, const int32_t *d_scratch, uint32_t s
     lnb_gather_windows_pipeline(ex, d_scratch, scratch_stride, d_wins, num_wins, num_items, d_dst, dst_stride);
     return dev->last_error == cudaSuccess ? 0 : 1;
 }
+int lnb_shim_gather_windows_packed(LnbDevice *dev, const int32_t *d_scratch, uint32_t scratch_stride, const LnbGatherWin *d_wins,
+                                   uint32_t num_wins, uint32_t num_items, uint8_t *d_dst, uint32_t channels, uint32_t bytes)
+{
+    bind_device(dev);
+    CudaExec ex{dev};
+    lnb_gather_windows_packed_pipeline(ex, d_scratch, scratch_stride, d_wins, num_wins, num_items, d_dst, channels, bytes);
+    return dev->last_error == cudaSuccess ? 0 : 1;
+}
 
 int lnb_shim_unpack_pcm(LnbDevice *dev, const uint8_t *d_packed, int32_t *d_pcm, uint32_t pcm_stride,
                         uint32_t frames, uint32_t channels, uint32_t bytes)

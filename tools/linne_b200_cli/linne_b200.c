@@ -16,9 +16,14 @@
  * (linne_codec.c:100-105) and written back the same way (:262-268).
  *
  *   linne_b200 -e [-m 0..7] [-l] [-a N] in.wav out.lnn [in2.wav out2.lnn ...]
- *   linne_b200 -d [-c]                  in.lnn out.wav [in2.lnn out2.wav ...]
+ *   linne_b200 -d [-c] [--start FRAME] [--length FRAMES]  in.lnn out.wav [in2.lnn out2.wav ...]
  *   linne_b200 -e|-d ... -L pairs.txt   (one "input output" pair per line)
  *   -j N  workers (default: min(4, files))      -s  print a timing summary (samples, seconds, MSamples/s)
+ *
+ * --start / --length cut the same excerpt of every stream of a -d run: frames [FRAME, FRAME + FRAMES), to the end of the
+ * stream when --length is not given.  Each file is indexed (LINNEB200_DecoderBuildIndex) and only the blocks the excerpt
+ * overlaps are decoded, in one LINNEB200_DecodeWindowsPacked call straight into the WAV staging buffer.  An excerpt that
+ * does not lie inside a stream fails that file, and nothing is written for it.
  */
 #define _POSIX_C_SOURCE 200809L
 #include <linne_encoder.h>
@@ -59,6 +64,8 @@ struct Worker {
     struct LINNEEncoder *enc;
     struct LINNEDecoder *dec;
     struct Staging in, out;
+    struct LINNEB200SeekPoint *points;         /* seek index of the current stream (excerpts), grow-only */
+    uint32_t points_cap;
     uint64_t samples;                          /* samples (frames x channels) that went through */
     int failures;
 };
@@ -130,7 +137,12 @@ static int wav_write(const char *path, uint8_t *buf, const struct Wav *w)
     return rc;
 }
 
-struct Options { int encode, decode, preset, learning, af, no_crc, jobs, stats; const char *list; };
+struct Options {
+    int encode, decode, preset, learning, af, no_crc, jobs, stats;
+    int excerpt, has_length;                   /* --start and/or --length given; --length given */
+    uint32_t start, length;
+    const char *list;
+};
 
 static pthread_mutex_t g_print = PTHREAD_MUTEX_INITIALIZER;
 #define SAY(stream, ...) do { pthread_mutex_lock(&g_print); fprintf(stream, __VA_ARGS__); pthread_mutex_unlock(&g_print); } while (0)
@@ -169,7 +181,31 @@ static int encode_one(struct Worker *wk, const struct Options *o, const char *in
     return 0;
 }
 
-static int decode_one(struct Worker *wk, const char *in, const char *out)
+/* the excerpt of a -d run: index the stream, then decode the frames [o->start, o->start + w->frames) as one window */
+static int decode_excerpt(struct Worker *wk, const struct Options *o, const char *in, const uint8_t *buf, uint32_t size,
+                          uint8_t *wav, const struct Wav *w)
+{
+    struct LINNEB200Window win;
+    LINNEApiResult ret;
+    uint32_t n = 0;
+    while ((ret = LINNEB200_DecoderBuildIndex(wk->dec, buf, NULL, size, wk->points, wk->points_cap, &n)) == LINNE_APIRESULT_INSUFFICIENT_BUFFER
+           && n > wk->points_cap) {
+        struct LINNEB200SeekPoint *p = (struct LINNEB200SeekPoint *)realloc(wk->points, (size_t)n * sizeof(*p));
+        if (!p) { SAY(stderr, "linne_b200: %s: out of memory for the seek index\n", in); return 1; }
+        wk->points = p;
+        wk->points_cap = n;
+    }
+    if (ret != LINNE_APIRESULT_OK) { SAY(stderr, "linne_b200: %s: cannot index the stream (%d)\n", in, (int)ret); return 1; }
+    win.first_sample = o->start; win.num_samples = w->frames; win.out_offset = 0; win.status = (int32_t)LINNE_APIRESULT_OK;
+    ret = LINNEB200_DecodeWindowsPacked(wk->dec, buf, size, wk->points, n, &win, 1u, wav + 44, w->frames);
+    if (ret != LINNE_APIRESULT_OK || win.status != (int32_t)LINNE_APIRESULT_OK) {
+        SAY(stderr, "linne_b200: %s: decode failed (%d)\n", in, ret != LINNE_APIRESULT_OK ? (int)ret : (int)win.status);
+        return 1;
+    }
+    return 0;
+}
+
+static int decode_one(struct Worker *wk, const struct Options *o, const char *in, const char *out)
 {
     size_t size = 0;
     uint8_t *buf = read_file(in, &wk->in, &size), *wav;
@@ -185,9 +221,22 @@ static int decode_one(struct Worker *wk, const char *in, const char *out)
     memset(&w, 0, sizeof(w));
     w.channels = h.num_channels; w.rate = h.sampling_rate; w.bits = h.bits_per_sample; w.frames = h.num_samples;
     if (w.channels == 0 || w.channels > LINNE_MAX_NUM_CHANNELS || (w.bits != 8 && w.bits != 16 && w.bits != 24)) return 1;
+    if (o->excerpt) {
+        if (o->start > h.num_samples || (o->has_length && o->length > h.num_samples - o->start)) {
+            SAY(stderr, "linne_b200: %s: excerpt [%u, +%u) outside the stream's %u frames\n", in, o->start,
+                o->has_length ? o->length : 0u, h.num_samples);
+            return 1;
+        }
+        w.frames = o->has_length ? o->length : h.num_samples - o->start;
+    }
     if (!(wav = staging_reserve(&wk->out, 44u + (size_t)w.frames * w.channels * (w.bits / 8u) + 16u))) return 1;
-    ret = LINNEB200_DecodeWholePacked(wk->dec, buf, (uint32_t)size, wav + 44, w.frames, &frames);
-    if (ret != LINNE_APIRESULT_OK) { SAY(stderr, "linne_b200: %s: decode failed (%d)\n", in, (int)ret); return 1; }
+    if (o->excerpt) {
+        if (decode_excerpt(wk, o, in, buf, (uint32_t)size, wav, &w)) return 1;
+        frames = w.frames;
+    } else if ((ret = LINNEB200_DecodeWholePacked(wk->dec, buf, (uint32_t)size, wav + 44, w.frames, &frames)) != LINNE_APIRESULT_OK) {
+        SAY(stderr, "linne_b200: %s: decode failed (%d)\n", in, (int)ret);
+        return 1;
+    }
     /* a stream that ends on a block boundary before num_samples decodes OK with fewer frames (as in the reference,
      * whose tool writes zeros there): the staging buffer is reused between files, so clear what was not written */
     if (frames < w.frames) {
@@ -221,9 +270,22 @@ static void *worker_main(void *p)
         pthread_mutex_unlock(&q->lock);
         if (i >= q->nfiles) break;
         a->wk.failures += q->opt->encode ? encode_one(&a->wk, q->opt, q->files[i], q->files[i + 1])
-                                         : decode_one(&a->wk, q->files[i], q->files[i + 1]);
+                                         : decode_one(&a->wk, q->opt, q->files[i], q->files[i + 1]);
     }
     return NULL;
+}
+
+/* a frame count: decimal digits only, below 2^32 */
+static int parse_frames(const char *a, uint32_t *v)
+{
+    unsigned long long x = 0;
+    if (!*a) return 1;
+    for (; *a; a++) {
+        if (*a < '0' || *a > '9') return 1;
+        if ((x = x * 10u + (unsigned)(*a - '0')) > 0xFFFFFFFFull) return 1;
+    }
+    *v = (uint32_t)x;
+    return 0;
 }
 
 static double now_s(void) { struct timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return (double)ts.tv_sec + 1e-9 * (double)ts.tv_nsec; }
@@ -232,12 +294,14 @@ static void usage(const char *argv0)
 {
     fprintf(stderr,
         "usage: %s -e [-m 0..7] [-l] [-a N] in.wav out.lnn [in2.wav out2.lnn ...]\n"
-        "       %s -d [-c] in.lnn out.wav [in2.lnn out2.wav ...]\n"
+        "       %s -d [-c] [--start FRAME] [--length FRAMES] in.lnn out.wav [in2.lnn out2.wav ...]\n"
         "       -L FILE reads \"input output\" pairs from FILE (one per line)\n"
         "       -j N    pipeline workers (handles) working on different files at the same time (default min(4, files))\n"
         "       -s      print a timing summary\n"
         "  -e encode  -d decode  -m compress mode (default 0)  -l learning  -a auxiliary-function iterations\n"
-        "  -c do NOT check CRC16 when decoding\n", argv0, argv0);
+        "  -c do NOT check CRC16 when decoding\n"
+        "  --start FRAME, --length FRAMES  decode only frames [FRAME, FRAME + FRAMES) of every stream (-d only;\n"
+        "                                  default start 0, length to the end of the stream)\n", argv0, argv0);
 }
 
 int main(int argc, char **argv)
@@ -262,6 +326,14 @@ int main(int argc, char **argv)
         else if (!strcmp(a, "-L") && i + 1 < argc) o.list = argv[++i];
         else if ((!strcmp(a, "-j") || !strcmp(a, "--jobs")) && i + 1 < argc) o.jobs = atoi(argv[++i]);
         else if (!strcmp(a, "-s") || !strcmp(a, "--stats")) o.stats = 1;
+        else if (!strcmp(a, "--start") || !strcmp(a, "--length")) {
+            const int is_len = (a[2] == 'l');
+            if (i + 1 >= argc || parse_frames(argv[++i], is_len ? &o.length : &o.start)) {
+                fprintf(stderr, "%s: %s needs a frame count\n", argv[0], a); usage(argv[0]); return 1;
+            }
+            o.excerpt = 1;
+            if (is_len) o.has_length = 1;
+        }
         else if (!strcmp(a, "-h") || !strcmp(a, "--help")) { usage(argv[0]); return 0; }
         else if (a[0] == '-' && a[1] != '\0') { fprintf(stderr, "%s: unknown option %s\n", argv[0], a); usage(argv[0]); return 1; }
         else if (nfiles < 4096) files[nfiles++] = a;
@@ -277,6 +349,7 @@ int main(int argc, char **argv)
         fclose(fp);
     }
     if (o.encode == o.decode) { fprintf(stderr, "%s: exactly one of -e and -d must be given\n", argv[0]); usage(argv[0]); return 1; }
+    if (o.excerpt && o.encode) { fprintf(stderr, "%s: --start and --length apply to -d only\n", argv[0]); usage(argv[0]); return 1; }
     if (nfiles < 2 || (nfiles & 1)) { fprintf(stderr, "%s: input and output files must come in pairs\n", argv[0]); return 1; }
     if (o.preset < 0 || o.preset >= LINNE_NUM_PARAMETER_PRESETS || o.af < 0 || o.af >= 255) { fprintf(stderr, "%s: option out of range\n", argv[0]); return 1; }
 
@@ -323,6 +396,7 @@ int main(int argc, char **argv)
         if (workers[i].wk.dec) LINNEDecoder_Destroy(workers[i].wk.dec);
         staging_release(&workers[i].wk.in);
         staging_release(&workers[i].wk.out);
+        free(workers[i].wk.points);
     }
     free(workers);
     pthread_mutex_destroy(&q.lock);

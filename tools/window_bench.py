@@ -3,14 +3,16 @@
 The stream is the BASELINE C3 shape: one hour of seeded synthetic 44.1 kHz 16-bit stereo at -m 7, block size 10240,
 built with the GPU encoder.  Measured, in one run:
   - LINNEB200_DecoderBuildIndex on the host image and on the device image;
-  - LINNEB200_DecodeWindows (host image in, host planes out) and LINNEB200_DecodeWindowsResident (both in HBM) for
-    W one-second windows at seeded random starts, W in {1, 8, 64, 512, 4096};
-  - DecodeWhole / DecodeWholeResident of the same stream, for comparison.
-Every window of every W is checked against the slice of a whole-stream decode before any time is reported.  Times are
+  - LINNEB200_DecodeWindows (host image in, host planes out), LINNEB200_DecodeWindowsPacked (host image in, packed
+    WAV data-chunk bytes out, into a page-locked buffer) and LINNEB200_DecodeWindowsResident (both in HBM) for W
+    one-second windows at seeded random starts, W in {1, 8, 64, 512, 4096};
+  - DecodeWhole / DecodeWholePacked / DecodeWholeResident of the same stream, for comparison.
+Every window of every W is checked against the slice of a whole-stream decode (the packed windows against the bytes of
+DecodeWholePacked) before any time is reported.  Times are
 medians of synchronous calls (host wall clock) after a warm-up.  One JSON line goes to stdout and to --out, with the GPU's
 name and power limit read in the same run.
 
-    python tools/window_bench.py [--seconds 3600] [--reps 7] [--out profiles/r3_windows.json]
+    python tools/window_bench.py [--seconds 3600] [--reps 7] [--out profiles/r4_windows_packed.json]
 """
 import argparse
 import ctypes as C
@@ -56,7 +58,7 @@ def main():
     ap.add_argument("--seconds", type=float, default=3600.0)
     ap.add_argument("--reps", type=int, default=7)
     ap.add_argument("--seed", type=int, default=2026)
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r3_windows.json"))
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r4_windows_packed.json"))
     args = ap.parse_args()
 
     import torch
@@ -96,8 +98,18 @@ def main():
     ms_whole = median_ms(lambda: dec.decode_whole(h_stream.data_ptr(), size, full_ptrs, nch, n), args.reps)
     ms_whole_res = median_ms(lambda: dec.decode_whole_resident(h_stream.data_ptr(), d_stream.data_ptr(), size,
                                                                d_full.data_ptr(), stride, nch, n), args.reps)
+    frame = nch * BITS // 8
+    h_full_pk = torch.zeros(n * frame, dtype=torch.uint8).pin_memory()
+    frames = C.c_uint32(0)
+
+    def whole_packed():
+        rc = L.LINNEB200_DecodeWholePacked(dec.h, h_data, size, C.cast(h_full_pk.data_ptr(), u8p), n, C.byref(frames))
+        assert rc == OK and frames.value == n, rc
+    ms_whole_pk = median_ms(whole_packed, args.reps)
     full = h_full.numpy()
+    full_pk = h_full_pk.numpy()
     assert np.array_equal(full, pcm), "whole-stream decode differs from the input"
+    assert full_pk.tobytes() == harness.pack_pcm(pcm, BITS), "packed whole-stream decode differs from the input"
     assert torch.equal(d_full[:, :n], d_pcm[:, :n]), "resident whole-stream decode differs from the input"
 
     # ---- seek index, host hop and device hop ----
@@ -128,9 +140,15 @@ def main():
         out = out_t.numpy()
         out_ptrs = (C.POINTER(C.c_int32) * nch)(*[out[c].ctypes.data_as(C.POINTER(C.c_int32)) for c in range(nch)])
         d_out = torch.full((nch, room), -1, dtype=torch.int32, device=dev)
+        out_pk_t = torch.full((room * frame,), 0xA5, dtype=torch.uint8).pin_memory()
+        out_pk = out_pk_t.numpy()
 
         def host_call():
             rc = L.LINNEB200_DecodeWindows(dec.h, h_data, size, pts_host, N, wins, W, out_ptrs, nch, room)
+            assert rc == OK, rc
+
+        def packed_call():
+            rc = L.LINNEB200_DecodeWindowsPacked(dec.h, h_data, size, pts_host, N, wins, W, out_pk.ctypes.data_as(u8p), room)
             assert rc == OK, rc
 
         def resident_call():
@@ -138,12 +156,15 @@ def main():
                                                    C.c_void_p(d_out.data_ptr()), room)
             assert rc == OK, rc
         host_call()
+        packed_call()
         resident_call()
         back = d_out.cpu().numpy()
         for w, s in enumerate(starts):
             want = full[:, s:s + RATE]
             assert np.array_equal(out[:, w * RATE:(w + 1) * RATE], want), f"W={W}: window {w} differs (host buffers)"
             assert np.array_equal(back[:, w * RATE:(w + 1) * RATE], want), f"W={W}: window {w} differs (resident)"
+            assert np.array_equal(out_pk[w * RATE * frame:(w + 1) * RATE * frame], full_pk[s * frame:(s + RATE) * frame]), \
+                f"W={W}: window {w} differs (packed)"
         marks = np.zeros(N + 1, np.int64)
         firsts = np.frombuffer(bytes(pts_host), np.uint32).reshape(-1, 2)[:, 0]
         k0 = np.searchsorted(firsts, starts, side="right") - 1
@@ -156,6 +177,7 @@ def main():
         launches = dec.launch_count() - before
         results[str(W)] = {"blocks": blocks, "launches": int(launches),
                            "host_ms": round(median_ms(host_call, args.reps), 3),
+                           "packed_ms": round(median_ms(packed_call, args.reps), 3),
                            "resident_ms": round(median_ms(resident_call, args.reps), 3)}
     dec.close()
 
@@ -167,10 +189,12 @@ def main():
                     f"{size} bytes; one-second windows at seeded random starts",
         "gpu": gpu_name, "power_limit": power_limit,
         "index_ms": {"host": round(ms_index_host, 3), "device": round(ms_index_dev, 3)},
-        "whole_ms": {"host": round(ms_whole, 3), "resident": round(ms_whole_res, 3)},
+        "whole_ms": {"host": round(ms_whole, 3), "packed": round(ms_whole_pk, 3), "resident": round(ms_whole_res, 3)},
         "windows": results,
-        "first_W_not_faster_than_whole": {"host": crossover("host_ms", ms_whole), "resident": crossover("resident_ms", ms_whole_res)},
-        "checked": "every window equals the whole-stream decode slice (host buffers and resident)",
+        "first_W_not_faster_than_whole": {"host": crossover("host_ms", ms_whole), "packed": crossover("packed_ms", ms_whole_pk),
+                                          "resident": crossover("resident_ms", ms_whole_res)},
+        "checked": "every window equals the whole-stream decode slice (host planes and resident) or the DecodeWholePacked "
+                   "bytes (packed)",
         "timing": f"median of {args.reps} synchronous calls after one warm-up, host wall clock",
     }
     text = json.dumps(line)
