@@ -179,7 +179,10 @@ void  LINNEB200_HostFree(void *h_ptr);
 
 /* ---- encode with externally supplied analysis results ------------------------------------------
  * One record per (block, channel), block-major.  Used to show that identical quantised
- * coefficients yield byte-identical residuals and coded bits (north star, parity leg 3). */
+ * coefficients yield byte-identical residuals and coded bits (north star, parity leg 3).
+ * For every layer of the preset, log2_units must be at most 7 and rshift at most 15: the stream
+ * stores them in 3 and 4 bits.  A record with a larger value makes the call return
+ * INVALID_ARGUMENT before anything is written.  A layer with more units than taps predicts nothing. */
 struct LINNEB200ChannelParams {
     uint8_t log2_units[3];
     uint8_t rshift[3];

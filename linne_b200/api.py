@@ -653,7 +653,7 @@ class Product(LinneApi):
         finally:
             self.lib.LINNEDecoder_Destroy(dec)
 
-    def encode_with_params(self, pcm, params, bits=16, rate=44100, block=10240, preset=0, ms=None):
+    def encode_with_params(self, pcm, params, bits=16, rate=44100, block=10240, preset=0, ms=None, return_code=False):
         """params: ctypes array of ChannelParams, one per (block, channel), block-major."""
         pcm = np.ascontiguousarray(pcm, dtype=np.int32)
         nch, n = pcm.shape
@@ -664,6 +664,8 @@ class Product(LinneApi):
             size = C.c_uint32(0)
             rc = self.lib.LINNEB200_EncodeWholeWithParams(sess.h, _chan_ptrs(pcm), n, params, len(params) // nch,
                                                           out.ctypes.data_as(C.POINTER(C.c_uint8)), cap, C.byref(size))
+            if return_code:
+                return rc, out[:size.value].tobytes() if rc == OK else b""
             if rc != OK:
                 raise RuntimeError(f"EncodeWholeWithParams rc={rc}")
             return out[:size.value].tobytes()

@@ -632,6 +632,10 @@ LINNEApiResult LINNEB200_EncodeWholeWithParams(struct LINNEEncoder *enc, const i
     C = enc->header.num_channels;
     blocks = (num_samples + enc->header.num_samples_per_block - 1u) / enc->header.num_samples_per_block;
     if (num_param_blocks < blocks) return LINNE_APIRESULT_INVALID_ARGUMENT;
+    /* the stream stores these in 3 and 4 bits: a larger value would be written masked but predicted with unmasked */
+    for (i = 0; i < blocks * C; i++)
+        for (l = 0; l < (uint32_t)g_lnb_presets[enc->header.preset].num_layers; l++)
+            if (params[i].log2_units[l] > 7u || params[i].rshift[l] > 15u) return LINNE_APIRESULT_INVALID_ARGUMENT;
     enc->header.num_samples = num_samples;
     if ((ret = LINNEEncoder_EncodeHeader(&enc->header, data, data_size)) != LINNE_APIRESULT_OK) return ret;
     forced = (LnbChanParams *)calloc((size_t)blocks * C, sizeof(LnbChanParams));

@@ -263,8 +263,7 @@ __global__ void __launch_bounds__(LNB_FR_THREADS) lnb_predict_plan_v2_kernel(Lnb
     int32_t *in = bufA, *out = bufB;
     for (uint32_t l = 0; l < b.cfg.num_layers; l++) {
         const uint32_t P = b.cfg.layer_params[l];
-        uint32_t U = 1u << prm.log2_units[l];
-        if (U > P) U = P;
+        const uint32_t U = 1u << prm.log2_units[l];
         const uint32_t p = P / U, m = n / U, rshift = prm.rshift[l];
         const uint32_t half = rshift ? (1u << (rshift - 1u)) : 0u;
         for (uint32_t k = tid; k < P; k += LNB_FR_THREADS) sm.coef[k] = (int32_t)prm.coef[l * LNB_MAX_PARAMS + k];
@@ -273,7 +272,8 @@ __global__ void __launch_bounds__(LNB_FR_THREADS) lnb_predict_plan_v2_kernel(Lnb
             const uint32_t u = (m > 0u) ? t / m : U;
             const uint32_t pos = t - u * m;
             int32_t v = in[t];
-            if (u < U && pos >= p && m > p) {
+            /* more units than taps: the layer predicts nothing, as in the reference and every decoder */
+            if (u < U && U <= P && pos >= p && m > p) {
                 const int32_t *h = in + t - p;
                 const int32_t *cf = sm.coef + u * p;
                 uint32_t acc = half;
