@@ -555,21 +555,20 @@ static int decode_whole_sharded(struct LINNEDecoder *dec, const uint8_t *data, u
     LnbTurnstile turn;
     LnbHopResult scan;
     const LnbBlockDesc *table;
-    uint32_t G, k, c, started = 0, ndev_used = 1;
-    int home, own;
+    uint32_t G, k, c, started = 0, ndev_used;
+    int home, ordinal[LNB_MAX_DEVICES];
     if (ndev <= 0) return 0;
     /* the handle's own block table: the children decode their ranges with tables of their own */
     if (hop_host(dec, h, data, data_size, LINNE_HEADER_SIZE, buffer_num_samples, h->num_samples, 0u, 0u, &scan)) return 0;
     table = (const LnbBlockDesc *)dec->h_blocks.ptr;
     /* ranges per requested device (pipelining), devices shared round-robin when fewer are visible than asked for */
     G = lnb_plan_ranges(scan.num_decodable, dec->num_devices > 1u ? dec->num_devices : 1u);
-    ndev_used = dec->num_devices > 1u ? (dec->num_devices < (uint32_t)ndev ? dec->num_devices : (uint32_t)ndev) : 1u;
     if (G < 2u) return 0;                                        /* a handful of blocks: the handle's own device */
     home = lnb_shim_current_device();
-    own = lnb_shim_device_ordinal(dec->dev);
+    ndev_used = lnb_place_ranges(dec->num_devices, ndev, lnb_shim_device_ordinal(dec->dev), G, ordinal);
     for (k = 0; k < G; k++) {
         if (!dec->child[k]) {
-            lnb_shim_set_device(dec->num_devices > 1u ? (int)(k % ndev_used) : own);
+            lnb_shim_set_device(ordinal[k]);
             dec->child[k] = LINNEDecoder_Create(&dec->config, NULL, 0);
             if (dec->child[k]) dec->child[k]->num_devices = 0;
         }
@@ -603,7 +602,7 @@ static int decode_whole_sharded(struct LINNEDecoder *dec, const uint8_t *data, u
         sh[k].room = buffer_num_samples - first->smp_off;
         sh[k].sample_limit = last ? h->num_samples - first->smp_off : table[b1].smp_off - first->smp_off;
         sh[k].block_limit = last ? 0u : b1 - b0;
-        sh[k].ordinal = dec->num_devices > 1u ? (int)(k % ndev_used) : own;
+        sh[k].ordinal = ordinal[k];
         dec->child[k]->turn = &turn; dec->child[k]->turn_index = k;
         if (pthread_create(&th[k], NULL, dec_shard_main, &sh[k]) != 0) {
             dec->child[k]->turn = NULL;

@@ -170,3 +170,11 @@ uint32_t lnb_plan_ranges(uint32_t blocks, uint32_t devices)
     if (ranges * 2u > blocks) ranges = blocks / 2u;              /* at least two blocks per range */
     return ranges < 1u ? 1u : ranges;
 }
+
+uint32_t lnb_place_ranges(uint32_t requested, int visible, int own, uint32_t G, int *ordinal)
+{
+    const uint32_t used = requested > 1u ? (requested < (uint32_t)visible ? requested : (uint32_t)visible) : 1u;
+    uint32_t k;
+    for (k = 0; k < G; k++) ordinal[k] = requested > 1u ? (int)(k % used) : own;
+    return used;
+}

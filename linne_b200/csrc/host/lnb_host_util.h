@@ -35,6 +35,10 @@ void lnb_fill_stream_cfg(LnbStreamCfg *cfg, const struct LINNEHeader *h);
  * Returns 1 when the call should simply run on the handle's own device. */
 uint32_t lnb_plan_ranges(uint32_t blocks, uint32_t devices);
 
+/* Devices of the G ranges of a sharded call: ordinal[k] = k mod D on a handle asked for `requested` > 1 devices, D = no
+ * more than the `visible` ones (>= 1); the handle's own device `own` otherwise.  Returns D, the devices in use. */
+uint32_t lnb_place_ranges(uint32_t requested, int visible, int own, uint32_t G, int *ordinal);
+
 /* rendezvous of the shard workers of one call with the thread that made it: every worker reports ("sized"), the caller
  * looks at all reports and releases them ("placed") */
 #include <pthread.h>
