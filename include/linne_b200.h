@@ -142,6 +142,61 @@ LINNEApiResult LINNEB200_DecodeWindowsPacked(struct LINNEDecoder *decoder, const
         const struct LINNEB200SeekPoint *points, uint32_t num_points, struct LINNEB200Window *windows, uint32_t num_windows,
         uint8_t *pcm, uint32_t pcm_capacity_frames);
 
+/* ---- salvage decodes: every intact block of a damaged stream -------------------------------------------------------
+ * DecodeSalvage decodes what is left of a damaged stream.  Every block that can be verified and placed is decoded to
+ * its place, samples it cannot account for are zero (silence; the biased 128 in 8-bit packed output), and the damage is
+ * reported.  The stream's header is the one latched on the handle (SetHeader or BuildIndex), as for DecodeWindows: the
+ * image's first 30 bytes are skipped and not parsed, so a caller who knows the parameters recovers a stream whose header
+ * is damaged.  CRCs are always checked, whatever the handle's check_crc.  B = num_samples_per_block, N = num_samples and
+ * T = N - B * (ceil(N / B) - 1), the length of the tail block, all from the header.
+ *
+ * A verified block at byte offset o >= 30 passes the framing checks of DecodeWhole with data_size - o bytes left, holds
+ * 1 .. B samples, is at most 2 * B * num_channels * ceil(bits_per_sample / 8) + 4171 bytes long (twice a raw block plus
+ * 4 KiB: more room than this library's encoder gives a block) and matches its CRC16.  Its successor is the offset DecodeWhole's hop goes to next.  It is confirmed
+ * when its successor is another verified block or data_size.  The walk runs from offset 30, sample 0:
+ *   - a verified block at the current offset is accepted at the current sample;
+ *   - otherwise a damaged region starts there; v is the first confirmed block after it.  When the damaged bytes still
+ *     frame as a block of B samples and a chain of such blocks (verified ones between them) leads from there exactly to
+ *     v (damaged payloads), the damaged block is lost in place: the walk moves on B samples and to its successor.  Any
+ *     other damage (a framing gap) ends the segment of blocks; a new one starts at v, not knowing its sample position.
+ *     With no v the region runs to the end of the image.
+ *   - the first segment (anchored at sample 0) ends when it reaches N samples; bytes after that are ignored.
+ * The last segment is placed when its chain ends exactly at data_size with a block of T samples (it then ends at sample
+ * N) and it starts at or after the end of the first.  Segments between two framing gaps are placed only when the last
+ * one is and the samples lost between the first and the last are B times the number of framing gaps, i.e. when each
+ * gap cost exactly one block (a damaged block header).  Any other segment is not decoded.
+ * Every placed block lands where it is in the intact stream and its samples are exactly what DecodeWhole writes for it;
+ * a block whose CRC failed never reaches the decode kernels.
+ *
+ * Two limits.  Blocks do not store their position, so whole blocks removed exactly at block boundaries leave no trace in
+ * the bytes and the walk cannot see them, just as DecodeWhole cannot.  And the rule for segments between framing gaps
+ * counts only the total: when the gaps cost different numbers of blocks that add up to B samples per gap (one gap of
+ * inserted bytes that cost nothing and one that cost two blocks, say), the segments between them are placed at the
+ * wrong sample positions, and samples outside the records then differ from the intact stream's.
+ *
+ * `damage` gets one record per maximal run of output samples that no placed block wrote, in stream order: the sample range,
+ * the bytes of the image it covers (undecoded segments included) and the status of its first failing position --
+ * INVALID_FORMAT or INSUFFICIENT_DATA when the bytes there do not frame as a block (sync code, size field; as DecodeWhole
+ * reports them), DETECT_DATA_CORRUPTION when they do.  Bytes inserted between two blocks give a record with
+ * num_samples = 0; a stream that ends on a block boundary before N gives (s, N - s, data_size, 0, INSUFFICIENT_DATA).
+ * `*num_damage` is always the number of records; the first `capacity` are written (damage may be NULL when capacity is 0).
+ *
+ * Returns OK when there are no records -- the output then equals DecodeWhole's / DecodeWholePacked's -- and
+ * DETECT_DATA_CORRUPTION when there are: the output is complete (N samples per channel) and the records say what is
+ * missing.  Rejected as a whole (nothing written): NULL pointers (INVALID_ARGUMENT), no latched header
+ * (PARAMETER_NOT_SET), fewer buffer channels than the stream has or room for fewer than N samples (buffer_num_samples,
+ * pcm_capacity_frames: INSUFFICIENT_BUFFER), and for the packed call bits_per_sample other than 8, 16, 24 or 32
+ * (INVALID_FORMAT).  The whole image goes to the device; a call is the scan, one CRC pass, one decode batch (and one
+ * conversion to packed PCM), whatever the damage.  A handle with several devices salvages on its own device; the
+ * DecodeBlock read-ahead cache is left as it was. */
+struct LINNEB200Damage { uint32_t first_sample, num_samples, byte_offset, byte_size; int32_t status; };
+LINNEApiResult LINNEB200_DecodeSalvage(struct LINNEDecoder *decoder, const uint8_t *data, uint32_t data_size,
+        int32_t **buffer, uint32_t buffer_num_channels, uint32_t buffer_num_samples,
+        struct LINNEB200Damage *damage, uint32_t capacity, uint32_t *num_damage);
+LINNEApiResult LINNEB200_DecodeSalvagePacked(struct LINNEDecoder *decoder, const uint8_t *data, uint32_t data_size,
+        uint8_t *pcm, uint32_t pcm_capacity_frames,
+        struct LINNEB200Damage *damage, uint32_t capacity, uint32_t *num_damage);
+
 /* ---- packed PCM entry points (SURVEY 8f.2) ------------------------------------------------------------
  * `pcm` = interleaved little-endian samples exactly as in a WAV data chunk (8-bit unsigned with a bias of 128,
  * 16/24/32-bit signed; bits per sample = the encoder's parameter / the stream header).  The conversion to and

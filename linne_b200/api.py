@@ -284,6 +284,53 @@ class LinneApi:
             return rc, [out[offs[w] * frame:offs[w + 1] * frame].tobytes() for w in range(nw)]
         return self._windows(data, starts, lengths, index, check_crc, return_code, "DecodeWindowsPacked", call)
 
+    # -- salvage (include/linne_b200.h: LINNEB200_DecodeSalvage / DecodeSalvagePacked) ------------------------------------
+    def _salvage(self, data: bytes, header, call):
+        """The handle with the stream's header latched -- `header` (a LINNEHeader) when given, e.g. for a stream whose own
+        header is damaged, else the image's -- then `call(dec, hdr, buf, damage, capacity, count)` -> (rc, output), run
+        again with room for every record when the first run found more than it had room for."""
+        if header is None:
+            rc, header = self.decode_header(data)
+            if rc != OK:
+                return rc, None, []
+        dec = self._open_decoder(header.num_channels, 1)
+        try:
+            rc = self.lib.LINNEDecoder_SetHeader(dec, C.byref(header))
+            if rc != OK:
+                return rc, None, []
+            buf = np.frombuffer(data, dtype=np.uint8)
+            cap, count = 64, C.c_uint32(0)
+            while True:
+                damage = (Damage * cap)()
+                rc, out = call(dec, header, buf.ctypes.data_as(C.POINTER(C.c_uint8)), damage, cap, count)
+                if count.value <= cap:
+                    break
+                cap = count.value
+            records = [(d.first_sample, d.num_samples, d.byte_offset, d.byte_size, d.status) for d in damage[:count.value]]
+            return rc, out, records
+        finally:
+            self.lib.LINNEDecoder_Destroy(dec)
+
+    def decode_salvage(self, data: bytes, header=None):
+        """Every intact block of a possibly damaged stream (LINNEB200_DecodeSalvage) -> (rc, int32 [C][N] planes, records),
+        records = [(first_sample, num_samples, byte_offset, byte_size, status)]; samples inside a record are zero."""
+        def call(dec, hdr, u8p, damage, cap, count):
+            out = np.zeros((max(hdr.num_channels, 1), max(hdr.num_samples, 1)), dtype=np.int32)
+            rc = self.lib.LINNEB200_DecodeSalvage(dec, u8p, len(data), _chan_ptrs(out), hdr.num_channels, hdr.num_samples,
+                                                  damage, cap, C.byref(count))
+            return rc, out[:, :hdr.num_samples]
+        return self._salvage(data, header, call)
+
+    def decode_salvage_packed(self, data: bytes, header=None):
+        """The same as WAV data-chunk bytes (LINNEB200_DecodeSalvagePacked) -> (rc, bytes, records)."""
+        def call(dec, hdr, u8p, damage, cap, count):
+            nbytes = hdr.num_samples * hdr.num_channels * (hdr.bits_per_sample // 8)
+            out = np.zeros(max(nbytes, 1), dtype=np.uint8)
+            rc = self.lib.LINNEB200_DecodeSalvagePacked(dec, u8p, len(data), out.ctypes.data_as(C.POINTER(C.c_uint8)),
+                                                        hdr.num_samples, damage, cap, C.byref(count))
+            return rc, out[:nbytes].tobytes()
+        return self._salvage(data, header, call)
+
 
 def bind_ext_api(lib):
     """Declare the LINNEB200_* extension entry points (include/linne_b200.h)."""
@@ -345,6 +392,12 @@ def bind_ext_api(lib):
     lib.LINNEB200_DecodeWindowsPacked.argtypes = [C.c_void_p, u8p, C.c_uint32, C.POINTER(SeekPoint), C.c_uint32, C.POINTER(Window),
                                                   C.c_uint32, u8p, C.c_uint32]
     lib.LINNEB200_DecodeWindowsPacked.restype = C.c_int
+    dmg = C.POINTER(Damage)
+    lib.LINNEB200_DecodeSalvage.argtypes = [C.c_void_p, u8p, C.c_uint32, C.POINTER(C.POINTER(C.c_int32)), C.c_uint32, C.c_uint32,
+                                            dmg, C.c_uint32, u32p]
+    lib.LINNEB200_DecodeSalvage.restype = C.c_int
+    lib.LINNEB200_DecodeSalvagePacked.argtypes = [C.c_void_p, u8p, C.c_uint32, u8p, C.c_uint32, dmg, C.c_uint32, u32p]
+    lib.LINNEB200_DecodeSalvagePacked.restype = C.c_int
     lib.LINNEB200_DecoderSetReadahead.argtypes = [C.c_void_p, C.c_uint32]
     lib.LINNEB200_DecoderSetThroughputBlocks.argtypes = [C.c_void_p, C.c_uint32]
     lib.LINNEB200_EncoderSetDevices.argtypes = [C.c_void_p, C.c_uint32]
@@ -399,6 +452,12 @@ class SeekPoint(C.Structure):
 class Window(C.Structure):
     """struct LINNEB200Window (include/linne_b200.h): one sample window of LINNEB200_DecodeWindows"""
     _fields_ = [("first_sample", C.c_uint32), ("num_samples", C.c_uint32), ("out_offset", C.c_uint32), ("status", C.c_int32)]
+
+
+class Damage(C.Structure):
+    """struct LINNEB200Damage (include/linne_b200.h): one run of samples a salvage decode could not recover"""
+    _fields_ = [("first_sample", C.c_uint32), ("num_samples", C.c_uint32), ("byte_offset", C.c_uint32),
+                ("byte_size", C.c_uint32), ("status", C.c_int32)]
 
 
 def index_points(index):

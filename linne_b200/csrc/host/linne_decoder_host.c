@@ -1201,3 +1201,239 @@ LINNEApiResult LINNEB200_DecodeWindowsResident(struct LINNEDecoder *dec, const u
     if (!(dec->flags & DEC_FLAG_HEADER_SET)) return LINNE_APIRESULT_PARAMETER_NOT_SET;
     return decode_windows(dec, NULL, d_data, data_size, points, num_points, windows, num_windows, NULL, d_pcm, NULL, pcm_stride);
 }
+
+/* ---- salvage decodes (include/linne_b200.h) -------------------------------------------------------------------------
+ * The resynchronising scan finds every position of the image that frames as a block, one CRC pass verifies them, and one
+ * serial walk over the verified blocks (sorted by offset) follows the stream's chain, steps over damage and places what it
+ * can account for.  The placed blocks go through the unchanged decode pipeline as one batch, at their sample positions in
+ * the intact stream. */
+static int by_byte_off(const void *a, const void *b)
+{
+    const uint32_t x = ((const LnbBlockDesc *)a)->byte_off, y = ((const LnbBlockDesc *)b)->byte_off;
+    return (x > y) - (x < y);
+}
+
+/* the offset DecodeWhole's hop goes to after the verified block *b */
+static uint32_t salvage_next(const struct LINNEHeader *h, const LnbBlockDesc *b)
+{
+    return lnb_block_next(b->byte_off, b->type, b->byte_size - 6u, b->nsmp, h->num_channels, h->bits_per_sample);
+}
+
+/* the first of the n verified blocks (sorted) at or after byte o */
+static uint32_t salvage_find(const LnbBlockDesc *v, uint32_t n, uint32_t o)
+{
+    uint32_t lo = 0, hi = n;
+    while (lo < hi) {
+        const uint32_t mid = lo + (hi - lo) / 2u;
+        if (v[mid].byte_off < o) lo = mid + 1u; else hi = mid;
+    }
+    return lo;
+}
+
+/* the status of damage that starts at byte pos: the framing error DecodeWhole reports there, or DETECT_DATA_CORRUPTION
+ * for bytes that frame as a block (a block that frames but is not verified failed its CRC or a later check) */
+static int32_t salvage_status(const uint8_t *data, uint32_t data_size, uint32_t pos)
+{
+    uint32_t size32 = 0, err;
+    if (pos >= data_size) return (int32_t)LINNE_APIRESULT_INSUFFICIENT_DATA;
+    err = lnb_block_frame(data + pos, data_size - pos, &size32);
+    return err != LNB_HOP_OK ? (int32_t)err : (int32_t)LINNE_APIRESULT_DETECT_DATA_CORRUPTION;
+}
+
+/* Damage in place: from pos a chain of blocks leads exactly to the confirmed block v -- damaged ones that still frame as
+ * blocks of B samples (a damaged payload), verified ones between them.  Their positions then follow from pos. */
+static int salvage_in_place(const struct LINNEHeader *h, const uint8_t *data, uint32_t data_size,
+                            const LnbBlockDesc *v, uint32_t nv, uint32_t pos, uint32_t to)
+{
+    while (pos < to) {
+        const uint32_t j = salvage_find(v, nv, pos);
+        uint32_t size32 = 0, ns;
+        if (j < nv && v[j].byte_off == pos) { pos = salvage_next(h, &v[j]); continue; }
+        if (lnb_block_frame(data + pos, data_size - pos, &size32) != LNB_HOP_OK) return 0;
+        if ((ns = lnb_rd_be(data + pos + 9, 2)) != h->num_samples_per_block) return 0;
+        pos = lnb_block_next(pos, data[pos + 8], size32, ns, h->num_channels, h->bits_per_sample);
+    }
+    return pos == to;
+}
+
+/* a segment of the walk: blocks [first, first + count) of the walk's table, the samples it spans (damage in place
+ * included), the offset where its chain ended, and its first sample once placed */
+typedef struct { uint32_t first, count, span, end, base, placed; } SalvageSeg;
+
+/* Shared by DecodeSalvage (planes into `buffer`) and DecodeSalvagePacked (packed PCM into `packed`); arguments checked. */
+static LINNEApiResult decode_salvage(struct LINNEDecoder *dec, const uint8_t *data, uint32_t data_size, int32_t **buffer,
+        uint8_t *packed, struct LINNEB200Damage *damage, uint32_t capacity, uint32_t *num_damage)
+{
+    const struct LINNEHeader *h = &dec->header;
+    const uint32_t C = h->num_channels, N = h->num_samples, B = h->num_samples_per_block, bytes = h->bits_per_sample / 8u;
+    const uint32_t nblocks = (uint32_t)(((uint64_t)N + B - 1u) / B), T = N ? N - B * (nblocks - 1u) : 0u;
+    const uint32_t start = data_size < LINNE_HEADER_SIZE ? data_size : (uint32_t)LINNE_HEADER_SIZE;
+    const size_t padded = LNB_ROUNDUP((size_t)data_size + 16u, 16u), stride = LNB_ROUNDUP((size_t)N + 4u, 4u);
+    LINNEApiResult overall = LINNE_APIRESULT_NG;
+    LnbDecodeBatch batch;
+    LnbBlockDesc *v, *w;
+    SalvageSeg *seg = NULL;
+    struct LINNEB200Damage *rec = NULL;
+    uint32_t *next_conf = NULL, cap = nblocks + nblocks / 8u + 64u, count, nv = 0, nw = 0, nseg = 1, nrec = 0, np = 0, i, k, c;
+    uint32_t pos, s, prev_s, prev_byte;
+
+    *num_damage = 0;
+    if (N == 0) return LINNE_APIRESULT_OK;
+    /* ---- the whole image up; scan and CRC pass; the candidates come back in one piece (grown and run again if they
+     * did not fit) ---- */
+    if (lnb_buf_reserve_device(dec->dev, &dec->d_stream, padded)
+        || lnb_buf_reserve_device(dec->dev, &dec->d_pcm, stride * C * sizeof(int32_t))
+        || (packed && lnb_buf_reserve_device(dec->dev, &dec->d_packed, (size_t)N * C * bytes + 16u))) return LINNE_APIRESULT_NG;
+    lnb_shim_memset(dec->dev, (uint8_t *)dec->d_stream.ptr + (padded - 16u), 0, 16u);
+    lnb_shim_h2d(dec->dev, dec->d_stream.ptr, data, data_size);
+    for (;;) {
+        const size_t table_bytes = 16u + (size_t)cap * sizeof(LnbBlockDesc);     /* the counter, then the table */
+        LnbBlockDesc *d_table;
+        if (lnb_buf_reserve_device(dec->dev, &dec->d_hop_table, table_bytes) || lnb_buf_reserve_host(&dec->h_hop, table_bytes))
+            return LINNE_APIRESULT_NG;
+        d_table = (LnbBlockDesc *)((uint8_t *)dec->d_hop_table.ptr + 16);
+        lnb_shim_memset(dec->dev, dec->d_hop_table.ptr, 0, sizeof(uint32_t));
+        if (lnb_shim_resync_scan(dec->dev, (const uint8_t *)dec->d_stream.ptr, data_size, C, h->bits_per_sample, B,
+                                 d_table, (uint32_t *)dec->d_hop_table.ptr, cap)
+            || lnb_shim_crc_blocks(dec->dev, (const uint8_t *)dec->d_stream.ptr, data_size, d_table,
+                                   (const uint32_t *)dec->d_hop_table.ptr, cap)) return LINNE_APIRESULT_NG;
+        lnb_shim_d2h(dec->dev, dec->h_hop.ptr, dec->d_hop_table.ptr, table_bytes);
+        if (lnb_shim_sync(dec->dev)) return LINNE_APIRESULT_NG;
+        count = *(const uint32_t *)dec->h_hop.ptr;
+        if (count <= cap) break;
+        cap = count + count / 8u + 64u;
+    }
+
+    /* ---- the verified blocks by offset; which are confirmed; the first confirmed one at or after each ---- */
+    v = (LnbBlockDesc *)((uint8_t *)dec->h_hop.ptr + 16);
+    for (i = 0; i < count; i++) if (!(v[i].status & LNB_ST_CRC_MISMATCH)) v[nv++] = v[i];
+    qsort(v, nv, sizeof(LnbBlockDesc), by_byte_off);
+    if (lnb_buf_reserve_host(&dec->h_blocks, ((size_t)nv + 1u) * sizeof(LnbBlockDesc))
+        || !(next_conf = (uint32_t *)malloc(((size_t)nv + 1u) * sizeof(uint32_t)))
+        || !(seg = (SalvageSeg *)calloc((size_t)nv + 2u, sizeof(SalvageSeg)))
+        || !(rec = (struct LINNEB200Damage *)malloc(((size_t)nv + 2u) * sizeof(struct LINNEB200Damage)))) goto done;
+    w = (LnbBlockDesc *)dec->h_blocks.ptr;
+    next_conf[nv] = nv;
+    for (k = nv; k-- > 0; ) {
+        const uint32_t succ = salvage_next(h, &v[k]), j = salvage_find(v, nv, succ);
+        next_conf[k] = (succ == data_size || (j < nv && v[j].byte_off == succ)) ? k : next_conf[k + 1u];
+    }
+
+    /* ---- the walk ---- */
+    pos = LINNE_HEADER_SIZE; s = 0;
+    seg[0].end = start;
+    while (pos < data_size) {
+        SalvageSeg *g = &seg[nseg - 1u];
+        const uint32_t j = salvage_find(v, nv, pos);
+        if (nseg == 1u && s >= N) break;
+        if (j < nv && v[j].byte_off == pos) {
+            if (nseg == 1u && v[j].nsmp > N - s) break;            /* it would run past the stream's samples */
+            w[nw] = v[j];
+            w[nw].smp_off = s;
+            w[nw].status = 0;
+            nw++; g->count++;
+            s += v[j].nsmp;
+            pos = salvage_next(h, &v[j]);
+            g->span = s; g->end = pos;
+            continue;
+        }
+        {
+            const uint32_t nc = next_conf[j];
+            if (nc < nv && salvage_in_place(h, data, data_size, v, nv, pos, v[nc].byte_off)) {
+                uint32_t size32 = 0;                                /* the damaged block: B samples of silence */
+                lnb_block_frame(data + pos, data_size - pos, &size32);
+                s += B;
+                pos = lnb_block_next(pos, data[pos + 8], size32, B, C, h->bits_per_sample);
+                g->span = s; g->end = pos;
+                continue;
+            }
+            if (nc == nv) break;                                    /* the damage runs to the end of the image */
+            seg[nseg].first = nw;
+            seg[nseg].end = pos = v[nc].byte_off;
+            nseg++;
+            s = 0;
+        }
+    }
+
+    /* ---- placing: the first segment as walked; the last one from the end; those between only when every framing gap
+     * cost exactly one block ---- */
+    seg[0].placed = 1;
+    if (nseg >= 2u) {
+        SalvageSeg *L = &seg[nseg - 1u];
+        uint64_t middle = 0;
+        for (k = 1; k + 1u < nseg; k++) middle += seg[k].span;
+        if (L->count && L->end == data_size && w[L->first + L->count - 1u].nsmp == T && L->span <= N - seg[0].span) {
+            L->base = N - L->span;
+            L->placed = 1;
+            if (nseg > 2u && (uint64_t)L->base - seg[0].span == middle + (uint64_t)B * (nseg - 1u)) {
+                uint32_t b = seg[0].span;
+                for (k = 1; k + 1u < nseg; k++) { seg[k].base = b + B; seg[k].placed = 1; b = seg[k].base + seg[k].span; }
+            }
+        }
+    }
+    for (k = 0; k < nseg; k++) {                                    /* the placed blocks, in stream order, compacted */
+        if (!seg[k].placed) continue;
+        for (i = seg[k].first; i < seg[k].first + seg[k].count; i++) { w[np] = w[i]; w[np].smp_off += seg[k].base; np++; }
+    }
+
+    /* ---- the report: every run of samples no placed block writes ---- */
+    prev_s = 0; prev_byte = start;
+    for (i = 0; i <= np; i++) {
+        const uint32_t at_s = i < np ? w[i].smp_off : N, at_byte = i < np ? w[i].byte_off : data_size;
+        if (at_s > prev_s || (i < np && at_byte > prev_byte)) {
+            struct LINNEB200Damage *r = &rec[nrec++];
+            r->first_sample = prev_s; r->num_samples = at_s - prev_s;
+            r->byte_offset = prev_byte; r->byte_size = at_byte - prev_byte;
+            r->status = salvage_status(data, data_size, prev_byte);
+        }
+        if (i < np) { prev_s = w[i].smp_off + w[i].nsmp; prev_byte = salvage_next(h, &w[i]); }
+    }
+
+    /* ---- the decode: silence where nothing is placed, the placed blocks as one batch ---- */
+    if (nrec) lnb_shim_memset(dec->dev, dec->d_pcm.ptr, 0, stride * C * sizeof(int32_t));
+    if (np) {
+        if (setup_batch(dec, &batch, w, np, (const uint8_t *)dec->d_stream.ptr, data_size, (int32_t *)dec->d_pcm.ptr, (uint32_t)stride)) goto done;
+        lnb_shim_h2d(dec->dev, dec->d_blocks.ptr, w, (size_t)np * sizeof(LnbBlockDesc));
+        if (lnb_shim_decode(dec->dev, &batch)) goto done;
+    }
+    if (packed) {
+        if (lnb_shim_pack_pcm(dec->dev, (const int32_t *)dec->d_pcm.ptr, (uint8_t *)dec->d_packed.ptr, (uint32_t)stride, N, C, bytes)) goto done;
+        lnb_shim_d2h(dec->dev, packed, dec->d_packed.ptr, (size_t)N * C * bytes);
+    } else {
+        for (c = 0; c < C; c++) lnb_shim_d2h(dec->dev, buffer[c], (const int32_t *)dec->d_pcm.ptr + (size_t)c * stride, (size_t)N * sizeof(int32_t));
+    }
+    if (lnb_shim_sync(dec->dev)) goto done;
+    for (i = 0; i < nrec && i < capacity; i++) damage[i] = rec[i];
+    *num_damage = nrec;
+    overall = nrec ? LINNE_APIRESULT_DETECT_DATA_CORRUPTION : LINNE_APIRESULT_OK;
+done:
+    free(next_conf);
+    free(seg);
+    free(rec);
+    return overall;
+}
+
+LINNEApiResult LINNEB200_DecodeSalvage(struct LINNEDecoder *dec, const uint8_t *data, uint32_t data_size,
+        int32_t **buffer, uint32_t buffer_num_channels, uint32_t buffer_num_samples,
+        struct LINNEB200Damage *damage, uint32_t capacity, uint32_t *num_damage)
+{
+    uint32_t c;
+    if (dec == NULL || data == NULL || buffer == NULL || num_damage == NULL || (damage == NULL && capacity)) return LINNE_APIRESULT_INVALID_ARGUMENT;
+    if (!(dec->flags & DEC_FLAG_HEADER_SET)) return LINNE_APIRESULT_PARAMETER_NOT_SET;
+    if (buffer_num_channels < dec->header.num_channels || buffer_num_samples < dec->header.num_samples) return LINNE_APIRESULT_INSUFFICIENT_BUFFER;
+    for (c = 0; c < dec->header.num_channels; c++) if (buffer[c] == NULL) return LINNE_APIRESULT_INVALID_ARGUMENT;
+    return decode_salvage(dec, data, data_size, buffer, NULL, damage, capacity, num_damage);
+}
+
+LINNEApiResult LINNEB200_DecodeSalvagePacked(struct LINNEDecoder *dec, const uint8_t *data, uint32_t data_size,
+        uint8_t *pcm, uint32_t pcm_capacity_frames,
+        struct LINNEB200Damage *damage, uint32_t capacity, uint32_t *num_damage)
+{
+    uint32_t bits;
+    if (dec == NULL || data == NULL || pcm == NULL || num_damage == NULL || (damage == NULL && capacity)) return LINNE_APIRESULT_INVALID_ARGUMENT;
+    if (!(dec->flags & DEC_FLAG_HEADER_SET)) return LINNE_APIRESULT_PARAMETER_NOT_SET;
+    if (pcm_capacity_frames < dec->header.num_samples) return LINNE_APIRESULT_INSUFFICIENT_BUFFER;
+    bits = dec->header.bits_per_sample;
+    if (bits != 8u && bits != 16u && bits != 24u && bits != 32u) return LINNE_APIRESULT_INVALID_FORMAT;
+    return decode_salvage(dec, data, data_size, NULL, pcm, damage, capacity, num_damage);
+}

@@ -8,12 +8,13 @@
 
 #define LNB_CRC_THREADS 256
 
-__global__ void __launch_bounds__(LNB_CRC_THREADS) lnb_crc_v2_kernel(LnbDecodeBatch b)
+/* the check of block i of the batch by the whole CTA (also the salvage decodes' CRC pass, lnb_salvage.cuh) */
+__device__ __forceinline__ void lnb_crc_v2_block(const LnbDecodeBatch &b, uint32_t i)
 {
     __shared__ uint16_t tab[256];
     __shared__ uint32_t part[LNB_CRC_THREADS];
     const uint32_t tid = threadIdx.x;
-    LnbBlockDesc &gblk = b.blocks[blockIdx.x];
+    LnbBlockDesc &gblk = b.blocks[i];
     const LnbBlockDesc blk = gblk;
     tab[tid] = b.tab.crc_table[tid];
     const uint8_t *base = b.stream + blk.byte_off;
@@ -42,4 +43,9 @@ __global__ void __launch_bounds__(LNB_CRC_THREADS) lnb_crc_v2_kernel(LnbDecodeBa
         gblk.crc = got;
         if (b.cfg.check_crc && got != lnb_get_be(base + 6, 2)) atomicOr(&gblk.status, (uint32_t)LNB_ST_CRC_MISMATCH);   /* the throughput entropy stage may flag the block at the same time */
     }
+}
+
+__global__ void __launch_bounds__(LNB_CRC_THREADS) lnb_crc_v2_kernel(LnbDecodeBatch b)
+{
+    lnb_crc_v2_block(b, blockIdx.x);
 }

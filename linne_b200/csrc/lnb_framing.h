@@ -1,7 +1,8 @@
 /* lnb_framing.h -- the framing of a stream's blocks: the checks of one block header and the hop over them.
  *
  * One definition for every reader of a stream: the host hop (csrc/host/linne_decoder_host.c), the device hop
- * (lnb_hop.cuh) and the seek of sample-window decodes (lnb_window.cuh).  Compiles as C99 (host code), as CUDA and as
+ * (lnb_hop.cuh), the seek of sample-window decodes (lnb_window.cuh) and the resynchronising scan of salvage decodes
+ * (lnb_salvage.cuh).  Compiles as C99 (host code), as CUDA and as
  * C++ (the CPU simulator).
  *
  * Per block the reference checks, in this order (linne_decoder.c:604-653):
@@ -50,6 +51,15 @@ LNB_FRAMING_FN uint32_t lnb_block_body(uint32_t type, uint32_t ns, uint32_t rema
     return LNB_HOP_OK;
 }
 
+/* the offset of the block after a framed block at `off` (the reference's hop rule): raw and silent blocks by what their
+ * payload holds, compressed ones by their size field (== 11 + ceil(bits/8) for any stream an encoder wrote) */
+LNB_FRAMING_FN uint32_t lnb_block_next(uint32_t off, uint32_t type, uint32_t size32, uint32_t ns, uint32_t channels, uint32_t bits)
+{
+    if (type == LNB_BLOCK_RAW) return off + LNB_BLOCK_HEADER_SIZE + (bits / 8u) * ns * channels;
+    if (type == LNB_BLOCK_SILENT) return off + LNB_BLOCK_HEADER_SIZE;
+    return off + size32 + 6u;
+}
+
 /* The hop over the blocks of data[off, data_size) until `sample_limit` samples or `block_limit` blocks (0: no limit),
  * checked against `room` samples of output.  Fills table[] (byte offsets plus `base`) and *out; sets out->overflow and
  * stops when more than `table_cap` entries are needed. */
@@ -78,9 +88,7 @@ LNB_FRAMING_FN void lnb_hop_blocks(const uint8_t *data, uint32_t data_size, uint
         if ((err = lnb_block_body(type, ns, remain, channels, bits)) != LNB_HOP_OK) { out->post_crc_error = err; break; }
         out->num_decodable = nb;
         progress += ns;
-        if (type == LNB_BLOCK_RAW) off += LNB_BLOCK_HEADER_SIZE + (bits / 8u) * ns * channels;
-        else if (type == LNB_BLOCK_SILENT) off += LNB_BLOCK_HEADER_SIZE;
-        else off += size32 + 6u;                                   /* == 11 + ceil(bits/8) for any stream an encoder wrote */
+        off = lnb_block_next(off, type, size32, ns, channels, bits);
         if (block_limit && nb >= block_limit) break;
     }
     out->num_blocks = nb;

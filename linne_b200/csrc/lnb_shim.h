@@ -84,6 +84,16 @@ int lnb_shim_gather_windows(LnbDevice *dev, const int32_t *d_scratch, uint32_t s
 int lnb_shim_gather_windows_packed(LnbDevice *dev, const int32_t *d_scratch, uint32_t scratch_stride, const LnbGatherWin *d_wins,
                                    uint32_t num_wins, uint32_t num_items, uint8_t *d_dst, uint32_t channels, uint32_t bytes);
 
+/* salvage decodes (lnb_salvage.cuh), enqueue only.  resync_scan: every position of d_image[30, data_size) whose bytes frame
+ * as a block of the stream (lnb_framing.h) with 1 .. block_size samples goes to d_table (at most `cap` entries, in no
+ * particular order); *d_count, zero before, counts them all.  d_image is padded to ROUNDUP(data_size + 16, 16) bytes.
+ * crc_blocks: the CRC check of the first min(*d_count, cap) entries of d_table (LNB_ST_CRC_MISMATCH in .status, the CRC
+ * in .crc), with the decoder's CRC arithmetic. */
+int lnb_shim_resync_scan(LnbDevice *dev, const uint8_t *d_image, uint32_t data_size, uint32_t channels, uint32_t bits,
+                         uint32_t block_size, LnbBlockDesc *d_table, uint32_t *d_count, uint32_t cap);
+int lnb_shim_crc_blocks(LnbDevice *dev, const uint8_t *d_image, uint32_t data_size, LnbBlockDesc *d_table,
+                        const uint32_t *d_count, uint32_t cap);
+
 /* packed interleaved PCM (WAV data-chunk layout, `bytes` per sample) <-> int32 planes, on the device (enqueue only) */
 int lnb_shim_unpack_pcm(LnbDevice *dev, const uint8_t *d_packed, int32_t *d_pcm, uint32_t pcm_stride,
                         uint32_t frames, uint32_t channels, uint32_t bytes);

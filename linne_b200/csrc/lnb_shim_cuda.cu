@@ -23,6 +23,7 @@
 #include "lnb_stream_v2.cuh"
 #include "lnb_hop.cuh"
 #include "lnb_window.cuh"
+#include "lnb_salvage.cuh"
 
 #define LNB_MAX_STAGES 32
 #define LNB_MAX_PENDING 8192
@@ -605,6 +606,34 @@ int lnb_shim_gather_windows_packed(LnbDevice *dev, const int32_t *d_scratch, uin
     bind_device(dev);
     CudaExec ex{dev};
     lnb_gather_windows_packed_pipeline(ex, d_scratch, scratch_stride, d_wins, num_wins, num_items, d_dst, channels, bytes);
+    return dev->last_error == cudaSuccess ? 0 : 1;
+}
+
+int lnb_shim_resync_scan(LnbDevice *dev, const uint8_t *d_image, uint32_t data_size, uint32_t channels, uint32_t bits,
+                         uint32_t block_size, LnbBlockDesc *d_table, uint32_t *d_count, uint32_t cap)
+{
+    bind_device(dev);
+    CudaExec ex{dev};
+    lnb_resync_scan_pipeline(ex, d_image, data_size, channels, bits, block_size, d_table, d_count, cap);
+    return dev->last_error == cudaSuccess ? 0 : 1;
+}
+int lnb_shim_crc_blocks(LnbDevice *dev, const uint8_t *d_image, uint32_t data_size, LnbBlockDesc *d_table,
+                        const uint32_t *d_count, uint32_t cap)
+{
+    bind_device(dev);
+    if (cap == 0) return 0;
+    CudaExec ex{dev};
+    LnbDecodeBatch b;
+    memset(&b, 0, sizeof(b));
+    b.cfg.check_crc = 1u;
+    b.tab = dev->tables;
+    b.stream = d_image;
+    b.stream_size = data_size;
+    b.blocks = d_table;
+    b.num_blocks = cap;
+    const int slot = ex.begin_stage("salvage_crc");
+    lnb_salvage_crc_kernel<<<cap, LNB_CRC_THREADS, 0, dev->stream>>>(b, d_count);
+    ex.end_stage(slot);
     return dev->last_error == cudaSuccess ? 0 : 1;
 }
 

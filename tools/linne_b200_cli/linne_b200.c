@@ -17,6 +17,7 @@
  *
  *   linne_b200 -e [-m 0..7] [-l] [-a N] in.wav out.lnn [in2.wav out2.lnn ...]
  *   linne_b200 -d [-c] [--start FRAME] [--length FRAMES]  in.lnn out.wav [in2.lnn out2.wav ...]
+ *   linne_b200 -d -F in.lnn out.wav [...]   (decode through damage)
  *   linne_b200 -e|-d ... -L pairs.txt   (one "input output" pair per line)
  *   -j N  workers (default: min(4, files))      -s  print a timing summary (samples, seconds, MSamples/s)
  *
@@ -24,6 +25,11 @@
  * stream when --length is not given.  Each file is indexed (LINNEB200_DecoderBuildIndex) and only the blocks the excerpt
  * overlaps are decoded, in one LINNEB200_DecodeWindowsPacked call straight into the WAV staging buffer.  An excerpt that
  * does not lie inside a stream fails that file, and nothing is written for it.
+ *
+ * -F decodes through damage (LINNEB200_DecodeSalvagePacked): every intact block lands where it belongs in a WAV of the
+ * stream's full length, what was lost is silence, and each lost run is reported on stderr as
+ * "in.lnn: frames [a, b) lost, bytes [x, y): STATUS".  The stream's own 30-byte header must be readable.  The exit code is
+ * 2 when a file was damaged (and none failed), 1 when one failed, 0 otherwise.  -F does not combine with --start / --length.
  */
 #define _POSIX_C_SOURCE 200809L
 #include <linne_encoder.h>
@@ -66,6 +72,9 @@ struct Worker {
     struct Staging in, out;
     struct LINNEB200SeekPoint *points;         /* seek index of the current stream (excerpts), grow-only */
     uint32_t points_cap;
+    struct LINNEB200Damage *damage;            /* salvage records of the current stream (-F), grow-only */
+    uint32_t damage_cap;
+    int damaged;                               /* files decoded through damage */
     uint64_t samples;                          /* samples (frames x channels) that went through */
     int failures;
 };
@@ -140,6 +149,7 @@ static int wav_write(const char *path, uint8_t *buf, const struct Wav *w)
 struct Options {
     int encode, decode, preset, learning, af, no_crc, jobs, stats;
     int excerpt, has_length;                   /* --start and/or --length given; --length given */
+    int salvage;                               /* -F: decode through damage */
     uint32_t start, length;
     const char *list;
 };
@@ -205,6 +215,45 @@ static int decode_excerpt(struct Worker *wk, const struct Options *o, const char
     return 0;
 }
 
+static const char *result_name(int32_t r)
+{
+    static const char *names[] = {"OK", "INVALID_ARGUMENT", "INVALID_FORMAT", "INSUFFICIENT_BUFFER", "INSUFFICIENT_DATA",
+                                  "PARAMETER_NOT_SET", "DETECT_DATA_CORRUPTION", "NG"};
+    return (r >= 0 && r < 8) ? names[r] : "?";
+}
+
+/* -F: the whole stream through damage, straight into the WAV staging buffer; one stderr line per lost run */
+static int decode_salvage(struct Worker *wk, const char *in, const uint8_t *buf, uint32_t size, uint8_t *wav,
+                          const struct LINNEHeader *h)
+{
+    LINNEApiResult ret;
+    uint32_t n = 0, i;
+    if ((ret = LINNEDecoder_SetHeader(wk->dec, h)) != LINNE_APIRESULT_OK) { SAY(stderr, "linne_b200: %s: decode failed (%d)\n", in, (int)ret); return 1; }
+    if (!wk->damage) {                         /* room for the usual reports: the call runs once */
+        if (!(wk->damage = (struct LINNEB200Damage *)malloc(256u * sizeof(*wk->damage)))) { SAY(stderr, "linne_b200: %s: out of memory for the damage report\n", in); return 1; }
+        wk->damage_cap = 256u;
+    }
+    for (;;) {
+        ret = LINNEB200_DecodeSalvagePacked(wk->dec, buf, size, wav + 44, h->num_samples, wk->damage, wk->damage_cap, &n);
+        if ((ret != LINNE_APIRESULT_OK && ret != LINNE_APIRESULT_DETECT_DATA_CORRUPTION) || n <= wk->damage_cap) break;
+        {   /* more lost runs than records: room for all of them, and the call again */
+            struct LINNEB200Damage *d = (struct LINNEB200Damage *)realloc(wk->damage, (size_t)n * sizeof(*d));
+            if (!d) { SAY(stderr, "linne_b200: %s: out of memory for the damage report\n", in); return 1; }
+            wk->damage = d;
+            wk->damage_cap = n;
+        }
+    }
+    if (ret != LINNE_APIRESULT_OK && ret != LINNE_APIRESULT_DETECT_DATA_CORRUPTION) { SAY(stderr, "linne_b200: %s: decode failed (%d)\n", in, (int)ret); return 1; }
+    pthread_mutex_lock(&g_print);
+    for (i = 0; i < n; i++)
+        fprintf(stderr, "%s: frames [%u, %u) lost, bytes [%u, %u): %s\n", in, wk->damage[i].first_sample,
+                wk->damage[i].first_sample + wk->damage[i].num_samples, wk->damage[i].byte_offset,
+                wk->damage[i].byte_offset + wk->damage[i].byte_size, result_name(wk->damage[i].status));
+    pthread_mutex_unlock(&g_print);
+    if (n) wk->damaged++;
+    return 0;
+}
+
 static int decode_one(struct Worker *wk, const struct Options *o, const char *in, const char *out)
 {
     size_t size = 0;
@@ -232,6 +281,9 @@ static int decode_one(struct Worker *wk, const struct Options *o, const char *in
     if (!(wav = staging_reserve(&wk->out, 44u + (size_t)w.frames * w.channels * (w.bits / 8u) + 16u))) return 1;
     if (o->excerpt) {
         if (decode_excerpt(wk, o, in, buf, (uint32_t)size, wav, &w)) return 1;
+        frames = w.frames;
+    } else if (o->salvage) {
+        if (decode_salvage(wk, in, buf, (uint32_t)size, wav, &h)) return 1;
         frames = w.frames;
     } else if ((ret = LINNEB200_DecodeWholePacked(wk->dec, buf, (uint32_t)size, wav + 44, w.frames, &frames)) != LINNE_APIRESULT_OK) {
         SAY(stderr, "linne_b200: %s: decode failed (%d)\n", in, (int)ret);
@@ -295,13 +347,16 @@ static void usage(const char *argv0)
     fprintf(stderr,
         "usage: %s -e [-m 0..7] [-l] [-a N] in.wav out.lnn [in2.wav out2.lnn ...]\n"
         "       %s -d [-c] [--start FRAME] [--length FRAMES] in.lnn out.wav [in2.lnn out2.wav ...]\n"
+        "       %s -d -F in.lnn out.wav [...]   decode through damage\n"
         "       -L FILE reads \"input output\" pairs from FILE (one per line)\n"
         "       -j N    pipeline workers (handles) working on different files at the same time (default min(4, files))\n"
         "       -s      print a timing summary\n"
         "  -e encode  -d decode  -m compress mode (default 0)  -l learning  -a auxiliary-function iterations\n"
         "  -c do NOT check CRC16 when decoding\n"
         "  --start FRAME, --length FRAMES  decode only frames [FRAME, FRAME + FRAMES) of every stream (-d only;\n"
-        "                                  default start 0, length to the end of the stream)\n", argv0, argv0);
+        "                                  default start 0, length to the end of the stream)\n"
+        "  -F decode every intact block of a damaged stream (-d only): a full-length WAV with silence where blocks\n"
+        "     were lost, one stderr line per lost run; exit code 2 when a file was damaged\n", argv0, argv0, argv0);
 }
 
 int main(int argc, char **argv)
@@ -309,7 +364,7 @@ int main(int argc, char **argv)
     struct Options o;
     const char *files[4096];
     char *owned[4096];
-    int nfiles = 0, nowned = 0, i, failures = 0, jobs;
+    int nfiles = 0, nowned = 0, i, failures = 0, damaged = 0, jobs;
     struct Queue q;
     struct WorkerArg *workers;
     uint64_t samples = 0;
@@ -326,6 +381,7 @@ int main(int argc, char **argv)
         else if (!strcmp(a, "-L") && i + 1 < argc) o.list = argv[++i];
         else if ((!strcmp(a, "-j") || !strcmp(a, "--jobs")) && i + 1 < argc) o.jobs = atoi(argv[++i]);
         else if (!strcmp(a, "-s") || !strcmp(a, "--stats")) o.stats = 1;
+        else if (!strcmp(a, "-F") || !strcmp(a, "--salvage")) o.salvage = 1;
         else if (!strcmp(a, "--start") || !strcmp(a, "--length")) {
             const int is_len = (a[2] == 'l');
             if (i + 1 >= argc || parse_frames(argv[++i], is_len ? &o.length : &o.start)) {
@@ -350,6 +406,7 @@ int main(int argc, char **argv)
     }
     if (o.encode == o.decode) { fprintf(stderr, "%s: exactly one of -e and -d must be given\n", argv[0]); usage(argv[0]); return 1; }
     if (o.excerpt && o.encode) { fprintf(stderr, "%s: --start and --length apply to -d only\n", argv[0]); usage(argv[0]); return 1; }
+    if (o.salvage && (o.encode || o.excerpt)) { fprintf(stderr, "%s: -F applies to -d without --start / --length\n", argv[0]); usage(argv[0]); return 1; }
     if (nfiles < 2 || (nfiles & 1)) { fprintf(stderr, "%s: input and output files must come in pairs\n", argv[0]); return 1; }
     if (o.preset < 0 || o.preset >= LINNE_NUM_PARAMETER_PRESETS || o.af < 0 || o.af >= 255) { fprintf(stderr, "%s: option out of range\n", argv[0]); return 1; }
 
@@ -391,12 +448,14 @@ int main(int argc, char **argv)
     t1 = now_s();
     for (i = 0; i < jobs; i++) {
         failures += workers[i].wk.failures;
+        damaged += workers[i].wk.damaged;
         samples += workers[i].wk.samples;
         if (workers[i].wk.enc) LINNEEncoder_Destroy(workers[i].wk.enc);
         if (workers[i].wk.dec) LINNEDecoder_Destroy(workers[i].wk.dec);
         staging_release(&workers[i].wk.in);
         staging_release(&workers[i].wk.out);
         free(workers[i].wk.points);
+        free(workers[i].wk.damage);
     }
     free(workers);
     pthread_mutex_destroy(&q.lock);
@@ -404,5 +463,5 @@ int main(int argc, char **argv)
         fprintf(stderr, "{\"files\": %d, \"workers\": %d, \"samples\": %llu, \"seconds\": %.6f, \"msamples_per_s\": %.3f}\n",
                 nfiles / 2, jobs, (unsigned long long)samples, t1 - t0, (t1 > t0) ? (double)samples / (t1 - t0) / 1e6 : 0.0);
     for (i = 0; i < nowned; i++) free(owned[i]);
-    return failures ? 1 : 0;
+    return failures ? 1 : damaged ? 2 : 0;
 }
